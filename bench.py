@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            (N>1: launched by torch.distributed.run)
     python bench.py --impl reference --steps K --warmup W    (CPU arm: the reference algorithm on host cores)
+    python bench.py ... --dump-outputs DIR                   (also write the outputs of the last timed step: dump_outputs)
 
 One "step" = one pass of the whole hot path over one synthetic gray mosaic: sliding window ->
 ViT-S/8 CLS attention rows per 224x224 tile -> head mean / per-tile min-max / bilinear / ramp-blended
@@ -597,6 +598,26 @@ def masks_sha(out, names=("th", "th3")):
     return h.hexdigest()[:16]
 
 
+DUMP_SAMPLE = 1 << 22      # most elements written per output: 16 MiB in float32, so a whole dump stays below 64 MB
+
+
+def dump_outputs(out, directory):
+    """Writes what MosaicSegmenter.segment returned to the caller as <directory>/<name>.npy, so that two builds can be compared
+    output for output: the masks th / th3, the per-tile low-res maps, the Otsu thresholds, the histograms and the min/max keys.
+    Integer outputs are written as float64 (exact), the others as float32.  An output of more than DUMP_SAMPLE elements is
+    represented by its elements at DUMP_SAMPLE distinct flat indices, drawn with seed 0 and sorted: the same indices for every
+    run and build at a given mosaic size.  Smaller outputs are written whole, in their own shape."""
+    os.makedirs(directory, exist_ok=True)
+    for name in ("th", "th3", "lowres", "thresholds", "hists", "minmax_ord"):
+        t = out[name]
+        if t.numel() > DUMP_SAMPLE:
+            idx = np.sort(np.random.default_rng(0).choice(t.numel(), DUMP_SAMPLE, replace=False))
+            t = t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+        t = t.cpu()
+        a = t.numpy().astype(np.float32 if t.is_floating_point() or t.dtype == torch.uint8 else np.float64)
+        np.save(os.path.join(directory, name + ".npy"), a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -614,7 +635,12 @@ def main():
     ap.add_argument("--workload", default="segmentation", choices=["segmentation", "mim_train"],
                     help="segmentation = BASELINE.json configs[1] (the headline); mim_train = configs[3] (MIM pre-training step)")
     ap.add_argument("--batch-per-gpu", type=int, default=32, help="mim_train: images per GPU per step (256 over 8 GPUs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="segmentation: write the outputs of the last timed step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.workload != "segmentation" or args.impl != "ours"):
+        ap.error("--dump-outputs writes the outputs of the GPU segmentation path (--workload segmentation --impl ours)")
     if args.workload == "mim_train":
         return main_mim(args)
     if args.impl == "reference":
@@ -654,6 +680,8 @@ def main():
     extra_warmup = getattr(time_segmentation, "extra_warmup", 0)
     launches = vob._lib.launch_count() - mark["l0"]
     value = mp / (ms_per_step / 1e3)
+    if args.dump_outputs and rank == 0:      # before a later segment() call may reuse the buffers of `out`
+        dump_outputs(out, args.dump_outputs)
 
     # ---- end to end through the public API with HOST buffers (pinned), copies inside the timed region
     host_masks, shm_paths = shared_host_masks(D, vob, extent)
