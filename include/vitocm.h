@@ -45,7 +45,7 @@ typedef enum vitocm_precision {
 } vitocm_precision;
 
 /* Constructor constants of VisionTransformer (vit.py:137-139) and of the factories
- * vit_tiny/small/base (vit.py:259-279).  head_dim must be 64. */
+ * vit_tiny/small/base (vit.py:259-279).  head_dim = embed_dim / num_heads must be 64 or 128. */
 typedef struct vitocm_config {
   int embed_dim;
   int depth;
@@ -274,7 +274,7 @@ int vitocm_block_tail(vitocm_engine* e, const void* CTX, int64_t ld_ctx, const v
                       const float* ln2_b, const void* W1, int64_t ldw1, const void* W2, int64_t ldw2, int M, int D, int hidden, const float* bias1,
                       const float* bias2, float* X, const float* next_ln_w, const float* next_ln_b, void* XN, int64_t ld_xn, const void* Wqkv,
                       int64_t ldwqkv, const float* bias_qkv, void* QKV, int64_t ld_qkv, int64_t* stamps, void* stream);
-/* ctx = MHSA(qkv) for B images of n_tokens tokens: qkv bf16 [B*N][ld], ctx bf16 [B*N][ldo]. */
+/* ctx = MHSA(qkv) for B images of n_tokens tokens: qkv bf16 [B*N][ld] (columns [3][heads][head_dim]), ctx bf16 [B*N][ldo]. */
 int vitocm_attention(vitocm_engine* e, const void* qkv, int64_t ld, int B, int n_tokens, void* ctx, int64_t ldo,
                      void* stream);
 /* Diagnostics: vitocm_attention that also records SM-clock stamps of the CTAs of query tiles 0 and 1 of
@@ -335,7 +335,7 @@ int vitocm_wgrad(vitocm_engine* e, const void* G, int64_t ldg, const void* A, in
  * multiple of 128, pad rows hold +inf */
 int vitocm_attention_fwd_lse(vitocm_engine* e, const void* qkv, int64_t ld, int B, int n_tokens, void* ctx, int64_t ldo,
                              float* lse2, void* stream);
-/* backward of vitocm_attention: dqkv bf16 [B*N][ldq] (columns [3][H][64]) from dctx; scratch: delta [B][heads][Npad] fp32,
+/* backward of vitocm_attention: dqkv bf16 [B*N][ldq] (columns [3][heads][head_dim]) from dctx; scratch: delta [B][heads][Npad] fp32,
  * dqacc [B*N][D] fp32 (zero on entry, zero again on return) */
 int vitocm_attention_bwd(vitocm_engine* e, const void* qkv, int64_t ld, const void* ctx, const void* dctx, int64_t ldc,
                          const float* lse2, float* delta, float* dqacc, void* dqkv, int64_t ldq, int B, int n_tokens,

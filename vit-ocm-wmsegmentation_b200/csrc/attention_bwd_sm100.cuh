@@ -1,4 +1,4 @@
-// Flash-attention backward for sm_100a (head_dim 64), tcgen05 + TMEM + TMA -- the `loss.backward()` half of
+// Flash-attention backward for sm_100a (head_dim DH = 64 or 128), tcgen05 + TMEM + TMA -- the `loss.backward()` half of
 // SSS/dino/vision_transformer.py:83-87 (q@k^T*scale, softmax, attn@v) inside the MIM training step (SSS/mim.py:153-182).
 // Nothing N x N is ever written to HBM: P is recomputed from the saved log-sum-exp of the forward pass.
 //
@@ -20,6 +20,12 @@
 //               a 3-D tensor map [B][N][D] clips the rows beyond the image.
 // The same shared-memory image of P / dS serves as MN-major A (dV, dK) and as K-major A (dQ): no transposes.
 // dK_j, dV_j leave through registers as bf16 into the dQKV activation; dQacc is converted by dq_convert_kernel.
+// Head_dim 128 (DH = 128): every item also names one 64-column half of the head, and dK / dV / dQ of that half are its only
+// outputs, so the TMEM map above (S 128 | dP 128 | dV 64 | dK 64 | dQ 64) and the drains stay as they are; S and dP contract over
+// all 128 columns (8 k-steps across the two swizzle atoms of every tile).  The two halves of a key block recompute the same
+// P / dS: twice the exponentials of one pass, against a 128-column dQ that has no room in TMEM next to 128-key S, dP, dV and dK.
+// A [128 x 128] tile is 32 KB, so K / V and Q / dO get one shared-memory slot each (211 KB in all) and the MMA warp issues the
+// next tile's S / dP only after the current tile's dV / dK / dQ (AbwCfg::ONE_SLOT): its operands land in the slot those free.
 // Warp roles: warps 0..7 softmax/drain (quadrant = warp % 4, key-column half = warp / 4: two warps per scheduler hide each
 // other's MUFU / TMEM latencies -- the backward needs no row reductions, so a row splits freely), warp 8 = TMA producer,
 // warp 9 = MMA issuer + TMEM allocator.  Ragged tails are trimmed: a short key block runs S / dP at N = 32 per 32 keys and
@@ -31,15 +37,15 @@ namespace vitocm {
 
 struct AttnBwdArgs {
   int n_tokens;       // N
-  int embed_dim;      // D = H * 64
+  int embed_dim;      // D = H * DH
   int heads;
   float scale;        // qk scale
   float scale_log2;   // scale * log2(e)
   const float* lse2;  // [B][H][Npad], Npad = N rounded up to 128; +inf in the pad rows
   const float* delta; // [B][H][Npad]; 0 in the pad rows
-  __nv_bfloat16* dqkv;  // [B*N][ld]: dK at column D + h*64, dV at 2D + h*64 (dQ comes from dq_convert_kernel)
+  __nv_bfloat16* dqkv;  // [B*N][ld]: dK at column D + h*DH, dV at 2D + h*DH (dQ comes from dq_convert_kernel)
   long long ld;
-  int n_items;        // work items = key blocks x heads x images; persistent CTAs walk them with stride gridDim.x
+  int n_items;        // work items = (DH / 64 column halves x) key blocks x heads x images; persistent CTAs walk them with stride gridDim.x
   int debug;          // diagnostics (VITOCM_ABW_DEBUG): 1 = skip the dQ reduce-add, 2 = timeline stamps
 };
 
@@ -56,6 +62,18 @@ constexpr int ABW_STAT_BYTES = 2 * 1024;   // [2 slots][LSE2 | Delta][128 rows] 
 constexpr int ABW_DQ_STG_BYTES = 4 * 4096;
 constexpr int ABW_SMEM_BYTES = 4 * ABW_TILE + 4 * ABW_TILE + 2 * ABW_TILE + 2 * ABW_TILE + ABW_DQ_STG_BYTES + ABW_STAT_BYTES + 1024 + 256;
 
+template <int DH>
+struct AbwCfg {
+  static_assert(DH == 64 || DH == 128, "head_dim 64 or 128");
+  static constexpr int ATOMS = DH / 64;              // 64-column swizzle atoms per tile row; also column halves per item
+  static constexpr int TILE = ATOMS * ABW_TILE;      // one [128 x DH] bf16 tile
+  static constexpr int SLOTS = DH == 64 ? 2 : 1;     // K / V and Q / dO slots
+  static constexpr bool ONE_SLOT = SLOTS == 1;
+  static constexpr int SMEM_BYTES = SLOTS * 2 * TILE + SLOTS * 2 * TILE + 2 * ABW_TILE + 2 * ABW_TILE + ABW_DQ_STG_BYTES + ABW_STAT_BYTES + 1024 + 256;
+  static_assert(SMEM_BYTES <= 227 * 1024, "shared memory");
+};
+static_assert(AbwCfg<64>::SMEM_BYTES == ABW_SMEM_BYTES, "head_dim 64 layout");
+
 // diagnostics (VITOCM_ABW_DEBUG=2): SM-clock stamps of CTA (1,0,0) -- [role 0 = softmax warp 0, 1 = MMA thread][query tile < 8][event < 8]
 __device__ long long g_abw_timeline[2 * 8 * 8];
 __device__ __forceinline__ void abw_stamp(bool on, int role, int i, int ev) {
@@ -68,14 +86,17 @@ __device__ __forceinline__ void tma_reduce_add_3d(const CUtensorMap* tmap, uint3
                : "memory");
 }
 
+template <int DH = 64>
 __global__ void __launch_bounds__(ABW_THREADS, 1)
 attn_bwd_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __grid_constant__ CUtensorMap tmap_do,
                         const __grid_constant__ CUtensorMap tmap_dq, const AttnBwdArgs args) {
+  using Cfg = AbwCfg<DH>;
+  constexpr int ATOMS = Cfg::ATOMS, TILE = Cfg::TILE, SLOTS = Cfg::SLOTS;
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   const uint32_t smem = (ptx::smem_u32(smem_raw) + 1023u) & ~1023u;
-  const uint32_t smem_kv = smem;                          // [2 slots][K | V]
-  const uint32_t smem_qdo = smem_kv + 4 * ABW_TILE;       // [2 slots][Q | dO]
-  const uint32_t smem_p = smem_qdo + 4 * ABW_TILE;        // [2 atoms of 64 keys][128 q][128 B]
+  const uint32_t smem_kv = smem;                          // [SLOTS][K | V]
+  const uint32_t smem_qdo = smem_kv + SLOTS * 2 * TILE;   // [SLOTS][Q | dO]
+  const uint32_t smem_p = smem_qdo + SLOTS * 2 * TILE;    // [2 atoms of 64 keys][128 q][128 B]
   const uint32_t smem_ds = smem_p + 2 * ABW_TILE;
   const uint32_t smem_dq = smem_ds + 2 * ABW_TILE;        // fp32 staging, one 32 x 32 box per drain warp
   const uint32_t smem_stat = smem_dq + ABW_DQ_STG_BYTES;  // per query tile: LSE2 and Delta rows (bulk-copied by the producer)
@@ -99,8 +120,13 @@ attn_bwd_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __gr
   // this CTA's items: blockIdx.x, blockIdx.x + gridDim.x, ...; tiles are numbered t = w * n_q + i across them
   const int my_items = (args.n_items - static_cast<int>(blockIdx.x) + static_cast<int>(gridDim.x) - 1) / static_cast<int>(gridDim.x);
   const int T = my_items * n_q;
-  auto item_of = [&](int w, int& j, int& h, int& b) {
-    const int it = blockIdx.x + w * gridDim.x;
+  auto item_of = [&](int w, int& j, int& h, int& b, int& hc) {   // hc: first column of the item's half inside the head
+    int it = blockIdx.x + w * gridDim.x;
+    hc = 0;
+    if (ATOMS == 2) {
+      hc = (it & 1) * 64;
+      it >>= 1;
+    }
     j = it % n_q;
     h = (it / n_q) % args.heads;
     b = it / (n_q * args.heads);
@@ -142,23 +168,29 @@ attn_bwd_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __gr
     // ===================== TMA producer =====================
     if (ptx::elect_one()) {
       for (int w = 0; w < my_items; ++w) {
-        int j, h, b;
-        item_of(w, j, h, b);
+        int j, h, b, hc;
+        item_of(w, j, h, b, hc);
         const int row_base = b * N;
-        const int ks = w & 1;
-        ptx::mbar_wait(kv_empty + 8 * ks, ((w >> 1) & 1) ^ 1, 40);
-        ptx::mbar_arrive_expect_tx(kv_full + 8 * ks, 2 * ABW_TILE);
-        ptx::tma_load_2d(smem_kv + ks * 2 * ABW_TILE, &tmap_qkv, kv_full + 8 * ks, D + h * 64, row_base + j * 128);
-        ptx::tma_load_2d(smem_kv + ks * 2 * ABW_TILE + ABW_TILE, &tmap_qkv, kv_full + 8 * ks, 2 * D + h * 64, row_base + j * 128);
+        const int ks = w & (SLOTS - 1);
+        ptx::mbar_wait(kv_empty + 8 * ks, ((w >> (SLOTS - 1)) & 1) ^ 1, 40);
+        ptx::mbar_arrive_expect_tx(kv_full + 8 * ks, 2 * TILE);
+        for (int at = 0; at < ATOMS; ++at) {
+          ptx::tma_load_2d(smem_kv + ks * 2 * TILE + at * ABW_TILE, &tmap_qkv, kv_full + 8 * ks, D + h * DH + at * 64, row_base + j * 128);
+          ptx::tma_load_2d(smem_kv + ks * 2 * TILE + TILE + at * ABW_TILE, &tmap_qkv, kv_full + 8 * ks, 2 * D + h * DH + at * 64,
+                           row_base + j * 128);
+        }
         const long long stat_base = (static_cast<long long>(b) * args.heads + h) * (n_q * 128);
         for (int i = 0; i < n_q; ++i) {
-          const int t = w * n_q + i, slot = t & 1;
-          ptx::mbar_wait(qdo_empty + 8 * slot, ((t >> 1) & 1) ^ 1, 41);
-          ptx::mbar_arrive_expect_tx(qdo_full + 8 * slot, 2 * ABW_TILE + 1024);
+          const int t = w * n_q + i, slot = t & (SLOTS - 1);
+          ptx::mbar_wait(qdo_empty + 8 * slot, ((t >> (SLOTS - 1)) & 1) ^ 1, 41);
+          ptx::mbar_arrive_expect_tx(qdo_full + 8 * slot, 2 * TILE + 1024);
           ptx::bulk_load_1d(smem_stat + slot * 1024, args.lse2 + stat_base + i * 128, 512, qdo_full + 8 * slot);
           ptx::bulk_load_1d(smem_stat + slot * 1024 + 512, args.delta + stat_base + i * 128, 512, qdo_full + 8 * slot);
-          ptx::tma_load_2d(smem_qdo + slot * 2 * ABW_TILE, &tmap_qkv, qdo_full + 8 * slot, h * 64, row_base + i * 128);
-          ptx::tma_load_2d(smem_qdo + slot * 2 * ABW_TILE + ABW_TILE, &tmap_do, qdo_full + 8 * slot, h * 64, row_base + i * 128);
+          for (int at = 0; at < ATOMS; ++at) {
+            ptx::tma_load_2d(smem_qdo + slot * 2 * TILE + at * ABW_TILE, &tmap_qkv, qdo_full + 8 * slot, h * DH + at * 64, row_base + i * 128);
+            ptx::tma_load_2d(smem_qdo + slot * 2 * TILE + TILE + at * ABW_TILE, &tmap_do, qdo_full + 8 * slot, h * DH + at * 64,
+                             row_base + i * 128);
+          }
         }
       }
     }
@@ -172,36 +204,40 @@ attn_bwd_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __gr
       const uint64_t ds_desc_k = ptx::make_smem_desc_sw128(smem_ds, 1024, 0);
       // S = Q K^T and dP = dO V^T of tile t (item w = t / n_q); only the 32-key chunks that hold keys
       auto issue_sdp = [&](int t) {
-        const int w = t / n_q, i = t - w * n_q, slot = t & 1, ks = w & 1;
-        int j, h, b;
-        item_of(w, j, h, b);
-        if (i == 0) ptx::mbar_wait(kv_full + 8 * ks, (w >> 1) & 1, 42);
-        ptx::mbar_wait(qdo_full + 8 * slot, (t >> 1) & 1, 41);
+        const int w = t / n_q, i = t - w * n_q, slot = t & (SLOTS - 1), ks = w & (SLOTS - 1);
+        int j, h, b, hc;
+        item_of(w, j, h, b, hc);
+        if (i == 0) ptx::mbar_wait(kv_full + 8 * ks, (w >> (SLOTS - 1)) & 1, 42);
+        ptx::mbar_wait(qdo_full + 8 * slot, (t >> (SLOTS - 1)) & 1, 41);
         ptx::tc_fence_after();
         const uint32_t idesc_s = ptx::make_idesc(128, ((kv_len_of(j) + 31) >> 5) * 32, false, false);
-        const uint64_t k_desc = ptx::make_smem_desc_sw128(smem_kv + ks * 2 * ABW_TILE, 1024, 0);
-        const uint64_t v_desc = ptx::desc_advance(k_desc, ABW_TILE);
-        const uint64_t q_desc = ptx::make_smem_desc_sw128(smem_qdo + slot * 2 * ABW_TILE, 1024, 0);
-        const uint64_t do_desc = ptx::desc_advance(q_desc, ABW_TILE);
+        const uint64_t k_desc = ptx::make_smem_desc_sw128(smem_kv + ks * 2 * TILE, 1024, 0);
+        const uint64_t v_desc = ptx::desc_advance(k_desc, TILE);
+        const uint64_t q_desc = ptx::make_smem_desc_sw128(smem_qdo + slot * 2 * TILE, 1024, 0);
+        const uint64_t do_desc = ptx::desc_advance(q_desc, TILE);
+        // k step = 16 columns: 32 B inside a swizzle atom, the next atom every 4 steps
 #pragma unroll
-        for (int k = 0; k < 4; ++k)
-          ptx::umma_bf16_ss(tmem_base + ABW_S_COL, ptx::desc_advance(q_desc, k * 32), ptx::desc_advance(k_desc, k * 32), idesc_s, k ? 1u : 0u);
+        for (int k = 0; k < DH / 16; ++k)
+          ptx::umma_bf16_ss(tmem_base + ABW_S_COL, ptx::desc_advance(q_desc, (k >> 2) * ABW_TILE + (k & 3) * 32),
+                            ptx::desc_advance(k_desc, (k >> 2) * ABW_TILE + (k & 3) * 32), idesc_s, k ? 1u : 0u);
 #pragma unroll
-        for (int k = 0; k < 4; ++k)
-          ptx::umma_bf16_ss(tmem_base + ABW_DP_COL, ptx::desc_advance(do_desc, k * 32), ptx::desc_advance(v_desc, k * 32), idesc_s, k ? 1u : 0u);
+        for (int k = 0; k < DH / 16; ++k)
+          ptx::umma_bf16_ss(tmem_base + ABW_DP_COL, ptx::desc_advance(do_desc, (k >> 2) * ABW_TILE + (k & 3) * 32),
+                            ptx::desc_advance(v_desc, (k >> 2) * ABW_TILE + (k & 3) * 32), idesc_s, k ? 1u : 0u);
         ptx::umma_commit(sdp_full);
       };
       if (T > 0) issue_sdp(0);
       for (int t = 0; t < T; ++t) {
-        const int w = t / n_q, i = t - w * n_q, slot = t & 1, ks = w & 1;
-        int j, h, b;
-        item_of(w, j, h, b);
+        const int w = t / n_q, i = t - w * n_q, slot = t & (SLOTS - 1), ks = w & (SLOTS - 1);
+        int j, h, b, hc;
+        item_of(w, j, h, b, hc);
         const int kv_len = kv_len_of(j);
         const bool tl = args.debug == 2 && blockIdx.x == 1 && w == 0;
         abw_stamp(tl, 1, i, 0);
         // the next tile's logits go first, as soon as the softmax warps hold S / dP of this tile in registers: they are ready
         // long before those warps finish tile t, and the tensor core runs dV / dK / dQ of tile t under the exponentials of t + 1
-        if (t + 1 < T) {
+        // (one slot: the next tile's operands replace this tile's, so its S / dP follow this tile's MMAs below)
+        if (!Cfg::ONE_SLOT && t + 1 < T) {
           ptx::mbar_wait(sdp_free, t & 1, 49);
           ptx::tc_fence_after();
           issue_sdp(t + 1);
@@ -213,9 +249,10 @@ attn_bwd_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __gr
           ptx::mbar_wait(dkv_empty, (w - 1) & 1, 51);
           ptx::tc_fence_after();
         }
-        const uint64_t q_desc_mn = ptx::make_smem_desc_sw128(smem_qdo + slot * 2 * ABW_TILE, 1024, 1024);
-        const uint64_t do_desc_mn = ptx::desc_advance(q_desc_mn, ABW_TILE);
-        const uint64_t k_desc_mn = ptx::make_smem_desc_sw128(smem_kv + ks * 2 * ABW_TILE, 1024, 1024);
+        // MN-major B operands: the item's 64-column half (atom hc / 64) of Q_i, dO_i, K_j
+        const uint64_t q_desc_mn = ptx::make_smem_desc_sw128(smem_qdo + slot * 2 * TILE + (hc / 64) * ABW_TILE, 1024, 1024);
+        const uint64_t do_desc_mn = ptx::desc_advance(q_desc_mn, TILE);
+        const uint64_t k_desc_mn = ptx::make_smem_desc_sw128(smem_kv + ks * 2 * TILE + (hc / 64) * ABW_TILE, 1024, 1024);
         const uint32_t acc0 = i > 0 ? 1u : 0u;
         int q_len = N - i * 128;
         q_len = q_len > 128 ? 128 : q_len;
@@ -257,6 +294,11 @@ attn_bwd_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __gr
         ptx::umma_commit(dq_full);
         if (i == n_q - 1) ptx::umma_commit(kv_empty + 8 * ks);   // last reader of this K / V slot
         abw_stamp(tl, 1, i, 2);
+        if (Cfg::ONE_SLOT && t + 1 < T) {
+          ptx::mbar_wait(sdp_free, t & 1, 49);
+          ptx::tc_fence_after();
+          issue_sdp(t + 1);
+        }
       }
     }
   } else if (warp >= ABW_DRAIN_WARP0 && warp < ABW_DRAIN_WARP0 + 4) {
@@ -268,8 +310,8 @@ attn_bwd_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __gr
     const int sw = lane & 7;
     for (int t = 0; t < T; ++t) {
       const int w = t / n_q, i = t - w * n_q;
-      int j, h, b;
-      item_of(w, j, h, b);
+      int j, h, b, hc;
+      item_of(w, j, h, b, hc);
       ptx::mbar_wait(dq_full, t & 1, 46);
       ptx::tc_fence_after();
       const bool store = i * 128 + q * 32 < N && args.debug != 1;
@@ -290,7 +332,7 @@ attn_bwd_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __gr
         ptx::fence_proxy_async_smem();
         __syncwarp();
         if (lane == 0 && store) {
-          tma_reduce_add_3d(&tmap_dq, stg, h * 64 + hb * 32, i * 128 + q * 32, b);
+          tma_reduce_add_3d(&tmap_dq, stg, h * DH + hc + hb * 32, i * 128 + q * 32, b);
           ptx::bulk_commit();
         }
       }
@@ -309,10 +351,10 @@ attn_bwd_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __gr
     // dK_j (warps 0..3) / dV_j (warps 4..7) of item w: TMEM -> registers -> bf16 rows of dQKV.  Called once all MMAs of the item
     // have retired (dq_full of its last tile); the MMA warp may overwrite the accumulators after the dkv_empty arrive.
     auto drain_dkv = [&](int w) {
-      int j, h, b;
-      item_of(w, j, h, b);
+      int j, h, b, hc;
+      item_of(w, j, h, b, hc);
       const int kv_len = kv_len_of(j);
-      __nv_bfloat16* o = args.dqkv + static_cast<long long>(b * N + j * 128 + r) * args.ld + h * 64 + (half == 0 ? D : 2 * D);
+      __nv_bfloat16* o = args.dqkv + static_cast<long long>(b * N + j * 128 + r) * args.ld + h * DH + hc + (half == 0 ? D : 2 * D);
       uint32_t t0[32], t1[32];
       ptx::tmem_ld_32x32b_x32(lane_addr + (half == 0 ? ABW_DK_COL : ABW_DV_COL), t0);        // warp-collective
       ptx::tmem_ld_32x32b_x32(lane_addr + (half == 0 ? ABW_DK_COL : ABW_DV_COL) + 32, t1);
@@ -339,17 +381,17 @@ attn_bwd_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __gr
     };
     for (int t = 0; t < T; ++t) {
       const int w = t / n_q, i = t - w * n_q;
-      int j, h, b;
-      item_of(w, j, h, b);
+      int j, h, b, hc;
+      item_of(w, j, h, b, hc);
       const int kv_len = kv_len_of(j);
       const int nch = (kv_len + 31) >> 5;          // 32-key chunks of this key block that hold keys
       const bool tl = args.debug == 2 && blockIdx.x == 1 && w == 0 && lane == 0;
       abw_stamp(tl && warp == 0, 0, i, 6);
       // row statistics of this query tile from shared memory (rows beyond the image: LSE2 = +inf -> P = 0 -> dS = 0; dP is
       // finite there: the rows hold other tokens or zeros)
-      ptx::mbar_wait(qdo_full + 8 * (t & 1), (t >> 1) & 1, 50);
-      const float lse = ptx::lds_f32(smem_stat + (t & 1) * 1024 + r * 4);
-      const float dlt = ptx::lds_f32(smem_stat + (t & 1) * 1024 + 512 + r * 4);
+      ptx::mbar_wait(qdo_full + 8 * (t & (SLOTS - 1)), (t >> (SLOTS - 1)) & 1, 50);
+      const float lse = ptx::lds_f32(smem_stat + (t & (SLOTS - 1)) * 1024 + r * 4);
+      const float dlt = ptx::lds_f32(smem_stat + (t & (SLOTS - 1)) * 1024 + 512 + r * 4);
       const uint64_t nlse_2 = ptx::dup_f32x2(-lse);
       const uint64_t ndl_2 = ptx::dup_f32x2(-dlt * args.scale);
       abw_stamp(tl && warp == 0, 0, i, 0);

@@ -1,24 +1,24 @@
-// Flash-style multi-head self-attention for sm_100a (head_dim 64), tcgen05 + TMEM + TMA:
-//     ctx[b, i, h*64:(h+1)*64] = softmax_j( scale * q_i . k_j ) @ v        (never materialises N x N)
+// Flash-style multi-head self-attention for sm_100a (head_dim DH = 64 or 128), tcgen05 + TMEM + TMA:
+//     ctx[b, i, h*DH:(h+1)*DH] = softmax_j( scale * q_i . k_j ) @ v        (never materialises N x N)
 // Replaces SSS/dino/vision_transformer.py:83-87 (q@k^T*scale, softmax, attn@v, transpose/reshape)
 // for the blocks whose attention matrix is not returned.
 //
 // One work item = one (image b, head h, 128-query tile); CTAs are persistent and walk the items.  q/k/v are read straight out of the fused
-// QKV activation [B*N, ld] (bf16, columns [3][H][64]) by one 2-D TMA tensor map (box 64 x 128,
-// SWIZZLE_128B).  Warp roles (256 threads): warps 0..3 = softmax (one thread per query row; TMEM lane
+// QKV activation [B*N, ld] (bf16, columns [3][H][DH]) by one 2-D TMA tensor map (box 64 x 128,
+// SWIZZLE_128B; DH / 64 boxes per tile).  Warp roles (256 threads): warps 0..3 = softmax (one thread per query row; TMEM lane
 // quadrant = warp % 4), warp 4 = TMA producer, warp 5 = MMA issuer + TMEM allocator, warps 6..7 idle.
 // setmaxnreg moves registers from warpgroup 1 to the softmax warpgroup (208 vs 48 per thread in bf16 mode).
-//   S = Q K_j^T      : tcgen05.mma  M128 x N(<=128) x K64, both operands K-major, into TMEM
+//   S = Q K_j^T      : tcgen05.mma  M128 x N(<=128) x K(DH), both operands K-major, into TMEM
 //   softmax          : one tcgen05.ld pass of S into registers; scale/shift on the packed f32x2 pipe
 //                      (FFMA2), MUFU.EX2, row sums on FADD2, P -> TMEM (tcgen05.st, packed bf16x2 columns):
 //                      no shared-memory round trip, no generic->async proxy fence
-//   O += P V_j       : tcgen05.mma  M128 x N64 x K(<=128), A = P from TMEM, B = V (smem, MN-major),
+//   O += P V_j       : tcgen05.mma  M128 x N(DH) x K(<=128), A = P from TMEM, B = V (smem, MN-major),
 //                      accumulating in TMEM
 // The running maximum is only raised when a row exceeds it by more than 2^8 ("lazy rescale"): softmax
 // is shift invariant, so a stale maximum changes nothing but keeps O in TMEM untouched in the
 // common case; when it is raised the softmax warps rescale their O rows in TMEM.
-// Two CTAs are co-resident per SM (65 KB smem, 256 TMEM columns each: S 128 | O 64 | P 64) so one CTA's MMAs overlap
-// the other's exponentials.
+// At head_dim 64 two CTAs are co-resident per SM (65 KB smem, 256 TMEM columns each: S 128 | O 64 | P 64) so one CTA's MMAs
+// overlap the other's exponentials; head_dim 128 runs one CTA per SM (AttnCfg, DESIGN.md section 3).
 // Ragged query tail ("packed" items): N = 785 leaves 17 query rows per (image, head) beyond the last full tile; a tile of
 // its own would spend a full tile's exponentials on them (1/7 of the kernel).  Instead the tails of `pack` = 4 (<= 32 rows)
 // or 2 (<= 64 rows) consecutive (image, head) pairs share ONE 128-row tile, one 32- or 64-lane slot each: the S and PV MMAs
@@ -44,7 +44,7 @@ struct AttnArgs {
   int group_items;   // pack * n_fullq + (N % 128 != 0)
   int n_pairs;       // images x heads
   int n_tokens;      // N per image (785 for 224^2 / patch 8)
-  int embed_dim;     // D = H * 64
+  int embed_dim;     // D = H * head_dim
   int lo_col_off;    // SPLIT: column offset of the lo halves inside the qkv activation (= 3D)
   float scale_log2;  // qk scale * log2(e)
   __nv_bfloat16* out;  // ctx [B*N, ldo]
@@ -86,7 +86,7 @@ constexpr int ATT_TILE_BYTES = 128 * 64 * 2;  // 16 KB: one [128 x 64] bf16 tile
 #endif
 constexpr int ATT_RING = VITOCM_ATT_RING;     // K / V tiles in flight (measured: 4 / 5 slots are 1-2 % slower, with or without packed tail items)
 constexpr int ATT_S_COL = 0;      // S: 128 columns (fp32)
-constexpr int ATT_O_COL = 128;    // O: 64 columns (fp32)
+constexpr int ATT_O_COL = 128;    // O: 64 columns (fp32) at head_dim 64 (AttnCfg::O_COL / P_COL for either width)
 constexpr int ATT_P_COL = 192;    // P: 64 columns of packed bf16x2 (128 keys); split mode: lo part in the next 64
 constexpr float ATT_RESCALE_THRESHOLD = 8.0f;  // log2 units: raise the running maximum (rescale O, l) before the next block
 constexpr float ATT_REDO_THRESHOLD = 60.0f;    // log2 units: exp2 of the current block may overflow -> redo it now
@@ -97,16 +97,27 @@ constexpr float ATT_SUM_TRIGGER = 1.2676506e30f;      // 2^100
 constexpr float ATT_SUM_TRIGGER_F16 = 16384.0f;       // 2^14
 constexpr int ATT_POLY_DEFAULT = 0;            // see run_attention (0: all MUFU, 1: 4/16 polynomial, 2: 7/16)
 
-template <bool SPLIT>
+// DH = head_dim, 64 or 128.  A head row of 128 is two 128-byte swizzle atoms: every Q / K / V tile is ATOMS boxes of
+// [128 rows x 64 columns], 16 KB apart; one part (hi or lo) of a tile = ATOMS x 16 KB.
+// DH = 128 runs one CTA per SM: O takes 128 TMEM columns (S 128 | O 128 | P 64 [| P lo 64] <= 512), and Q + a 3-slot ring of
+// 32 KB K / V blocks (2 slots of 64 KB in split mode) leaves no room for a second CTA's shared memory.
+template <bool SPLIT, int DH = 64>
 struct AttnCfg {
+  static_assert(DH == 64 || DH == 128, "head_dim 64 or 128");
+  static constexpr int ATOMS = DH / 64;
   static constexpr int NPART = SPLIT ? 2 : 1;                     // hi (+ lo)
-  static constexpr int SLOT_BYTES = ATT_TILE_BYTES * NPART;       // one K or V block
-  static constexpr int Q_BYTES = ATT_TILE_BYTES * NPART;
-  static constexpr int SMEM_BYTES = Q_BYTES + ATT_RING * SLOT_BYTES + 1024 + 256;   // + alignment slack + barrier block
-  static constexpr int TMEM_COLS = SPLIT ? 512 : 256;
-  // setmaxnreg budgets: 2 CTAs/SM x 128 x (208 + 48) = 64 K registers (bf16); one CTA/SM in split mode
-  static constexpr int REGS_SOFTMAX = SPLIT ? 240 : 208;
-  static constexpr int REGS_OTHER = SPLIT ? 64 : 48;
+  static constexpr int PART_BYTES = ATT_TILE_BYTES * ATOMS;       // one [128 x DH] bf16 tile
+  static constexpr int SLOT_BYTES = PART_BYTES * NPART;           // one K or V block
+  static constexpr int Q_BYTES = PART_BYTES * NPART;
+  static constexpr int RING = (DH == 128 && SPLIT) ? 2 : ATT_RING;
+  static constexpr int SMEM_BYTES = Q_BYTES + RING * SLOT_BYTES + 1024 + 256;   // + alignment slack + barrier block
+  static constexpr bool ONE_CTA = SPLIT || DH == 128;             // one CTA per SM
+  static constexpr int TMEM_COLS = ONE_CTA ? 512 : 256;
+  static constexpr int O_COL = ATT_O_COL;                         // O: DH columns (fp32)
+  static constexpr int P_COL = ATT_O_COL + DH;                    // P: 64 columns of packed bf16x2; split mode: lo part in the next 64
+  // setmaxnreg budgets: 2 CTAs/SM x 128 x (208 + 48) = 64 K registers (bf16 at head_dim 64); one CTA/SM otherwise
+  static constexpr int REGS_SOFTMAX = ONE_CTA ? 240 : 208;
+  static constexpr int REGS_OTHER = ONE_CTA ? 64 : 48;
 };
 
 // work item -> (query tile, first pair, packed?); false = the item does not exist (pair beyond the batch in the last group)
@@ -148,27 +159,31 @@ __device__ __forceinline__ void att_slot_mask(int s, int nslots, uint32_t (&m)[4
 // F16: q / k / v, P and ctx are IEEE fp16 instead of bf16 (fp16 engines): 11 significand bits at the same tensor-core rate.  P is
 //      exp2 of (logit - running maximum) <= 2^ATT_RESCALE_THRESHOLD, or <= 2^redo threshold inside one block: the redo threshold
 //      drops to 14 so that P stays below fp16's 65504; below 6e-8 P flushes to zero, like everything under 2^-24 of the row sum.
-template <bool SPLIT, uint32_t POLY_MASK, bool PACKED, bool F16 = false>
-__global__ void __launch_bounds__(ATT_THREADS, SPLIT ? 1 : 2)
+// DH: head_dim (64 or 128, see AttnCfg)
+template <bool SPLIT, uint32_t POLY_MASK, bool PACKED, bool F16 = false, int DH = 64>
+__global__ void __launch_bounds__(ATT_THREADS, AttnCfg<SPLIT, DH>::ONE_CTA ? 1 : 2)
 attn_fwd_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __grid_constant__ CUtensorMap tmap_q32, const AttnArgs args) {
-  using Cfg = AttnCfg<SPLIT>;
+  using Cfg = AttnCfg<SPLIT, DH>;
   constexpr int NPART = Cfg::NPART;
+  constexpr int ATOMS = Cfg::ATOMS;
+  constexpr int RING = Cfg::RING;
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   const uint32_t smem = (ptx::smem_u32(smem_raw) + 1023u) & ~1023u;
   const uint32_t smem_q = smem;
   const uint32_t smem_ring = smem_q + Cfg::Q_BYTES;
-  const uint32_t bars = smem_ring + ATT_RING * Cfg::SLOT_BYTES;
+  const uint32_t bars = smem_ring + RING * Cfg::SLOT_BYTES;
   const uint32_t q_full = bars;             // [1]
-  const uint32_t kv_full = bars + 8;        // [ATT_RING]
-  const uint32_t kv_empty = kv_full + 8 * ATT_RING;   // [ATT_RING]
-  const uint32_t s_full = kv_empty + 8 * ATT_RING;    // MMA -> softmax
+  const uint32_t kv_full = bars + 8;        // [RING]
+  const uint32_t kv_empty = kv_full + 8 * RING;   // [RING]
+  const uint32_t s_full = kv_empty + 8 * RING;    // MMA -> softmax
   const uint32_t s_empty = s_full + 8;      // softmax -> MMA   (4 warps)
   const uint32_t p_full = s_full + 16;      // softmax -> MMA   (4 warps)
   const uint32_t o_full = s_full + 24;      // MMA -> softmax
   const uint32_t q_empty = s_full + 32;     // MMA -> producer: all S MMAs of the work item retired (Q tile reusable)
   const uint32_t o_empty = s_full + 40;     // softmax -> MMA: O of the finished work item has been read (4 warps)
   const uint32_t tmem_ptr_smem = s_full + 48;
-  static_assert(8 + 16 * ATT_RING + 56 <= 256, "barrier block overflows its 256 bytes");
+  static_assert(8 + 16 * RING + 56 <= 256, "barrier block overflows its 256 bytes");
+  static_assert(Cfg::SMEM_BYTES <= 227 * 1024, "shared memory");
 
   // Persistent CTA: work items (query tile, head, image), query tile fastest so that the CTAs running side by side share
   // one image-head's K / V through L2.  Barriers, the K/V ring and TMEM live across items (all phase counters run on), so
@@ -184,7 +199,7 @@ attn_fwd_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __gr
     ptx::prefetch_tmap(&tmap_qkv);
     ptx::prefetch_tmap(&tmap_q32);
     ptx::mbar_init(q_full, 1);
-    for (int i = 0; i < ATT_RING; ++i) {
+    for (int i = 0; i < RING; ++i) {
       ptx::mbar_init(kv_full + 8 * i, 1);
       ptx::mbar_init(kv_empty + 8 * i, 1);
     }
@@ -225,36 +240,39 @@ attn_fwd_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __gr
       if (!PACKED || !packed) {
         const int b = pair0 / args.heads, h = pair0 - b * args.heads;
         for (int part = 0; part < NPART; ++part)
-          ptx::tma_load_2d(smem_q + part * ATT_TILE_BYTES, &tmap_qkv, q_full, part * args.lo_col_off + h * ATT_DH,
-                           b * N + qt * ATT_BQ);
+          for (int at = 0; at < ATOMS; ++at)
+            ptx::tma_load_2d(smem_q + part * Cfg::PART_BYTES + at * ATT_TILE_BYTES, &tmap_qkv, q_full,
+                             part * args.lo_col_off + h * DH + at * 64, b * N + qt * ATT_BQ);
       } else {
         // four 32-row boxes; slot s owns tile rows [s * 128 / nslots, (s + 1) * 128 / nslots) = the first rows of its pair's tail
         const int per = 4 / nslots;
         for (int part = 0; part < NPART; ++part)
-          for (int u = 0; u < 4; ++u) {
-            const int pr = pair_of(u / per);
-            const int b = pr / args.heads, h = pr - b * args.heads;
-            ptx::tma_load_2d(smem_q + part * ATT_TILE_BYTES + u * 4096, &tmap_q32, q_full, part * args.lo_col_off + h * ATT_DH,
-                             b * N + qt * ATT_BQ + (u % per) * 32);
-          }
+          for (int at = 0; at < ATOMS; ++at)
+            for (int u = 0; u < 4; ++u) {
+              const int pr = pair_of(u / per);
+              const int b = pr / args.heads, h = pr - b * args.heads;
+              ptx::tma_load_2d(smem_q + part * Cfg::PART_BYTES + at * ATT_TILE_BYTES + u * 4096, &tmap_q32, q_full,
+                               part * args.lo_col_off + h * DH + at * 64, b * N + qt * ATT_BQ + (u % per) * 32);
+            }
       }
       // ring order = consumption order of the MMA warp: K0, K1, V0, K2, V1, ..., V_{n-1} (each entry = one tile per slot)
       int kv_col[4], kv_row[4];   // per slot: first column (head) and first row (image) of its pair's K / V, decoded once per item
       for (int sl = 0; sl < nslots; ++sl) {
         const int pr = pair_of(sl);
         const int b = pr / args.heads;
-        kv_col[sl] = (pr - b * args.heads) * ATT_DH;
+        kv_col[sl] = (pr - b * args.heads) * DH;
         kv_row[sl] = b * N;
       }
       auto load = [&](int which /*1 = K, 2 = V*/, int j) {
         for (int sl = 0; sl < nslots; ++sl) {
-          const int slot = item % ATT_RING;
-          const uint32_t parity = ((item / ATT_RING) & 1) ^ 1;
+          const int slot = item % RING;
+          const uint32_t parity = ((item / RING) & 1) ^ 1;
           ptx::mbar_wait(kv_empty + 8 * slot, parity, 10);
           ptx::mbar_arrive_expect_tx(kv_full + 8 * slot, Cfg::SLOT_BYTES);
           for (int part = 0; part < NPART; ++part)
-            ptx::tma_load_2d(smem_ring + slot * Cfg::SLOT_BYTES + part * ATT_TILE_BYTES, &tmap_qkv, kv_full + 8 * slot,
-                             part * args.lo_col_off + which * D + kv_col[sl], kv_row[sl] + j * ATT_BKV);
+            for (int at = 0; at < ATOMS; ++at)
+              ptx::tma_load_2d(smem_ring + slot * Cfg::SLOT_BYTES + part * Cfg::PART_BYTES + at * ATT_TILE_BYTES, &tmap_qkv,
+                               kv_full + 8 * slot, part * args.lo_col_off + which * D + kv_col[sl] + at * 64, kv_row[sl] + j * ATT_BKV);
           ++item;
         }
       };
@@ -272,7 +290,7 @@ attn_fwd_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __gr
     // leader-election loop); descriptors are advanced by compile-time constants in fully unrolled loops.
     if (ptx::elect_one()) {
       const uint32_t s_tmem = tmem_base + ATT_S_COL;
-      const uint32_t o_tmem = tmem_base + ATT_O_COL;
+      const uint32_t o_tmem = tmem_base + Cfg::O_COL;
       const uint64_t q_desc = ptx::make_smem_desc_sw128(smem_q, 1024, 0);
       int item = 0;   // K/V ring position, running across work items
       int g = 0;      // KV blocks processed so far (all work items): phase counter of s_full / s_empty / p_full / o_full
@@ -291,37 +309,40 @@ attn_fwd_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __gr
       auto issue_s = [&](int j) {
         const uint32_t idesc = ptx::make_idesc(ATT_BQ, kv_len_mma(j), false, false, F16 ? 0u : 1u);
         if (nslots == 1) {   // ordinary item: straight-line issue (this is the path every full tile takes)
-          const int slot = item % ATT_RING;
-          ptx::mbar_wait(kv_full + 8 * slot, (item / ATT_RING) & 1, 11);
+          const int slot = item % RING;
+          ptx::mbar_wait(kv_full + 8 * slot, (item / RING) & 1, 11);
           ptx::tc_fence_after();
           const uint64_t k_desc = ptx::make_smem_desc_sw128(smem_ring + slot * Cfg::SLOT_BYTES, 1024, 0);
           // terms: (Qhi,Khi) [, (Qhi,Klo), (Qlo,Khi)]; K-major operands advance 32 B per 16-wide k step
 #pragma unroll
           for (int t = 0; t < (SPLIT ? 3 : 1); ++t) {
-            const uint64_t qa = ptx::desc_advance(q_desc, t == 2 ? ATT_TILE_BYTES : 0);
-            const uint64_t ka = ptx::desc_advance(k_desc, t == 1 ? ATT_TILE_BYTES : 0);
+            const uint64_t qa = ptx::desc_advance(q_desc, t == 2 ? Cfg::PART_BYTES : 0);
+            const uint64_t ka = ptx::desc_advance(k_desc, t == 1 ? Cfg::PART_BYTES : 0);
+            // k step = 16 columns: 32 B inside a swizzle atom, the next atom every 4 steps
 #pragma unroll
-            for (int k = 0; k < ATT_DH / 16; ++k)
-              ptx::umma_bf16_ss(s_tmem, ptx::desc_advance(qa, k * 32), ptx::desc_advance(ka, k * 32), idesc, (t | k) ? 1u : 0u);
+            for (int k = 0; k < DH / 16; ++k)
+              ptx::umma_bf16_ss(s_tmem, ptx::desc_advance(qa, (k >> 2) * ATT_TILE_BYTES + (k & 3) * 32),
+                                ptx::desc_advance(ka, (k >> 2) * ATT_TILE_BYTES + (k & 3) * 32), idesc, (t | k) ? 1u : 0u);
           }
           ptx::umma_commit(kv_empty + 8 * slot);
           ++item;
         } else {
 #pragma unroll 1
           for (int sl = 0; sl < nslots; ++sl) {   // packed item: one masked MMA group per slot, each against its own pair's K
-            const int slot = item % ATT_RING;
-            ptx::mbar_wait(kv_full + 8 * slot, (item / ATT_RING) & 1, 11);
+            const int slot = item % RING;
+            ptx::mbar_wait(kv_full + 8 * slot, (item / RING) & 1, 11);
             ptx::tc_fence_after();
             const uint64_t k_desc = ptx::make_smem_desc_sw128(smem_ring + slot * Cfg::SLOT_BYTES, 1024, 0);
             uint32_t lm[4];
             att_slot_mask(sl, nslots, lm);
 #pragma unroll
             for (int t = 0; t < (SPLIT ? 3 : 1); ++t) {
-              const uint64_t qa = ptx::desc_advance(q_desc, t == 2 ? ATT_TILE_BYTES : 0);
-              const uint64_t ka = ptx::desc_advance(k_desc, t == 1 ? ATT_TILE_BYTES : 0);
+              const uint64_t qa = ptx::desc_advance(q_desc, t == 2 ? Cfg::PART_BYTES : 0);
+              const uint64_t ka = ptx::desc_advance(k_desc, t == 1 ? Cfg::PART_BYTES : 0);
 #pragma unroll
-              for (int k = 0; k < ATT_DH / 16; ++k)
-                ptx::umma_bf16_ss_masked(s_tmem, ptx::desc_advance(qa, k * 32), ptx::desc_advance(ka, k * 32), idesc, (t | k) ? 1u : 0u, lm);
+              for (int k = 0; k < DH / 16; ++k)
+                ptx::umma_bf16_ss_masked(s_tmem, ptx::desc_advance(qa, (k >> 2) * ATT_TILE_BYTES + (k & 3) * 32),
+                                         ptx::desc_advance(ka, (k >> 2) * ATT_TILE_BYTES + (k & 3) * 32), idesc, (t | k) ? 1u : 0u, lm);
             }
             ptx::umma_commit(kv_empty + 8 * slot);
             ++item;
@@ -333,8 +354,10 @@ attn_fwd_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __gr
       auto issue_pv = [&](int j) {
         // O accumulates across KV blocks in TMEM.
         // A = P in TMEM: 16 keys = 8 packed columns per step
-        // B = V: MN-major [keys x 64]; 16 keys = two 8-row groups of 1024 B
-        constexpr uint32_t idesc = ptx::make_idesc(ATT_BQ, ATT_DH, false, /*B = V is MN-major*/ true, F16 ? 0u : 1u);
+        // B = V: MN-major [keys x DH]; 16 keys = two 8-row groups of 1024 B; at DH = 128 the second 64 columns are the
+        // next swizzle atom (leading byte offset 16 KB)
+        constexpr uint32_t idesc = ptx::make_idesc(ATT_BQ, DH, false, /*B = V is MN-major*/ true, F16 ? 0u : 1u);
+        constexpr uint32_t v_lbo = DH == 64 ? 1024 : ATT_TILE_BYTES;
         const int ksteps = kv_len_mma(j) / 16;
         const uint32_t acc0 = j > 0 ? 1u : 0u;
         if (j == 0 && w > 0) {   // O still holds the previous work item until the softmax warps have read it out
@@ -342,15 +365,15 @@ attn_fwd_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __gr
           ptx::tc_fence_after();
         }
         if (nslots == 1) {   // ordinary item: straight-line issue
-          const int slot = item % ATT_RING;
-          ptx::mbar_wait(kv_full + 8 * slot, (item / ATT_RING) & 1, 12);
+          const int slot = item % RING;
+          ptx::mbar_wait(kv_full + 8 * slot, (item / RING) & 1, 12);
           ptx::tc_fence_after();
-          const uint64_t v_desc = ptx::make_smem_desc_sw128(smem_ring + slot * Cfg::SLOT_BYTES, 1024, 1024);
+          const uint64_t v_desc = ptx::make_smem_desc_sw128(smem_ring + slot * Cfg::SLOT_BYTES, 1024, v_lbo);
           // terms: (Phi,Vhi) [, (Phi,Vlo), (Plo,Vhi)]
 #pragma unroll
           for (int t = 0; t < (SPLIT ? 3 : 1); ++t) {
-            const uint32_t pa = tmem_base + ATT_P_COL + (t == 2 ? 64 : 0);
-            const uint64_t va = ptx::desc_advance(v_desc, t == 1 ? ATT_TILE_BYTES : 0);
+            const uint32_t pa = tmem_base + Cfg::P_COL + (t == 2 ? 64 : 0);
+            const uint64_t va = ptx::desc_advance(v_desc, t == 1 ? Cfg::PART_BYTES : 0);
             if (ksteps == ATT_BKV / 16) {
 #pragma unroll
               for (int k = 0; k < ATT_BKV / 16; ++k)
@@ -366,16 +389,16 @@ attn_fwd_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __gr
         } else {
 #pragma unroll 1
           for (int sl = 0; sl < nslots; ++sl) {   // packed item: slot sl's rows of P against its own pair's V
-            const int slot = item % ATT_RING;
-            ptx::mbar_wait(kv_full + 8 * slot, (item / ATT_RING) & 1, 12);
+            const int slot = item % RING;
+            ptx::mbar_wait(kv_full + 8 * slot, (item / RING) & 1, 12);
             ptx::tc_fence_after();
-            const uint64_t v_desc = ptx::make_smem_desc_sw128(smem_ring + slot * Cfg::SLOT_BYTES, 1024, 1024);
+            const uint64_t v_desc = ptx::make_smem_desc_sw128(smem_ring + slot * Cfg::SLOT_BYTES, 1024, v_lbo);
             uint32_t lm[4];
             att_slot_mask(sl, nslots, lm);
 #pragma unroll
             for (int t = 0; t < (SPLIT ? 3 : 1); ++t) {
-              const uint32_t pa = tmem_base + ATT_P_COL + (t == 2 ? 64 : 0);
-              const uint64_t va = ptx::desc_advance(v_desc, t == 1 ? ATT_TILE_BYTES : 0);
+              const uint32_t pa = tmem_base + Cfg::P_COL + (t == 2 ? 64 : 0);
+              const uint64_t va = ptx::desc_advance(v_desc, t == 1 ? Cfg::PART_BYTES : 0);
 #pragma unroll 1
               for (int k = 0; k < ksteps; ++k)
                 ptx::umma_bf16_ts_masked(o_tmem, pa + k * 8, ptx::desc_advance(va, k * 2048), idesc, (t | k) ? 1u : acc0, lm);
@@ -484,13 +507,13 @@ attn_fwd_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __gr
       att_stamp(args, tl && warp == 0, 0, j, 3);   // scale known
       auto rescale_o = [&](float a) {
 #pragma unroll
-        for (int c = 0; c < ATT_DH; c += 32) {
+        for (int c = 0; c < DH; c += 32) {
           uint32_t t[32];
-          ptx::tmem_ld_32x32b_x32(lane_addr + ATT_O_COL + c, t);
+          ptx::tmem_ld_32x32b_x32(lane_addr + Cfg::O_COL + c, t);
           ptx::tmem_ld_wait(t);
 #pragma unroll
           for (int i = 0; i < 32; ++i) t[i] = __float_as_uint(__uint_as_float(t[i]) * a);
-          ptx::tmem_st_32x32b_x32(lane_addr + ATT_O_COL + c, t);
+          ptx::tmem_st_32x32b_x32(lane_addr + Cfg::O_COL + c, t);
         }
       };
       if (j > 0) {
@@ -528,8 +551,8 @@ attn_fwd_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __gr
               ph[i] = ptx::pack_h2<F16>(e0, e1);
               if (SPLIT) pl[i] = ptx::pack_h2<F16>(e0 - ptx::round_h<F16>(e0), e1 - ptx::round_h<F16>(e1));
             }
-            ptx::tmem_st_32x32b_x16(lane_addr + ATT_P_COL + c * 16, ph);
-            if (SPLIT) ptx::tmem_st_32x32b_x16(lane_addr + ATT_P_COL + 64 + c * 16, pl);
+            ptx::tmem_st_32x32b_x16(lane_addr + Cfg::P_COL + c * 16, ph);
+            if (SPLIT) ptx::tmem_st_32x32b_x16(lane_addr + Cfg::P_COL + 64 + c * 16, pl);
           }
         }
       };
@@ -605,33 +628,39 @@ attn_fwd_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __gr
       lrow[qrow] = qrow < N ? m_used * sl2 + log2f(l_run) : INFINITY;
       for (int k = slot_rows; k < ATT_BQ; k += slot_rows) lrow[qrow + k] = INFINITY;   // packed item: the rest of the pad rows
     }
-    __nv_bfloat16* o = args.out + static_cast<long long>(row_base + qrow) * args.ldo + h * ATT_DH;
-    uint32_t t[ATT_DH / 32][32];
+    __nv_bfloat16* o = args.out + static_cast<long long>(row_base + qrow) * args.ldo + h * DH;
+    // 64 columns of O (64 registers) per pass: all 128 columns of head_dim 128 at once would spill
 #pragma unroll
-    for (int c = 0; c < ATT_DH / 32; ++c) ptx::tmem_ld_32x32b_x32(lane_addr + ATT_O_COL + c * 32, t[c]);
+    for (int ps = 0; ps < DH / 64; ++ps) {
+      uint32_t t[2][32];
 #pragma unroll
-    for (int c = 0; c < ATT_DH / 32; ++c) ptx::tmem_ld_wait(t[c]);
-    // O is in registers: the MMA warp may start accumulating the next work item into the same columns
-    ptx::tc_fence_before();
-    __syncwarp();
-    if (lane == 0) ptx::mbar_arrive(o_empty);
-    if (qrow < N && pair_ok) {
+      for (int c = 0; c < 2; ++c) ptx::tmem_ld_32x32b_x32(lane_addr + Cfg::O_COL + ps * 64 + c * 32, t[c]);
 #pragma unroll
-      for (int c = 0; c < ATT_DH / 32; ++c) {
+      for (int c = 0; c < 2; ++c) ptx::tmem_ld_wait(t[c]);
+      if (ps == DH / 64 - 1) {
+        // O is in registers: the MMA warp may start accumulating the next work item into the same columns
+        ptx::tc_fence_before();
+        __syncwarp();
+        if (lane == 0) ptx::mbar_arrive(o_empty);
+      }
+      if (qrow < N && pair_ok) {
 #pragma unroll
-        for (int q4 = 0; q4 < 4; ++q4) {
-          float v[8];
+        for (int c = 0; c < 2; ++c) {
 #pragma unroll
-          for (int i = 0; i < 8; ++i) v[i] = __uint_as_float(t[c][8 * q4 + i]) * inv;
-          reinterpret_cast<uint4*>(o + c * 32)[q4] = make_uint4(ptx::pack_h2<F16>(v[0], v[1]), ptx::pack_h2<F16>(v[2], v[3]),
-                                                               ptx::pack_h2<F16>(v[4], v[5]), ptx::pack_h2<F16>(v[6], v[7]));
-          if (SPLIT) {
-            float lo[8];
+          for (int q4 = 0; q4 < 4; ++q4) {
+            float v[8];
 #pragma unroll
-            for (int i = 0; i < 8; ++i) lo[i] = v[i] - ptx::round_h<F16>(v[i]);
-            reinterpret_cast<uint4*>(o + args.out_lo_off + c * 32)[q4] =
-                make_uint4(ptx::pack_h2<F16>(lo[0], lo[1]), ptx::pack_h2<F16>(lo[2], lo[3]), ptx::pack_h2<F16>(lo[4], lo[5]),
-                           ptx::pack_h2<F16>(lo[6], lo[7]));
+            for (int i = 0; i < 8; ++i) v[i] = __uint_as_float(t[c][8 * q4 + i]) * inv;
+            reinterpret_cast<uint4*>(o + ps * 64 + c * 32)[q4] = make_uint4(ptx::pack_h2<F16>(v[0], v[1]), ptx::pack_h2<F16>(v[2], v[3]),
+                                                                            ptx::pack_h2<F16>(v[4], v[5]), ptx::pack_h2<F16>(v[6], v[7]));
+            if (SPLIT) {
+              float lo[8];
+#pragma unroll
+              for (int i = 0; i < 8; ++i) lo[i] = v[i] - ptx::round_h<F16>(v[i]);
+              reinterpret_cast<uint4*>(o + args.out_lo_off + ps * 64 + c * 32)[q4] =
+                  make_uint4(ptx::pack_h2<F16>(lo[0], lo[1]), ptx::pack_h2<F16>(lo[2], lo[3]), ptx::pack_h2<F16>(lo[4], lo[5]),
+                             ptx::pack_h2<F16>(lo[6], lo[7]));
+            }
           }
         }
       }

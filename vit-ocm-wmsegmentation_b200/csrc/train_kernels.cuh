@@ -129,9 +129,9 @@ ln_bwd_kernel(const float* __restrict__ x, const __nv_bfloat16* __restrict__ dy,
 }
 
 // ------------------------------------------------------------------------------------------------ attention backward helpers
-// delta[b][h][q] (row pitch npad) = sum_d dO[row][h*64 + d] * O[row][h*64 + d]; one warp per token row, two bf16 per lane per
-// head; all heads' loads are issued before the first reduction (HG heads at a time) so that a row costs one memory latency
-template <int HG>
+// delta[b][h][q] (row pitch npad) = sum_d dO[row][h*DH + d] * O[row][h*DH + d]; one warp per token row, DH / 32 bf16 per lane
+// per head; all heads' loads are issued before the first reduction (HG heads at a time) so that a row costs one memory latency
+template <int HG, int DH = 64>
 __global__ void __launch_bounds__(256)
 attn_delta_kernel(const __nv_bfloat16* __restrict__ O, const __nv_bfloat16* __restrict__ dO, long long ld, float* __restrict__ delta,
                   int B, int N, int heads, int npad) {
@@ -141,18 +141,25 @@ attn_delta_kernel(const __nv_bfloat16* __restrict__ O, const __nv_bfloat16* __re
        row += static_cast<long long>(gridDim.x) * (blockDim.x >> 5)) {
     const int b = static_cast<int>(row / N), q = static_cast<int>(row - static_cast<long long>(b) * N);
     for (int h0 = 0; h0 < heads; h0 += HG) {
-      uint32_t o[HG], d[HG];
+      constexpr int W = DH / 64;   // 32-bit words (bf16 pairs) per lane and head
+      uint32_t o[HG][W], d[HG][W];
 #pragma unroll
       for (int k = 0; k < HG; ++k) {
         if (h0 + k < heads) {
-          o[k] = *reinterpret_cast<const uint32_t*>(O + row * ld + (h0 + k) * 64 + 2 * lane);
-          d[k] = *reinterpret_cast<const uint32_t*>(dO + row * ld + (h0 + k) * 64 + 2 * lane);
+#pragma unroll
+          for (int u = 0; u < W; ++u) {
+            o[k][u] = *reinterpret_cast<const uint32_t*>(O + row * ld + (h0 + k) * DH + 2 * (W * lane + u));
+            d[k][u] = *reinterpret_cast<const uint32_t*>(dO + row * ld + (h0 + k) * DH + 2 * (W * lane + u));
+          }
         }
       }
 #pragma unroll
       for (int k = 0; k < HG; ++k) {
         if (h0 + k < heads) {
-          const float s = warp_sum(bf16lo(o[k]) * bf16lo(d[k]) + bf16hi(o[k]) * bf16hi(d[k]));
+          float p = bf16lo(o[k][0]) * bf16lo(d[k][0]) + bf16hi(o[k][0]) * bf16hi(d[k][0]);
+#pragma unroll
+          for (int u = 1; u < W; ++u) p += bf16lo(o[k][u]) * bf16lo(d[k][u]) + bf16hi(o[k][u]) * bf16hi(d[k][u]);
+          const float s = warp_sum(p);
           if (lane == 0) delta[(static_cast<long long>(b) * heads + h0 + k) * npad + q] = s;
         }
       }

@@ -114,19 +114,20 @@ layernorm_kernel(const float* __restrict__ x, const float* __restrict__ gamma, c
 // Last block, CLS query only (the slice every hot-path caller reads, SSS/utils.py:232 with
 // query = 0): one block per (head, image):
 //   xn  = LayerNorm(X[b, 0, :])                       (fp32)
-//   q_h = Wq[h*64:(h+1)*64, :] . xn + bq              (fp32 weights, fp32 math)
-//   out[b, h, j] = softmax_j( scale * q_h . K[b, j, h*64:(h+1)*64] )   for j in [0, N)
-// K comes from the (split-precision) K-projection GEMM as fp32 [B*N, D].
+//   q_h = Wq[h*DH:(h+1)*DH, :] . xn + bq              (fp32 weights, fp32 math)
+//   out[b, h, j] = softmax_j( scale * q_h . K[b, j, h*DH:(h+1)*DH] )   for j in [0, N)
+// K comes from the (split-precision) K-projection GEMM as fp32 [B*N, D].  DH = head_dim (64 or 128).
 // ---------------------------------------------------------------------------------------
+template <int DH>
 __global__ void __launch_bounds__(256)
 cls_attn_row_kernel(const float* __restrict__ X, const float* __restrict__ ln_w, const float* __restrict__ ln_b, float eps,
                     const float* __restrict__ Wq /*[D][D] rows = q outputs*/, const float* __restrict__ bq,
                     const float* __restrict__ Kmat /*[B*N][D] fp32*/, float* __restrict__ out /*[B][H][nq][N]*/, int N, int D,
                     int heads, float scale, const int* __restrict__ queries /*[nq] token indices or nullptr = {0}*/, int nq) {
-  extern __shared__ float cls_smem[];  // xn[D] | q[64] | logits[N] | red[32]
+  extern __shared__ float cls_smem[];  // xn[D] | q[DH] | logits[N] | red[32]
   float* xn = cls_smem;
   float* qv = xn + D;
-  float* logits = qv + 64;
+  float* logits = qv + DH;
   float* red = logits + N;
   const int h = blockIdx.x, b = blockIdx.y;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, nwarps = blockDim.x >> 5;
@@ -158,24 +159,34 @@ cls_attn_row_kernel(const float* __restrict__ X, const float* __restrict__ ln_w,
   for (int d = tid; d < D; d += blockDim.x) xn[d] = (xr[d] - mean) * rstd * ln_w[d] + ln_b[d];
   __syncthreads();
 
-  // q_h: 64 outputs, one warp per output (coalesced weight rows)
-  for (int o = warp; o < 64; o += nwarps) {
-    const float* wr = Wq + static_cast<long long>(h * 64 + o) * D;
+  // q_h: DH outputs, one warp per output (coalesced weight rows)
+  for (int o = warp; o < DH; o += nwarps) {
+    const float* wr = Wq + static_cast<long long>(h * DH + o) * D;
     float acc = 0.f;
     for (int d = lane; d < D; d += 32) acc = fmaf(wr[d], xn[d], acc);
     acc = warp_sum(acc);
-    if (lane == 0) qv[o] = acc + bq[h * 64 + o];
+    if (lane == 0) qv[o] = acc + bq[h * DH + o];
   }
   __syncthreads();
 
-  // logits: one warp per key, two channels per lane
-  const float q0 = qv[2 * lane], q1 = qv[2 * lane + 1];
+  // logits: one warp per key, DH / 32 channels per lane
   float lmax = -INFINITY;
-  for (int j = warp; j < N; j += nwarps) {
-    const float2 kk = *reinterpret_cast<const float2*>(Kmat + (static_cast<long long>(b) * N + j) * D + h * 64 + 2 * lane);
-    float acc = warp_sum(fmaf(q0, kk.x, q1 * kk.y)) * scale;
-    if (lane == 0) logits[j] = acc;
-    lmax = fmaxf(lmax, acc);
+  if constexpr (DH == 64) {
+    const float q0 = qv[2 * lane], q1 = qv[2 * lane + 1];
+    for (int j = warp; j < N; j += nwarps) {
+      const float2 kk = *reinterpret_cast<const float2*>(Kmat + (static_cast<long long>(b) * N + j) * D + h * 64 + 2 * lane);
+      float acc = warp_sum(fmaf(q0, kk.x, q1 * kk.y)) * scale;
+      if (lane == 0) logits[j] = acc;
+      lmax = fmaxf(lmax, acc);
+    }
+  } else {
+    const float4 qq = reinterpret_cast<const float4*>(qv)[lane];
+    for (int j = warp; j < N; j += nwarps) {
+      const float4 kk = *reinterpret_cast<const float4*>(Kmat + (static_cast<long long>(b) * N + j) * D + h * DH + 4 * lane);
+      float acc = warp_sum(fmaf(qq.x, kk.x, fmaf(qq.y, kk.y, fmaf(qq.z, kk.z, qq.w * kk.w)))) * scale;
+      if (lane == 0) logits[j] = acc;
+      lmax = fmaxf(lmax, acc);
+    }
   }
   if (lane == 0) red[warp] = lmax;
   __syncthreads();
@@ -202,42 +213,45 @@ cls_attn_row_kernel(const float* __restrict__ X, const float* __restrict__ ln_w,
 // Full attention probabilities of one block, fp32 math on CUDA cores (API-complete path for
 // get_last_selfattention / get_intermediate_feat; the hot path never materialises N x N).
 // Reads q and k from an fp32 [B*N, 3D] activation.  One block = (qrows-query group, head, image);
-// K_h is staged once per block in smem as fp32 with a padded row (65 floats) so that the
-// lane-per-key dot products are bank-conflict free.
+// K_h is staged once per block in smem as fp32 with a padded row (DH + 1 floats) so that the
+// lane-per-key dot products are bank-conflict free.  DH = head_dim (64 or 128).
 // ---------------------------------------------------------------------------------------
 constexpr int AP_QROWS = 16;
 
+template <int DH>
 __global__ void __launch_bounds__(256)
 attn_probs_kernel(const float* __restrict__ qkv /*[B*N][3D]*/, float* __restrict__ attn /*[B][H][N][N]*/, int N, int D,
                   int heads, float scale, int kchunk /*keys staged per pass*/, int qrows) {
-  extern __shared__ float ap_smem[];  // K chunk [kchunk][65] | q [qrows][64] | logits [qrows][N]
+  extern __shared__ float ap_smem[];  // K chunk [kchunk][DH + 1] | q [qrows][DH] | logits [qrows][N]
+  constexpr int KP = DH + 1;
   float* ks = ap_smem;
-  float* qs = ks + kchunk * 65;
-  float* lg = qs + qrows * 64;
+  float* qs = ks + kchunk * KP;
+  float* lg = qs + qrows * DH;
   const int q0 = blockIdx.x * qrows, h = blockIdx.y, b = blockIdx.z;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, nwarps = blockDim.x >> 5;
   const long long ld = 3LL * D;
   const float* base = qkv + static_cast<long long>(b) * N * ld;
-  for (int i = tid; i < qrows * 64; i += blockDim.x) {
-    const int r = i >> 6, c = i & 63;
-    qs[i] = (q0 + r < N) ? base[(q0 + r) * ld + h * 64 + c] : 0.f;
+  constexpr int LOG_DH = DH == 64 ? 6 : 7;
+  for (int i = tid; i < qrows * DH; i += blockDim.x) {
+    const int r = i >> LOG_DH, c = i & (DH - 1);
+    qs[i] = (q0 + r < N) ? base[(q0 + r) * ld + h * DH + c] : 0.f;
   }
   for (int k0 = 0; k0 < N; k0 += kchunk) {
     const int kn = min(kchunk, N - k0);
     __syncthreads();
-    for (int i = tid; i < kn * 64; i += blockDim.x) {
-      const int r = i >> 6, c = i & 63;
-      ks[r * 65 + c] = base[(k0 + r) * ld + D + h * 64 + c];
+    for (int i = tid; i < kn * DH; i += blockDim.x) {
+      const int r = i >> LOG_DH, c = i & (DH - 1);
+      ks[r * KP + c] = base[(k0 + r) * ld + D + h * DH + c];
     }
     __syncthreads();
     // each warp: 2 query rows; lane-per-key
     for (int r = warp; r < qrows; r += nwarps) {
-      const float* qr = qs + r * 64;
+      const float* qr = qs + r * DH;
       for (int j = lane; j < kn; j += 32) {
-        const float* kr = ks + j * 65;
+        const float* kr = ks + j * KP;
         float acc = 0.f;
 #pragma unroll 16
-        for (int c = 0; c < 64; ++c) acc = fmaf(qr[c], kr[c], acc);
+        for (int c = 0; c < DH; ++c) acc = fmaf(qr[c], kr[c], acc);
         lg[r * N + k0 + j] = acc * scale;
       }
     }

@@ -639,6 +639,7 @@ int run_block_tail(const vitocm_engine* e, const void* CTX, long long ld_ctx, co
 int run_attention(const vitocm_engine* e, const void* qkv, long long ld, int B, int N, void* ctx, long long ldo, cudaStream_t st,
                   long long* timeline = nullptr, float* lse2 = nullptr) {
   const int D = e->cfg.embed_dim, H = e->cfg.num_heads;
+  const bool hd128 = D == 128 * H;   // head_dim 128: the generic kernel's DH = 128 instantiations (no four-pipeline kernel)
   const long long M = static_cast<long long>(B) * N;
   ProfScope prof(PC_ATTN, st);
   CUtensorMap tq, tq32;
@@ -665,7 +666,7 @@ int run_attention(const vitocm_engine* e, const void* qkv, long long ld, int B, 
   // 16-bit engines, inference: the full query tiles go through the four-pipeline kernel (attention_quad_sm100.cuh), the ragged
   // tails through the packed items of the kernel below (VITOCM_ATTN_QUAD=0: everything through the kernel below)
   static const int quad = [] { const char* v = getenv("VITOCM_ATTN_QUAD"); return v ? atoi(v) : 1; }();
-  if (quad && !e->split && lse2 == nullptr && a.n_fullq >= 1) {
+  if (quad && !hd128 && !e->split && lse2 == nullptr && a.n_fullq >= 1) {
     const long long full_items = static_cast<long long>(a.n_pairs) * a.n_fullq;
     if (full_items > 0x7fffffffLL) return fail(VITOCM_ERR_INVALID, "attention: too many work items");
     AttnArgs aq = a;
@@ -706,8 +707,8 @@ int run_attention(const vitocm_engine* e, const void* qkv, long long ld, int B, 
     a.timeline = nullptr;   // (the stamps of a timeline call come from the four-pipeline kernel)
     a.n_items = (a.n_pairs + a.pack - 1) / a.pack;
   }
-  // persistent CTAs: as many as are co-resident (2 per SM in bf16 mode, 1 in split mode)
-  const int resident = e->num_sms * (e->split ? 1 : 2);
+  // persistent CTAs: as many as are co-resident (2 per SM in bf16 mode at head_dim 64, 1 in split mode or at head_dim 128)
+  const int resident = e->num_sms * ((e->split || hd128) ? 1 : 2);
   static const int persist = [] { const char* v = getenv("VITOCM_ATTN_PERSISTENT"); return v ? atoi(v) : 1; }();
   const dim3 grid(persist && a.n_items > resident ? resident : a.n_items);
   auto launch = [&](auto kern, int smem_bytes, bool& attr) -> int {
@@ -716,6 +717,24 @@ int run_attention(const vitocm_engine* e, const void* qkv, long long ld, int B, 
     return 0;
   };
   // (the FMA-pipe exp2 polynomial variants of round 1 measured 15-19 % slower and are no longer instantiated)
+  if (hd128) {
+    static bool attr128[8] = {false, false, false, false, false, false, false, false};
+    if (a.pack > 1) {
+      if (e->split) {
+        if (e->f16) TRY(launch(attn_fwd_tcgen05_kernel<true, 0u, true, true, 128>, AttnCfg<true, 128>::SMEM_BYTES, attr128[1]));
+        else TRY(launch(attn_fwd_tcgen05_kernel<true, 0u, true, false, 128>, AttnCfg<true, 128>::SMEM_BYTES, attr128[3]));
+      } else if (e->f16) TRY(launch(attn_fwd_tcgen05_kernel<false, 0u, true, true, 128>, AttnCfg<false, 128>::SMEM_BYTES, attr128[2]));
+      else TRY(launch(attn_fwd_tcgen05_kernel<false, 0u, true, false, 128>, AttnCfg<false, 128>::SMEM_BYTES, attr128[0]));
+    } else {
+      if (e->split) {
+        if (e->f16) TRY(launch(attn_fwd_tcgen05_kernel<true, 0u, false, true, 128>, AttnCfg<true, 128>::SMEM_BYTES, attr128[5]));
+        else TRY(launch(attn_fwd_tcgen05_kernel<true, 0u, false, false, 128>, AttnCfg<true, 128>::SMEM_BYTES, attr128[7]));
+      } else if (e->f16) TRY(launch(attn_fwd_tcgen05_kernel<false, 0u, false, true, 128>, AttnCfg<false, 128>::SMEM_BYTES, attr128[6]));
+      else TRY(launch(attn_fwd_tcgen05_kernel<false, 0u, false, false, 128>, AttnCfg<false, 128>::SMEM_BYTES, attr128[4]));
+    }
+    LAUNCH_CHECK();
+    return 0;
+  }
   static bool attr[8] = {false, false, false, false, false, false, false, false};
   if (a.pack > 1) {   // kernels with the packed-item logic
     if (e->split) {
@@ -946,8 +965,8 @@ int vitocm_profile_read(double* ms, int64_t* counts, int nclasses) {
 
 int vitocm_create(const vitocm_config* cfg, vitocm_engine** out) {
   if (cfg == nullptr || out == nullptr) return fail(VITOCM_ERR_INVALID, "null argument");
-  if (cfg->num_heads <= 0 || cfg->embed_dim != cfg->num_heads * 64)
-    return fail(VITOCM_ERR_INVALID, "head_dim must be 64 (embed_dim %d, heads %d)", cfg->embed_dim, cfg->num_heads);
+  if (cfg->num_heads <= 0 || (cfg->embed_dim != cfg->num_heads * 64 && cfg->embed_dim != cfg->num_heads * 128))
+    return fail(VITOCM_ERR_INVALID, "head_dim (embed_dim / num_heads) must be 64 or 128 (embed_dim %d, heads %d)", cfg->embed_dim, cfg->num_heads);
   if (cfg->mlp_hidden % 64 != 0 || cfg->depth < 1) return fail(VITOCM_ERR_INVALID, "bad mlp_hidden/depth");
   if (cfg->precision != VITOCM_BF16 && cfg->precision != VITOCM_FP32 && cfg->precision != VITOCM_FP16) return fail(VITOCM_ERR_INVALID, "bad precision");
   int dev = 0;
@@ -1224,11 +1243,13 @@ static int forward_rows(vitocm_engine* e, const float* x, int B, int H, int W, c
   const int n_chunks = (B + chunk_tiles - 1) / chunk_tiles;
   if (lanes > n_chunks) lanes = n_chunks;
   const LayerW& last = e->layers[e->cfg.depth - 1];
-  const size_t cls_smem = static_cast<size_t>(D + 64 + N + 32) * sizeof(float);
-  static size_t cls_smem_set = 0;
-  if (cls_smem > 48 * 1024 && cls_smem > cls_smem_set) {
-    CUDA_TRY(cudaFuncSetAttribute(cls_attn_row_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(cls_smem)));
-    cls_smem_set = cls_smem;
+  const int dh = D / heads;
+  const size_t cls_smem = static_cast<size_t>(D + dh + N + 32) * sizeof(float);
+  static size_t cls_smem_set[2] = {0, 0};
+  if (cls_smem > 48 * 1024 && cls_smem > cls_smem_set[dh == 128]) {
+    if (dh == 128) CUDA_TRY(cudaFuncSetAttribute(cls_attn_row_kernel<128>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(cls_smem)));
+    else CUDA_TRY(cudaFuncSetAttribute(cls_attn_row_kernel<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(cls_smem)));
+    cls_smem_set[dh == 128] = cls_smem;
   }
   cudaStream_t lane_st[vitocm_engine::MAX_LANES];
   Workspace lane_ws[vitocm_engine::MAX_LANES];
@@ -1281,9 +1302,9 @@ static int forward_rows(vitocm_engine* e, const float* x, int B, int H, int W, c
       TRY(run_gemm(e, wsp.XN, 2LL * D, last.wk_split.p, 2LL * D, M, D, D, 1, EPI_BIAS_F32, last.bqkv + D, KF, D, 0, 0, lane_st[k], PC_GEMM_KLAST));
       ProfScope prof(PC_CLSROW, lane_st[k]);
       dim3 grid(heads, bcs[k], nq);
-      cls_attn_row_kernel<<<grid, 256, cls_smem, lane_st[k]>>>(wsp.X, last.ln1w, last.ln1b, e->cfg.ln_eps, last.wqkv_f32, last.bqkv, KF,
-                                                               out_rows + static_cast<long long>(b0s[k]) * heads * nq * N, N, D, heads, e->cfg.qk_scale,
-                                                               queries, nq);
+      (dh == 128 ? cls_attn_row_kernel<128> : cls_attn_row_kernel<64>)<<<grid, 256, cls_smem, lane_st[k]>>>(
+          wsp.X, last.ln1w, last.ln1b, e->cfg.ln_eps, last.wqkv_f32, last.bqkv, KF, out_rows + static_cast<long long>(b0s[k]) * heads * nq * N,
+          N, D, heads, e->cfg.qk_scale, queries, nq);
       LAUNCH_CHECK();
       if (k_out != nullptr)   // last-block K features (SSS/analyse_attention.py:139-163, SSS/eval.py:186-202 cluster these)
         CUDA_TRY(cudaMemcpyAsync(k_out + static_cast<long long>(b0s[k]) * N * D, KF, static_cast<size_t>(M) * D * sizeof(float), cudaMemcpyDeviceToDevice,
@@ -1323,19 +1344,21 @@ int vitocm_block_attn_probs(vitocm_engine* e, int layer, const float* X, int B, 
   const int M = B * N;
   TRY(run_layernorm(X, L.ln1w, L.ln1b, wsp.XN, 2LL * D, S, D, nullptr, 0, M, D, e->cfg.ln_eps, st, nullptr, e->f16));
   TRY(run_gemm(e, wsp.XN, 2LL * D, L.wqkv.p, static_cast<long long>(D) * P, M, 3 * D, D, S, EPI_BIAS_F32, L.bqkv, qkv_out, 3LL * D, 0, 0, st));
-  const int kchunk = 256;
+  const int dh = D / heads;
+  const int kchunk = dh == 128 ? 128 : 256;
   int qrows = AP_QROWS;
-  auto smem_for = [&](int qr) { return static_cast<size_t>(kchunk * 65 + qr * 64 + static_cast<size_t>(qr) * N) * sizeof(float); };
+  auto smem_for = [&](int qr) { return static_cast<size_t>(kchunk * (dh + 1) + qr * dh + static_cast<size_t>(qr) * N) * sizeof(float); };
   while (qrows > 1 && smem_for(qrows) > 200 * 1024) qrows >>= 1;
   const size_t smem = smem_for(qrows);
   if (smem > 220 * 1024) return fail(VITOCM_ERR_INVALID, "n_tokens=%d too large for attn_probs", N);
-  static size_t smem_set = 0;
-  if (smem > smem_set) {
-    CUDA_TRY(cudaFuncSetAttribute(attn_probs_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
-    smem_set = smem;
+  static size_t smem_set[2] = {0, 0};
+  if (smem > smem_set[dh == 128]) {
+    if (dh == 128) CUDA_TRY(cudaFuncSetAttribute(attn_probs_kernel<128>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
+    else CUDA_TRY(cudaFuncSetAttribute(attn_probs_kernel<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
+    smem_set[dh == 128] = smem;
   }
   dim3 grid((N + qrows - 1) / qrows, heads, B);
-  attn_probs_kernel<<<grid, 256, smem, st>>>(qkv_out, attn, N, D, heads, e->cfg.qk_scale, kchunk, qrows);
+  (dh == 128 ? attn_probs_kernel<128> : attn_probs_kernel<64>)<<<grid, 256, smem, st>>>(qkv_out, attn, N, D, heads, e->cfg.qk_scale, kchunk, qrows);
   LAUNCH_CHECK();
   return 0;
 }

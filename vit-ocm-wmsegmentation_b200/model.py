@@ -388,9 +388,9 @@ class MIM(nn.Module):
 
 
 def build_model(args, depth=12, num_heads=6, precision="bf16"):
-    """SSS/model.py:91-108.  The reference currently hard-codes an experimental depth=4 / num_heads=3 (head_dim 128);
-    the shipped training log (SSS/output/log_rank0.txt) is the 12-block, 6-head ViT-S/8 used here by default --
-    the kernels are specialised for head_dim 64."""
+    """SSS/model.py:91-108.  The reference's build_model hard-codes depth=4 / num_heads=3 at embed_dim 384 (head_dim 128):
+    ``build_model(args, depth=4, num_heads=3)`` builds exactly that encoder.  The defaults (12 blocks, 6 heads, head_dim 64)
+    are the ViT-S/8 of the shipped training log (SSS/output/log_rank0.txt)."""
     return VisionTransformerForSimMIM(patch_size=args.MODEL.PATCH_SIZE, embed_dim=384, depth=depth, num_heads=num_heads,
                                       mlp_ratio=4, img_size=[args.DATA.IMG_SIZE], qkv_bias=True,
                                       norm_layer=partial(nn.LayerNorm, eps=1e-6), interpolate_encoding=True,

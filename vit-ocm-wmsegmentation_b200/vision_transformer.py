@@ -172,8 +172,9 @@ class VisionTransformer(nn.Module):
         super().__init__()
         if drop_rate or attn_drop_rate or drop_path_rate:
             raise NotImplementedError("vitocm: dropout / drop-path rates must be 0 on this path")
-        if embed_dim % num_heads or embed_dim // num_heads != 64:
-            raise NotImplementedError("vitocm kernels are specialised for head_dim 64")
+        if embed_dim % num_heads or embed_dim // num_heads not in (64, 128):
+            raise NotImplementedError("vitocm kernels support head_dim 64 and 128 (embed_dim %d / num_heads %d)"
+                                      % (embed_dim, num_heads))
         parse_precision(precision, depth)
         self.num_features = self.embed_dim = embed_dim
         self.num_heads = num_heads
@@ -403,7 +404,7 @@ class VisionTransformer(nn.Module):
     def attention_rows(self, x: torch.Tensor, queries, return_keys: bool = False):
         """get_last_selfattention(x)[:, :, queries, :] -> [B, heads, nq, N] fp32 for a list of query tokens (0 = CLS,
         1 + i = patch i; SSS/analyse_attention.py:183-247 region queries), without forming N x N.  With ``return_keys``
-        also the last block's K features [B, heads, N, 64] (= qkv[1] of get_intermediate_feat; SSS/eval.py:186-202)."""
+        also the last block's K features [B, heads, N, head_dim] (= qkv[1] of get_intermediate_feat; SSS/eval.py:186-202)."""
         x = self._check_input(x)
         eng = self._ensure_engine()
         B, _, H, W = x.shape
