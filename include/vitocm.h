@@ -284,10 +284,11 @@ int vitocm_attention_timeline(vitocm_engine* e, const void* qkv, int64_t ld, int
 /* LayerNorm rows of X [M][D] fp32 with affine (gamma, beta) -> out bf16 [M][ldo] (hi | lo if split). */
 int vitocm_layernorm(vitocm_engine* e, const float* X, const float* gamma, const float* beta, void* out_bf16,
                      int64_t ldo, int split, int lo_off, int M, void* stream);
-/* ---- MIM training step (SSS/mim.py:153-182; model.py:71-77 under autograd).  bf16 engines only. ---- */
+/* ---- MIM training step (SSS/mim.py:153-182; model.py:71-77 under autograd).  16-bit engines: VITOCM_BF16 or VITOCM_FP16
+ * (the fp32-parity mode is refused). ---- */
 
 /* Master weights owned by the caller (training): `name` as in vitocm_load_weight, dev_data = DEVICE fp32, 16-byte aligned,
- * used in place (no copy) -- an optimizer updates it and vitocm_refresh_weights repacks the bf16 operand copies on
+ * used in place (no copy) -- an optimizer updates it and vitocm_refresh_weights repacks the 16-bit operand copies (the engine's format) on
  * `stream` without synchronising.  The first use still needs one vitocm_finalize_weights. */
 int vitocm_bind_weight(vitocm_engine* e, const char* name, float* dev_data, int64_t numel);
 int vitocm_refresh_weights(vitocm_engine* e, void* stream);
@@ -302,7 +303,12 @@ int vitocm_mim_train_forward(vitocm_engine* e, const float* x, int B, int H, int
                              float* x_rec, double* loss_sums, void* ws, size_t ws_bytes, void* stream);
 /* loss.backward() (mim.py:174) for the batch vitocm_mim_train_forward just ran on the same ws: gradients of
  * (*grad_scale) * loss (grad_scale = DEVICE pointer to the upstream gradient of the scalar loss, NULL = 1) are accumulated into the buffers bound with vitocm_bind_grad (all parameters except pos_embed);
- * dpos [N][D] fp32 is WRITTEN with the gradient of the (interpolated) position table passed to the forward. */
+ * dpos [N][D] fp32 is WRITTEN with the gradient of the (interpolated) position table passed to the forward.
+ * Loss scale (fp16 engines): fp16's range would flush the loss gradient (~4e-7 at batch 32, 224^2) towards zero, so the backward
+ * runs on gradients multiplied by S = 2^e, chosen on the device (no host sync) from the exponent of the loss gradient
+ * *grad_scale / (3 (sum(mask) + 1e-5)) so that its magnitude times S lies in [1, 2); S = 1 if that is 0.  S and 1 / S are kept in
+ * 8 bytes of ws.  Every parameter gradient and dpos are multiplied by 1 / S before they are written or accumulated, which is
+ * exact: callers see the unscaled gradients, and a power-of-two grad_scale scales them exactly.  bf16 engines use no scale. */
 int vitocm_mim_backward(vitocm_engine* e, const float* x, int B, int H, int W, const float* mask, const float* x_rec,
                         const double* loss_sums, const float* grad_scale, float* dpos, void* ws, size_t ws_bytes, void* stream);
 
@@ -327,7 +333,8 @@ int vitocm_grad_clip(float* g, int64_t n, float max_norm, const double* sumsq, v
 int vitocm_adamw_step(float* p, float* g, float* m, float* v, const uint8_t* decay, int64_t n, float lr, float beta1, float beta2,
                       float eps, float weight_decay, int step, float max_norm, float grad_scale, const double* sumsq, void* stream);
 
-/* kernel-level: dW[R][C] (fp32) += G[M][R]^T . A[M][C], bf16 row-major activations (the weight gradient of nn.Linear);
+/* kernel-level: dW[R][C] (fp32) += G[M][R]^T . A[M][C], 16-bit row-major activations in the engine's format (bf16 or fp16; the weight
+ * gradient of nn.Linear);
  * db[R] (fp32, or NULL) += column sums of G (its bias gradient, computed by the same tensor-core pass) */
 int vitocm_wgrad(vitocm_engine* e, const void* G, int64_t ldg, const void* A, int64_t lda, int M, int R, int C, float* dW,
                  float* db, void* stream);
@@ -335,7 +342,8 @@ int vitocm_wgrad(vitocm_engine* e, const void* G, int64_t ldg, const void* A, in
  * multiple of 128, pad rows hold +inf */
 int vitocm_attention_fwd_lse(vitocm_engine* e, const void* qkv, int64_t ld, int B, int n_tokens, void* ctx, int64_t ldo,
                              float* lse2, void* stream);
-/* backward of vitocm_attention: dqkv bf16 [B*N][ldq] (columns [3][heads][head_dim]) from dctx; scratch: delta [B][heads][Npad] fp32,
+/* backward of vitocm_attention on bf16 or fp16 engines (operands and dqkv in the engine's format): dqkv [B*N][ldq] (columns
+ * [3][heads][head_dim]) from dctx; scratch: delta [B][heads][Npad] fp32,
  * dqacc [B*N][D] fp32 (zero on entry, zero again on return) */
 int vitocm_attention_bwd(vitocm_engine* e, const void* qkv, int64_t ld, const void* ctx, const void* dctx, int64_t ldc,
                          const float* lse2, float* delta, float* dqacc, void* dqkv, int64_t ldq, int B, int n_tokens,

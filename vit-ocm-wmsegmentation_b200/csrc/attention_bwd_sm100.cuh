@@ -12,20 +12,21 @@
 // double-buffered K/V slot and TMEM live across items, so the next item's K/V arrive under the current item's last tiles
 // and its first S / dP MMAs run while dK_j / dV_j are drained.  Per (i, j):
 //   MMA   S  = Q_i K_j^T, dP = dO_i V_j^T                    (K-major operands)            -> TMEM S | dP
-//   warps 0..3 (thread = query row): tcgen05.ld S, dP -> P, dS (bf16) -> shared memory, row-major [q][k]
+//   warps 0..3 (thread = query row): tcgen05.ld S, dP -> P, dS (16-bit) -> shared memory, row-major [q][k]
 //   MMA   dV += P^T dO_i, dK += dS^T Q_i                     (A = P / dS read MN-major: the contraction runs over the
 //                                                             rows q; B = dO_i / Q_i MN-major)  -> TMEM dV | dK
 //   MMA   dQ_i = dS K_j                                      (A = dS K-major, B = K_j MN-major) -> TMEM dQ
 //   softmax warps: dQ tile -> shared memory -> TMA reduce-add (fp32, done by the L2) into dQacc[b, i*128.., h*64..];
 //               a 3-D tensor map [B][N][D] clips the rows beyond the image.
 // The same shared-memory image of P / dS serves as MN-major A (dV, dK) and as K-major A (dQ): no transposes.
-// dK_j, dV_j leave through registers as bf16 into the dQKV activation; dQacc is converted by dq_convert_kernel.
+// dK_j, dV_j leave through registers as 16-bit values into the dQKV activation; dQacc is converted by dq_convert_kernel.
 // Head_dim 128 (DH = 128): every item also names one 64-column half of the head, and dK / dV / dQ of that half are its only
 // outputs, so the TMEM map above (S 128 | dP 128 | dV 64 | dK 64 | dQ 64) and the drains stay as they are; S and dP contract over
 // all 128 columns (8 k-steps across the two swizzle atoms of every tile).  The two halves of a key block recompute the same
 // P / dS: twice the exponentials of one pass, against a 128-column dQ that has no room in TMEM next to 128-key S, dP, dV and dK.
 // A [128 x 128] tile is 32 KB, so K / V and Q / dO get one shared-memory slot each (211 KB in all) and the MMA warp issues the
 // next tile's S / dP only after the current tile's dV / dK / dQ (AbwCfg::ONE_SLOT): its operands land in the slot those free.
+// F16 = true: fp16 Q / K / V / dO operands (fp16 engines); P and dS are packed to fp16 with satfinite, dK / dV leave as fp16.
 // Warp roles: warps 0..7 softmax/drain (quadrant = warp % 4, key-column half = warp / 4: two warps per scheduler hide each
 // other's MUFU / TMEM latencies -- the backward needs no row reductions, so a row splits freely), warp 8 = TMA producer,
 // warp 9 = MMA issuer + TMEM allocator.  Ragged tails are trimmed: a short key block runs S / dP at N = 32 per 32 keys and
@@ -86,7 +87,7 @@ __device__ __forceinline__ void tma_reduce_add_3d(const CUtensorMap* tmap, uint3
                : "memory");
 }
 
-template <int DH = 64>
+template <int DH = 64, bool F16 = false>
 __global__ void __launch_bounds__(ABW_THREADS, 1)
 attn_bwd_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __grid_constant__ CUtensorMap tmap_do,
                         const __grid_constant__ CUtensorMap tmap_dq, const AttnBwdArgs args) {
@@ -197,8 +198,9 @@ attn_bwd_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __gr
   } else if (warp == ABW_MMA_WARP) {
     // ===================== MMA issuer =====================
     if (ptx::elect_one()) {
-      constexpr uint32_t idesc_t = ptx::make_idesc(128, 64, true, true);      // dV, dK: A (P / dS) and B (dO / Q) MN-major
-      constexpr uint32_t idesc_q = ptx::make_idesc(128, 64, false, true);     // dQ: A = dS K-major, B = K_j MN-major
+      constexpr uint32_t FMT = F16 ? 0u : 1u;
+      constexpr uint32_t idesc_t = ptx::make_idesc(128, 64, true, true, FMT);      // dV, dK: A (P / dS) and B (dO / Q) MN-major
+      constexpr uint32_t idesc_q = ptx::make_idesc(128, 64, false, true, FMT);     // dQ: A = dS K-major, B = K_j MN-major
       const uint64_t p_desc_mn = ptx::make_smem_desc_sw128(smem_p, 1024, ABW_TILE);    // 64-key atoms 16 KB apart
       const uint64_t ds_desc_mn = ptx::make_smem_desc_sw128(smem_ds, 1024, ABW_TILE);
       const uint64_t ds_desc_k = ptx::make_smem_desc_sw128(smem_ds, 1024, 0);
@@ -210,7 +212,7 @@ attn_bwd_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __gr
         if (i == 0) ptx::mbar_wait(kv_full + 8 * ks, (w >> (SLOTS - 1)) & 1, 42);
         ptx::mbar_wait(qdo_full + 8 * slot, (t >> (SLOTS - 1)) & 1, 41);
         ptx::tc_fence_after();
-        const uint32_t idesc_s = ptx::make_idesc(128, ((kv_len_of(j) + 31) >> 5) * 32, false, false);
+        const uint32_t idesc_s = ptx::make_idesc(128, ((kv_len_of(j) + 31) >> 5) * 32, false, false, FMT);
         const uint64_t k_desc = ptx::make_smem_desc_sw128(smem_kv + ks * 2 * TILE, 1024, 0);
         const uint64_t v_desc = ptx::desc_advance(k_desc, TILE);
         const uint64_t q_desc = ptx::make_smem_desc_sw128(smem_qdo + slot * 2 * TILE, 1024, 0);
@@ -367,15 +369,15 @@ attn_bwd_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __gr
 #pragma unroll
         for (int g = 0; g < 4; ++g) {
           reinterpret_cast<uint4*>(o)[g] =
-              make_uint4(ptx::pack_bf16x2(__uint_as_float(t0[8 * g]), __uint_as_float(t0[8 * g + 1])),
-                         ptx::pack_bf16x2(__uint_as_float(t0[8 * g + 2]), __uint_as_float(t0[8 * g + 3])),
-                         ptx::pack_bf16x2(__uint_as_float(t0[8 * g + 4]), __uint_as_float(t0[8 * g + 5])),
-                         ptx::pack_bf16x2(__uint_as_float(t0[8 * g + 6]), __uint_as_float(t0[8 * g + 7])));
+              make_uint4(ptx::pack_h2<F16>(__uint_as_float(t0[8 * g]), __uint_as_float(t0[8 * g + 1])),
+                         ptx::pack_h2<F16>(__uint_as_float(t0[8 * g + 2]), __uint_as_float(t0[8 * g + 3])),
+                         ptx::pack_h2<F16>(__uint_as_float(t0[8 * g + 4]), __uint_as_float(t0[8 * g + 5])),
+                         ptx::pack_h2<F16>(__uint_as_float(t0[8 * g + 6]), __uint_as_float(t0[8 * g + 7])));
           reinterpret_cast<uint4*>(o + 32)[g] =
-              make_uint4(ptx::pack_bf16x2(__uint_as_float(t1[8 * g]), __uint_as_float(t1[8 * g + 1])),
-                         ptx::pack_bf16x2(__uint_as_float(t1[8 * g + 2]), __uint_as_float(t1[8 * g + 3])),
-                         ptx::pack_bf16x2(__uint_as_float(t1[8 * g + 4]), __uint_as_float(t1[8 * g + 5])),
-                         ptx::pack_bf16x2(__uint_as_float(t1[8 * g + 6]), __uint_as_float(t1[8 * g + 7])));
+              make_uint4(ptx::pack_h2<F16>(__uint_as_float(t1[8 * g]), __uint_as_float(t1[8 * g + 1])),
+                         ptx::pack_h2<F16>(__uint_as_float(t1[8 * g + 2]), __uint_as_float(t1[8 * g + 3])),
+                         ptx::pack_h2<F16>(__uint_as_float(t1[8 * g + 4]), __uint_as_float(t1[8 * g + 5])),
+                         ptx::pack_h2<F16>(__uint_as_float(t1[8 * g + 6]), __uint_as_float(t1[8 * g + 7])));
         }
       }
     };
@@ -433,8 +435,8 @@ attn_bwd_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __gr
             const uint64_t d2 = ptx::mul_f32x2(ptx::pack_f32x2(p0, p1), g2);
             float d0, d1;
             ptx::unpack_f32x2(d2, d0, d1);
-            sv[cc][u] = ptx::pack_bf16x2(p0, p1);     // words u <= 2u have been consumed
-            dp[cc][u] = ptx::pack_bf16x2(d0, d1);
+            sv[cc][u] = ptx::pack_h2<F16>(p0, p1);     // words u <= 2u have been consumed
+            dp[cc][u] = ptx::pack_h2<F16>(d0, d1);
           }
           if (c * 32 + 32 > kv_len) {   // ragged key block: keys beyond the image contribute nothing
 #pragma unroll

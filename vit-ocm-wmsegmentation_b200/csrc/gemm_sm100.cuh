@@ -255,6 +255,35 @@ __device__ __forceinline__ void gelu_grad_mul_x2(float& v0, float& v1, float x0,
   ptx::unpack_f32x2(r, v0, v1);
 }
 
+// Derivative of the five-coefficient form gelu_sigmoid5_x2 (fp16 engines, which run their forward fc1 in that form): with
+// t = x P(u), P(u) = p0 + p1 u + p2 u^2 + p3 u^3 + p4 u^4 (= -(its coefficients) / log2(e)), u = x^2:
+//     gelu'(x) = s + x s (1 - s) t'(x),   t' = p0 + 3 p1 u + 5 p2 u^2 + 7 p3 u^3 + 9 p4 u^4
+// Max |error| against the exact erf-form derivative 1.5e-5 over [-12, 12].  No clamp of u: the saved input is fp16 (|x| <= 65504),
+// where t' stays finite (< 1e35), and x s (1 - s) is exactly 0 once the sigmoid has saturated.  v <- v * gelu'(x).
+__device__ __forceinline__ void gelu5_grad_mul_x2(float& v0, float& v1, float x0, float x1) {
+  const uint64_t x2 = ptx::pack_f32x2(x0, x1);
+  const uint64_t u = ptx::mul_f32x2(x2, x2);
+  uint64_t poly = ptx::fma_f32x2(u, ptx::dup_f32x2(2.238172939e-06f), ptx::dup_f32x2(-6.116215382e-05f));
+  poly = ptx::fma_f32x2(poly, u, ptx::dup_f32x2(-2.497226093e-04f));
+  poly = ptx::fma_f32x2(poly, u, ptx::dup_f32x2(7.293758349e-02f));
+  poly = ptx::fma_f32x2(poly, u, ptx::dup_f32x2(1.595656209f));
+  const uint64_t arg = ptx::mul_f32x2(ptx::mul_f32x2(x2, poly), ptx::dup_f32x2(-1.4426950408889634f));
+  float a0, a1;
+  ptx::unpack_f32x2(arg, a0, a1);
+  const uint64_t den = ptx::add_f32x2(ptx::pack_f32x2(ptx::ex2_approx(a0), ptx::ex2_approx(a1)), ptx::dup_f32x2(1.0f));
+  float d0, d1;
+  ptx::unpack_f32x2(den, d0, d1);
+  const uint64_t sg = ptx::pack_f32x2(ptx::rcp_approx(d0), ptx::rcp_approx(d1));
+  uint64_t dt = ptx::fma_f32x2(u, ptx::dup_f32x2(2.014355645e-05f), ptx::dup_f32x2(-4.281350767e-04f));
+  dt = ptx::fma_f32x2(dt, u, ptx::dup_f32x2(-1.248613046e-03f));
+  dt = ptx::fma_f32x2(dt, u, ptx::dup_f32x2(2.188127505e-01f));
+  dt = ptx::fma_f32x2(dt, u, ptx::dup_f32x2(1.595656209f));
+  const uint64_t om = ptx::fma_f32x2(sg, ptx::dup_f32x2(-1.0f), ptx::dup_f32x2(1.0f));
+  const uint64_t g = ptx::fma_f32x2(ptx::mul_f32x2(ptx::mul_f32x2(x2, sg), om), dt, sg);
+  const uint64_t r = ptx::mul_f32x2(ptx::pack_f32x2(v0, v1), g);
+  ptx::unpack_f32x2(r, v0, v1);
+}
+
 template <int BN, int EPI, bool A_PATCH, bool B_RES = false, int CS = 1, bool PAIR = false>
 __global__ void __launch_bounds__(gemm_threads(BN, EPI), 1)
 gemm_bf16_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ CUtensorMap tmap_b,
@@ -762,19 +791,35 @@ gemm_bf16_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __gri
         float v[32];
 #pragma unroll
         for (int j = 0; j < 32; ++j) v[j] = __uint_as_float(r[j]) + bv[j];
-        if (EPI == EPI_DGELU_BF16) {
+        if (EPI == EPI_DGELU_BF16) {   // the derivative of the GELU form the forward used: gelu_mode 2 on fp16 engines, else 0
+          if (args.f16) {
 #pragma unroll
-          for (int g = 0; g < 4; ++g) {
-            const uint32_t wds[4] = {pq[g].x, pq[g].y, pq[g].z, pq[g].w};
+            for (int g = 0; g < 4; ++g) {
+              const uint32_t wds[4] = {pq[g].x, pq[g].y, pq[g].z, pq[g].w};
 #pragma unroll
-            for (int k = 0; k < 4; ++k)
-              gelu_grad_mul_x2(v[8 * g + 2 * k], v[8 * g + 2 * k + 1], __uint_as_float(wds[k] << 16), __uint_as_float(wds[k] & 0xffff0000u));
+              for (int k = 0; k < 4; ++k)
+                gelu5_grad_mul_x2(v[8 * g + 2 * k], v[8 * g + 2 * k + 1], __half2float(__ushort_as_half(static_cast<unsigned short>(wds[k] & 0xffffu))),
+                                  __half2float(__ushort_as_half(static_cast<unsigned short>(wds[k] >> 16))));
+            }
+          } else {
+#pragma unroll
+            for (int g = 0; g < 4; ++g) {
+              const uint32_t wds[4] = {pq[g].x, pq[g].y, pq[g].z, pq[g].w};
+#pragma unroll
+              for (int k = 0; k < 4; ++k)
+                gelu_grad_mul_x2(v[8 * g + 2 * k], v[8 * g + 2 * k + 1], __uint_as_float(wds[k] << 16), __uint_as_float(wds[k] & 0xffff0000u));
+            }
           }
         }
-        uint32_t pre[16];   // training: the GELU input, kept for the backward (vit.py:59)
+        uint32_t pre[16];   // training: the GELU input, kept for the backward (vit.py:59), in the engine's 16-bit format
         if (EPI == EPI_BIAS_GELU_BF16 && args.split_out == 2) {
+          if (args.f16) {
 #pragma unroll
-          for (int j = 0; j < 16; ++j) pre[j] = ptx::pack_bf16x2(v[2 * j], v[2 * j + 1]);
+            for (int j = 0; j < 16; ++j) pre[j] = ptx::pack_f16x2(v[2 * j], v[2 * j + 1]);
+          } else {
+#pragma unroll
+            for (int j = 0; j < 16; ++j) pre[j] = ptx::pack_bf16x2(v[2 * j], v[2 * j + 1]);
+          }
         }
         if (EPI == EPI_BIAS_GELU_BF16) {
           if (args.gelu_mode == 0) {

@@ -8,6 +8,9 @@
 //   sumsq_kernel, adamw_kernel           torch.nn.utils.clip_grad_norm_ + torch.optim.AdamW (optimizer.py:73-75)
 //   repack_weights_kernel                fp32 masters -> bf16 [R][C] and [C][R] (forward / input-gradient B operands), one launch
 // All vectorised and coalesced; statistics and accumulations in fp32 (fp64 for the global gradient norm).
+// The backward kernels take the 16-bit element type as a template parameter F16 (false: bf16, true: IEEE fp16).  On fp16
+// engines every 16-bit gradient tensor, the fp32 residual gradient dX, dQacc and Delta carry the loss scale S = 2^e chosen by
+// mim_loss_bwd_kernel (lscale[0] = S, lscale[1] = 1 / S); the writers of parameter gradients multiply by 1 / S, which is exact.
 #pragma once
 #include "gemm_sm100.cuh"
 #include "ptx.cuh"
@@ -17,6 +20,22 @@ namespace vitocm {
 
 __device__ __forceinline__ float bf16lo(uint32_t v) { return __uint_as_float(v << 16); }
 __device__ __forceinline__ float bf16hi(uint32_t v) { return __uint_as_float(v & 0xffff0000u); }
+// low / high element of a pair of 16-bit values in the format F16 selects
+template <bool F16>
+__device__ __forceinline__ float h16lo(uint32_t v) {
+  if (F16) return __half2float(__ushort_as_half(static_cast<unsigned short>(v & 0xffffu)));
+  return bf16lo(v);
+}
+template <bool F16>
+__device__ __forceinline__ float h16hi(uint32_t v) {
+  if (F16) return __half2float(__ushort_as_half(static_cast<unsigned short>(v >> 16)));
+  return bf16hi(v);
+}
+
+// Loss scale of fp16 engines: S = 2^e with |coef| * S in [2^LOSS_SCALE_K0, 2^(LOSS_SCALE_K0 + 1)), coef the loss gradient's
+// magnitude (mim_loss_bwd_kernel).  Derived from coef's exponent alone, so a power-of-two change of coef (gscale) changes S
+// and nothing else: every scaled 16-bit tensor keeps its bits.  The value of K0 and the headroom it leaves: DESIGN.md §6.
+constexpr int LOSS_SCALE_K0 = 0;
 
 // ------------------------------------------------------------------------------------------------ LayerNorm backward
 // One warp per row (grid-stride).  y = (x - mean) * rstd * gamma + beta,  dy = dL/dy (bf16):
@@ -25,11 +44,12 @@ __device__ __forceinline__ float bf16hi(uint32_t v) { return __uint_as_float(v &
 //   dgamma += dy * xhat,  dbeta += dy           (per-lane partials -> shared memory -> one atomicAdd per block and column)
 //   dbias_out += column sums of the new dX      (= the bias gradient of the Linear whose output was added into this
 //                                                residual stream: proj of this block / fc2 of the previous one)
-template <int NV>
+// F16: dy / dXb are fp16 and carry the loss scale; dgamma, dbeta and dbias_out are multiplied by lscale[1] = 1 / S.
+template <int NV, bool F16 = false>
 __global__ void __launch_bounds__(256)
 ln_bwd_kernel(const float* __restrict__ x, const __nv_bfloat16* __restrict__ dy, long long ld_dy, const float* __restrict__ gamma,
               float* __restrict__ dX, __nv_bfloat16* __restrict__ dXb, float* __restrict__ dgamma, float* __restrict__ dbeta,
-              float* __restrict__ dbias_out, int accumulate, int M, int D, float eps) {
+              float* __restrict__ dbias_out, int accumulate, int M, int D, float eps, const float* __restrict__ lscale = nullptr) {
   constexpr int CNT = NV > 0 ? NV : LN_MAX_VEC;
   extern __shared__ float ln_red[];   // [3][D]
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarps = blockDim.x >> 5;
@@ -60,7 +80,7 @@ ln_bwd_kernel(const float* __restrict__ x, const __nv_bfloat16* __restrict__ dy,
         // the running residual gradient is requested together with x and dy: one exposed memory latency per row, not two
         acc_in[i] = accumulate ? dxr[idx] : make_float4(0.f, 0.f, 0.f, 0.f);
         const uint2 d2 = dr[idx];
-        g[i] = make_float4(bf16lo(d2.x), bf16hi(d2.x), bf16lo(d2.y), bf16hi(d2.y));
+        g[i] = make_float4(h16lo<F16>(d2.x), h16hi<F16>(d2.x), h16lo<F16>(d2.y), h16hi<F16>(d2.y));
         s += (v[i].x + v[i].y) + (v[i].z + v[i].w);
       }
     }
@@ -101,7 +121,7 @@ ln_bwd_kernel(const float* __restrict__ x, const __nv_bfloat16* __restrict__ dy,
         o.z += rstd * (g[i].z - c1 - v[i].z * c2);
         o.w += rstd * (g[i].w - c1 - v[i].w * c2);
         dxr[idx] = o;
-        dbr[idx] = make_uint2(ptx::pack_bf16x2(o.x, o.y), ptx::pack_bf16x2(o.z, o.w));
+        dbr[idx] = make_uint2(ptx::pack_h2<F16>(o.x, o.y), ptx::pack_h2<F16>(o.z, o.w));
         acco[i].x += o.x; acco[i].y += o.y; acco[i].z += o.z; acco[i].w += o.w;
       }
     }
@@ -121,6 +141,15 @@ ln_bwd_kernel(const float* __restrict__ x, const __nv_bfloat16* __restrict__ dy,
     }
   }
   __syncthreads();
+  if (F16) {
+    const float inv = lscale != nullptr ? lscale[1] : 1.0f;
+    for (int i = threadIdx.x; i < D; i += blockDim.x) {
+      atomicAdd(dgamma + i, ln_red[i] * inv);
+      atomicAdd(dbeta + i, ln_red[D + i] * inv);
+      if (dbias_out != nullptr) atomicAdd(dbias_out + i, ln_red[2 * D + i] * inv);
+    }
+    return;
+  }
   for (int i = threadIdx.x; i < D; i += blockDim.x) {
     atomicAdd(dgamma + i, ln_red[i]);
     atomicAdd(dbeta + i, ln_red[D + i]);
@@ -129,9 +158,9 @@ ln_bwd_kernel(const float* __restrict__ x, const __nv_bfloat16* __restrict__ dy,
 }
 
 // ------------------------------------------------------------------------------------------------ attention backward helpers
-// delta[b][h][q] (row pitch npad) = sum_d dO[row][h*DH + d] * O[row][h*DH + d]; one warp per token row, DH / 32 bf16 per lane
-// per head; all heads' loads are issued before the first reduction (HG heads at a time) so that a row costs one memory latency
-template <int HG, int DH = 64>
+// delta[b][h][q] (row pitch npad) = sum_d dO[row][h*DH + d] * O[row][h*DH + d]; one warp per token row, DH / 32 16-bit values per
+// lane per head; all heads' loads are issued before the first reduction (HG heads at a time) so that a row costs one memory latency
+template <int HG, int DH = 64, bool F16 = false>
 __global__ void __launch_bounds__(256)
 attn_delta_kernel(const __nv_bfloat16* __restrict__ O, const __nv_bfloat16* __restrict__ dO, long long ld, float* __restrict__ delta,
                   int B, int N, int heads, int npad) {
@@ -156,9 +185,9 @@ attn_delta_kernel(const __nv_bfloat16* __restrict__ O, const __nv_bfloat16* __re
 #pragma unroll
       for (int k = 0; k < HG; ++k) {
         if (h0 + k < heads) {
-          float p = bf16lo(o[k][0]) * bf16lo(d[k][0]) + bf16hi(o[k][0]) * bf16hi(d[k][0]);
+          float p = h16lo<F16>(o[k][0]) * h16lo<F16>(d[k][0]) + h16hi<F16>(o[k][0]) * h16hi<F16>(d[k][0]);
 #pragma unroll
-          for (int u = 1; u < W; ++u) p += bf16lo(o[k][u]) * bf16lo(d[k][u]) + bf16hi(o[k][u]) * bf16hi(d[k][u]);
+          for (int u = 1; u < W; ++u) p += h16lo<F16>(o[k][u]) * h16lo<F16>(d[k][u]) + h16hi<F16>(o[k][u]) * h16hi<F16>(d[k][u]);
           const float s = warp_sum(p);
           if (lane == 0) delta[(static_cast<long long>(b) * heads + h0 + k) * npad + q] = s;
         }
@@ -167,8 +196,9 @@ attn_delta_kernel(const __nv_bfloat16* __restrict__ O, const __nv_bfloat16* __re
   }
 }
 
-// dqkv[row][0:D] = bf16(acc[row][:]);  acc <- 0.  One warp per pair of rows (grid-strided); all loads of a pass (up to
+// dqkv[row][0:D] = 16-bit(acc[row][:]);  acc <- 0.  One warp per pair of rows (grid-strided); all loads of a pass (up to
 // 2 rows x 4 float4 per lane) are issued before the first store so that a warp keeps 4 KB in flight.
+template <bool F16 = false>
 __global__ void __launch_bounds__(256)
 dq_convert_kernel(float4* __restrict__ acc, __nv_bfloat16* __restrict__ dqkv, long long ld, int M, int D) {
   const int nvec = D >> 2;
@@ -192,7 +222,7 @@ dq_convert_kernel(float4* __restrict__ acc, __nv_bfloat16* __restrict__ dqkv, lo
           if (row0 + r < M && c < nvec) {
             acc[static_cast<long long>(row0 + r) * nvec + c] = make_float4(0.f, 0.f, 0.f, 0.f);
             *reinterpret_cast<uint2*>(dqkv + static_cast<long long>(row0 + r) * ld + 4 * c) =
-                make_uint2(ptx::pack_bf16x2(v[r][u].x, v[r][u].y), ptx::pack_bf16x2(v[r][u].z, v[r][u].w));
+                make_uint2(ptx::pack_h2<F16>(v[r][u].x, v[r][u].y), ptx::pack_h2<F16>(v[r][u].z, v[r][u].w));
           }
         }
     }
@@ -203,12 +233,30 @@ dq_convert_kernel(float4* __restrict__ acc, __nv_bfloat16* __restrict__ dqkv, lo
 // loss = sum |x - x_rec| * mask / (sum mask + 1e-5) / C  (model.py:75-76), x_rec = PixelShuffle(Y) (model.py:61-66):
 //   dY[b*(n+1) + 1 + tok][c p^2 + i p + j] = *gscale * mask[b, tok] * sign(x_rec - x) / ((sums[1] + 1e-5) * C)
 // CLS rows of dY are zero.  One thread per 8 consecutive columns (one patch row of one channel when p == 8).
+// F16: dY is fp16 and multiplied by the loss scale S = 2^e (|coef| S in [2^LOSS_SCALE_K0, 2^(LOSS_SCALE_K0 + 1)); S = 1 when coef
+// is 0 or not finite), chosen here on the device from coef's exponent; S and 1 / S go to lscale[0], lscale[1].
+template <bool F16 = false>
 __global__ void __launch_bounds__(256)
 mim_loss_bwd_kernel(const float* __restrict__ x, const float* __restrict__ x_rec, const float* __restrict__ mask,
                     const double* __restrict__ sums, const float* __restrict__ gscale, __nv_bfloat16* __restrict__ dY, int B, int C, int H,
-                    int W, int p) {
+                    int W, int p, float* __restrict__ lscale = nullptr) {
   const int Wp = W / p, n = (H / p) * Wp, ldy = C * p * p, groups = ldy / 8;
-  const float coef = (gscale != nullptr ? *gscale : 1.0f) / (static_cast<float>(sums[1] + 1e-5) * static_cast<float>(C));
+  float coef = (gscale != nullptr ? *gscale : 1.0f) / (static_cast<float>(sums[1] + 1e-5) * static_cast<float>(C));
+  if (F16) {
+    int e = 0;
+    if (coef != 0.f && isfinite(coef)) {
+      int ex;
+      frexpf(coef, &ex);                     // |coef| = f 2^ex, f in [0.5, 1)
+      e = LOSS_SCALE_K0 + 1 - ex;
+      e = e < -126 ? -126 : (e > 126 ? 126 : e);
+    }
+    const float S = __int_as_float((127 + e) << 23), inv = __int_as_float((127 - e) << 23);
+    coef *= S;                               // exact
+    if (blockIdx.x == 0 && threadIdx.x == 0 && lscale != nullptr) {
+      lscale[0] = S;
+      lscale[1] = inv;
+    }
+  }
   const long long total = static_cast<long long>(B) * (n + 1) * groups;
   for (long long idx = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; idx < total;
        idx += static_cast<long long>(gridDim.x) * blockDim.x) {
@@ -231,12 +279,13 @@ mim_loss_bwd_kernel(const float* __restrict__ x, const float* __restrict__ x_rec
       }
     }
     *reinterpret_cast<uint4*>(dY + row * ldy + col) =
-        make_uint4(ptx::pack_bf16x2(g[0], g[1]), ptx::pack_bf16x2(g[2], g[3]), ptx::pack_bf16x2(g[4], g[5]), ptx::pack_bf16x2(g[6], g[7]));
+        make_uint4(ptx::pack_h2<F16>(g[0], g[1]), ptx::pack_h2<F16>(g[2], g[3]), ptx::pack_h2<F16>(g[4], g[5]), ptx::pack_h2<F16>(g[6], g[7]));
   }
 }
 
 // ------------------------------------------------------------------------------------------------ token-embedding backward
-// G[b*n + i][:] = bf16((1 - mask[b, i]) * dX0[b, 1 + i, :])    (model.py:31-33: only unmasked patches see the conv)
+// G[b*n + i][:] = 16-bit((1 - mask[b, i]) * dX0[b, 1 + i, :])    (model.py:31-33: only unmasked patches see the conv)
+template <bool F16 = false>
 __global__ void __launch_bounds__(256)
 patch_grad_rows_kernel(const float4* __restrict__ dX0, const float* __restrict__ mask, __nv_bfloat16* __restrict__ G, int B, int n, int D) {
   const int nvec = D >> 2;
@@ -248,11 +297,12 @@ patch_grad_rows_kernel(const float4* __restrict__ dX0, const float* __restrict__
     const int b = static_cast<int>(m / n), i = static_cast<int>(m - static_cast<long long>(b) * n);
     const float w = 1.0f - mask[m];
     const float4 v = dX0[(static_cast<long long>(b) * (n + 1) + 1 + i) * nvec + c];
-    *reinterpret_cast<uint2*>(G + m * D + 4 * c) = make_uint2(ptx::pack_bf16x2(v.x * w, v.y * w), ptx::pack_bf16x2(v.z * w, v.w * w));
+    *reinterpret_cast<uint2*>(G + m * D + 4 * c) = make_uint2(ptx::pack_h2<F16>(v.x * w, v.y * w), ptx::pack_h2<F16>(v.z * w, v.w * w));
   }
 }
 
-// P[b*n + py*Wp + px][c p^2 + yi p + xi] = bf16(x[b, c, py p + yi, px p + xi]); one thread per 8 consecutive pixels
+// P[b*n + py*Wp + px][c p^2 + yi p + xi] = 16-bit(x[b, c, py p + yi, px p + xi]); one thread per 8 consecutive pixels
+template <bool F16 = false>
 __global__ void __launch_bounds__(256)
 im2col_bf16_kernel(const float* __restrict__ x, __nv_bfloat16* __restrict__ P, int B, int C, int H, int W, int p) {
   const int Wp = W / p, n = (H / p) * Wp, K = C * p * p, groups = K / 8;
@@ -267,15 +317,17 @@ im2col_bf16_kernel(const float* __restrict__ x, __nv_bfloat16* __restrict__ P, i
     const float* src = x + ((static_cast<long long>(b) * C + c) * H + py * p + yi) * W + px * p + xi;
     const float4 a = *reinterpret_cast<const float4*>(src), bq = *reinterpret_cast<const float4*>(src + 4);
     *reinterpret_cast<uint4*>(P + m * K + k) =
-        make_uint4(ptx::pack_bf16x2(a.x, a.y), ptx::pack_bf16x2(a.z, a.w), ptx::pack_bf16x2(bq.x, bq.y), ptx::pack_bf16x2(bq.z, bq.w));
+        make_uint4(ptx::pack_h2<F16>(a.x, a.y), ptx::pack_h2<F16>(a.z, a.w), ptx::pack_h2<F16>(bq.x, bq.y), ptx::pack_h2<F16>(bq.z, bq.w));
   }
 }
 
 // dpos[t][:] = sum_b dX0[b, t, :];  dcls += dpos[0];  dmask_token += sum_{b, i} mask[b, i] * dX0[b, 1 + i, :]
-// one thread per (token t, float4 column group), looping over the batch
+// one thread per (token t, float4 column group), looping over the batch.  F16: dX0 carries the loss scale; the sums are
+// multiplied by lscale[1] = 1 / S
+template <bool F16 = false>
 __global__ void __launch_bounds__(256)
 token_grad_kernel(const float4* __restrict__ dX0, const float* __restrict__ mask, float4* __restrict__ dpos, float* __restrict__ dcls,
-                  float* __restrict__ dmask_token, int B, int n, int D) {
+                  float* __restrict__ dmask_token, int B, int n, int D, const float* __restrict__ lscale = nullptr) {
   const int nvec = D >> 2;
   const int total = (n + 1) * nvec;
   const int idx = blockIdx.x * blockDim.x + threadIdx.x;
@@ -289,6 +341,11 @@ token_grad_kernel(const float4* __restrict__ dX0, const float* __restrict__ mask
       const float w = mask[static_cast<long long>(b) * n + t - 1];
       sm.x += w * v.x; sm.y += w * v.y; sm.z += w * v.z; sm.w += w * v.w;
     }
+  }
+  if (F16) {
+    const float inv = lscale != nullptr ? lscale[1] : 1.0f;
+    s.x *= inv; s.y *= inv; s.z *= inv; s.w *= inv;
+    sm.x *= inv; sm.y *= inv; sm.z *= inv; sm.w *= inv;
   }
   dpos[idx] = s;
   if (t == 0) {

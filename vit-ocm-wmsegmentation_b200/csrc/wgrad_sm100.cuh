@@ -13,6 +13,8 @@
 // Bias gradient for free: the column sums of G are G^T . 1, so the CTAs of the first column tile issue one extra N = 16 MMA per
 // k-step against a constant all-ones B tile (8 KB of bf16 1.0: any swizzle of ones is ones) into 16 spare TMEM columns; the
 // epilogue adds column 0 into db with 128 atomics per CTA.  No separate pass over G.
+// F16 = true: fp16 operands (fp16 engines).  G then carries the loss scale S of the training step, and the epilogue multiplies
+// the accumulator (and the bias column) by *inv_scale = 1 / S before the reduce-add: exact, S being a power of two.
 #pragma once
 #include "ptx.cuh"
 
@@ -25,6 +27,7 @@ struct WgradArgs {
   int splits;     // token splits
   int kblocks;    // ceil(M / 64)
   float* colsum;  // [R] or nullptr: colsum[r] += sum_m G[m][r] -- the bias gradient of the same Linear, from the tensor core
+  const float* inv_scale;   // F16 only: device scalar multiplied into dW and colsum (nullptr: 1)
 };
 
 constexpr int WG_BM = 128;      // rows of dW per tile (features of G)
@@ -39,7 +42,7 @@ struct WgradCfg {
   static constexpr int B_BYTES = (WIDTH / 64) * WG_ATOM_BYTES;      // WIDTH features of A
   static constexpr int STAGE_BYTES = A_BYTES + B_BYTES;
   static constexpr int STG_BYTES = 4 * 4096;                        // per epilogue warp one 32 x 32 fp32 box
-  static constexpr int ONES_BYTES = WG_ATOM_BYTES;                  // [64 tokens][64 x bf16 1.0]
+  static constexpr int ONES_BYTES = WG_ATOM_BYTES;                  // [64 tokens][64 x 16-bit 1.0]
   static constexpr int FIXED = STG_BYTES + ONES_BYTES + 1024 + 256;
   static constexpr int STAGES_FIT = (227 * 1024 - FIXED) / STAGE_BYTES;
   static constexpr int STAGES = STAGES_FIT > 6 ? 6 : STAGES_FIT;
@@ -50,7 +53,7 @@ struct WgradCfg {
   static_assert(STAGES >= 3, "not enough shared memory for a 3-stage pipeline");
 };
 
-template <int BN, int NB>
+template <int BN, int NB, bool F16 = false>
 __global__ void __launch_bounds__(WG_THREADS, 1)
 wgrad_bf16_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_g, const __grid_constant__ CUtensorMap tmap_a,
                           const __grid_constant__ CUtensorMap tmap_w, const WgradArgs args) {
@@ -95,8 +98,9 @@ wgrad_bf16_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_g, const __gr
     ptx::tmem_relinquish();
   }
   if (do_colsum && warp >= 2) {   // the all-ones B tile of the bias-gradient MMA
+    constexpr uint32_t ONE2 = F16 ? 0x3c003c00u : 0x3f803f80u;   // 1.0 twice, fp16 / bf16
     for (int i = (warp - 2) * 32 + lane; i < Cfg::ONES_BYTES / 16; i += 128)
-      ptx::sts_v4(smem_ones + i * 16, 0x3f803f80u, 0x3f803f80u, 0x3f803f80u, 0x3f803f80u);
+      ptx::sts_v4(smem_ones + i * 16, ONE2, ONE2, ONE2, ONE2);
     ptx::fence_proxy_async_smem();
   }
   ptx::tc_fence_before();
@@ -125,8 +129,8 @@ wgrad_bf16_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_g, const __gr
   } else if (warp == 1) {
     // ===================== MMA issuer =====================
     if (ptx::elect_one()) {
-      constexpr uint32_t idesc = ptx::make_idesc(WG_BM, BN, /*A MN-major*/ true, /*B MN-major*/ true);
-      constexpr uint32_t idesc_ones = ptx::make_idesc(WG_BM, 16, true, true);
+      constexpr uint32_t idesc = ptx::make_idesc(WG_BM, BN, /*A MN-major*/ true, /*B MN-major*/ true, F16 ? 0u : 1u);
+      constexpr uint32_t idesc_ones = ptx::make_idesc(WG_BM, 16, true, true, F16 ? 0u : 1u);
       const uint64_t ones_desc = ptx::make_smem_desc_sw128(smem_ones, 1024, WG_ATOM_BYTES);
       int stage = 0;
       uint32_t phase = 0;
@@ -160,11 +164,12 @@ wgrad_bf16_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_g, const __gr
     ptx::mbar_wait(acc_bar, 0, 33);
     ptx::tc_fence_after();
     const int row = r0 + q * 32;
+    const float inv = F16 && args.inv_scale != nullptr ? *args.inv_scale : 1.0f;
     if (do_colsum) {   // column 0 of the ones-MMA accumulator = sum over this split's tokens of G[:, row + lane]
       uint32_t cs;
       ptx::tmem_ld_32x32b_x1(tmem_base + (static_cast<uint32_t>(q * 32) << 16) + static_cast<uint32_t>(Cfg::WIDTH), cs);
       ptx::tmem_ld_wait1(cs);
-      if (row + lane < args.R) atomicAdd(args.colsum + row + lane, __uint_as_float(cs));
+      if (row + lane < args.R) atomicAdd(args.colsum + row + lane, F16 ? __uint_as_float(cs) * inv : __uint_as_float(cs));
     }
     if (row < args.R) {
 #pragma unroll 1
@@ -175,6 +180,10 @@ wgrad_bf16_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_g, const __gr
         if (lane == 0) ptx::bulk_wait_read0();   // the previous chunk's reduce has finished reading the box
         __syncwarp();
         ptx::tmem_ld_wait(r);
+        if (F16) {
+#pragma unroll
+          for (int j = 0; j < 32; ++j) r[j] = __float_as_uint(__uint_as_float(r[j]) * inv);
+        }
         const uint32_t rowaddr = stg + lane * 128;
         const int sw = lane & 7;
 #pragma unroll
