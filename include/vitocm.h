@@ -116,6 +116,12 @@ int vitocm_forward_cls_attn_gray(vitocm_engine* e, const float* x, int B, int H,
 int vitocm_forward_cls_attn_mosaic(vitocm_engine* e, const uint8_t* mosaic, int mos_h, int mos_w, int64_t pitch, int n, int W, int S,
                                    int t0, int T, const float* pos, float* out_rows, void* ws, size_t ws_bytes, int chunk_tiles,
                                    void* stream);
+/* The same on a rectangular ny x nx grid (rows of windows over the mosaic's height, columns over its width; the reference's
+ * SSS/sw_processing.py:151-163 walk with the axes taken from the height and the width of a rectangle): window t0 + i has origin
+ * ((t / nx) * S, (t % nx) * S).  Needs ny, nx >= 1 and t0 + T <= ny * nx.  vitocm_forward_cls_attn_mosaic is this with ny = nx = n. */
+int vitocm_forward_cls_attn_mosaic_grid(vitocm_engine* e, const uint8_t* mosaic, int mos_h, int mos_w, int64_t pitch, int ny, int nx, int W,
+                                        int S, int t0, int T, const float* pos, float* out_rows, void* ws, size_t ws_bytes, int chunk_tiles,
+                                        void* stream);
 
 /* The same forward for a LIST of query tokens (SSS/analyse_attention.py:183-247: compute_attention(..., query=q) for a
  * region query) and, optionally, the last block's K features (SSS/analyse_attention.py:139-163, SSS/eval.py:186-202, the
@@ -183,12 +189,27 @@ int vitocm_tile_threshold_aux(const float* lowres, const float* x, int T, int C,
  * mosaic u8 gray [mos_h][pitch] -> x [T][C][W][W] fp32. */
 int vitocm_extract_tiles(const uint8_t* mosaic, int mos_h, int mos_w, int64_t pitch, int n, int W, int S, int t0, int T,
                          int C, float* x, void* stream);
+/* The same for tiles t0..t0+T-1 (row-major) of an ny x nx grid (SSS/sw_processing.py:151-163 with rows over the height and
+ * columns over the width); needs t0 + T <= ny * nx. */
+int vitocm_extract_tiles_grid(const uint8_t* mosaic, int mos_h, int mos_w, int64_t pitch, int ny, int nx, int W, int S, int t0, int T,
+                              int C, float* x, void* stream);
 
 /* concat_crops on the uint8 image crops (SSS/sw_processing.py:113-149 at :225) for output rows
  * [y_begin, y_end): out [E][E] u8 (full-size buffer, E = (n-1) S + W).  wtab = host-computed
  * numpy.linspace(1, 0, W - S) copied to the device (double[W - S]). */
 int vitocm_stitch_gray(const uint8_t* mosaic, int mos_h, int mos_w, int64_t pitch, int n, int W, int S,
                        const double* wtab, int y_begin, int y_end, uint8_t* out, void* stream);
+
+/* Rectangular grids.  The *_grid forms below take an ny x nx window grid where the functions above take n (each n-form is its
+ * grid form with ny = nx = n): tile t = i * nx + j sits at (i S, j S); the stitched extent is Ey x Ex = ((ny-1) S + W) x
+ * ((nx-1) S + W); concat_crops (SSS/sw_processing.py:113-134) blends along x inside each of the ny strips of nx crops, then along
+ * y across the strips, in the reference's order with its ramp and its truncations.  Row bands [y_begin, y_end) lie in [0, Ey);
+ * full-size buffers (gray, map_out, map_in) have row pitch Ex; per-band outputs are [(y_end-y_begin)][Ex].  With map_in and
+ * lowres == NULL only the extent of the geometry is used: any (ny, nx, W, S) whose extent is the map's addresses it (e.g.
+ * W = 2, S = 1, ny = Ey - 1, nx = Ex - 1).  Grids with ny, nx < 1, W <= S or W > 4 S, and bands outside [0, Ey) are refused
+ * before any launch. */
+int vitocm_stitch_gray_grid(const uint8_t* mosaic, int mos_h, int mos_w, int64_t pitch, int ny, int nx, int W, int S,
+                            const double* wtab, int y_begin, int y_end, uint8_t* out, void* stream);
 
 /* Stitched attention map = resize pair (SSS/sw_processing.py:255-257) + concat_crops (:259) of the
  * per-tile maps lowres [n*n][lh][lw]; pass 1 of sw_processing.threshold (:43): global min / max over
@@ -221,11 +242,30 @@ int vitocm_stitch_result(const float* lowres, int n, int W, int S, int lh, int l
                          const int* minmax_ord, int y_begin, int y_end, uint8_t* result, uint8_t* att_u8, const float* map_in,
                          void* stream);
 
+/* Grid forms of the three passes and of the weighted image (SSS/sw_processing.py:37-61, :255-259 on an ny x nx grid; see
+ * vitocm_stitch_gray_grid for the geometry): lowres [ny*nx][lh][lw] row-major; map_in / map_out [Ey][Ex]. */
+int vitocm_stitch_minmax_grid(const float* lowres, int ny, int nx, int W, int S, int lh, int lw, const double* wtab, int y_begin,
+                              int y_end, int* minmax_ord, float* map_out, const float* map_in, void* stream);
+int vitocm_stitch_hist_grid(const float* lowres, int ny, int nx, int W, int S, int lh, int lw, const double* wtab,
+                            const uint8_t* gray, const int* minmax_ord, int y_begin, int y_end, uint64_t* hists,
+                            const float* map_in, void* stream);
+int vitocm_stitch_mask_grid(const float* lowres, int ny, int nx, int W, int S, int lh, int lw, const double* wtab,
+                            const uint8_t* gray, const int* minmax_ord, const int* thr, int y_begin, int y_end, uint8_t* th,
+                            uint8_t* th2, uint8_t* th3, const float* map_in, void* stream);
+int vitocm_stitch_result_grid(const float* lowres, int ny, int nx, int W, int S, int lh, int lw, const double* wtab,
+                              const uint8_t* gray, const int* minmax_ord, int y_begin, int y_end, uint8_t* result, uint8_t* att_u8,
+                              const float* map_in, void* stream);
+
 /* concat_crops(crops, stride, window_size) (SSS/sw_processing.py:113-149) on full-resolution crops:
  * float32 [n*n][W][W] -> out [E][E]; uint8 HWC [n*n][W][W][C] -> out [E][E][C]. */
 int vitocm_concat_crops_f32(const float* crops, int n, int W, int S, const double* wtab, float* out, void* stream);
 int vitocm_concat_crops_u8(const uint8_t* crops, int n, int W, int S, int C, const double* wtab, uint8_t* out,
                            void* stream);
+/* The same on a row-major ny x nx grid of crops (SSS/sw_processing.py:113-134 with the strip loop over ny and the crop loop
+ * over nx): float32 [ny*nx][W][W] -> out [Ey][Ex]; uint8 HWC [ny*nx][W][W][C] -> out [Ey][Ex][C]. */
+int vitocm_concat_crops_grid_f32(const float* crops, int ny, int nx, int W, int S, const double* wtab, float* out, void* stream);
+int vitocm_concat_crops_grid_u8(const uint8_t* crops, int ny, int nx, int W, int S, int C, const double* wtab, uint8_t* out,
+                                void* stream);
 /* sliding_window(image, stride, window_size) (SSS/sw_processing.py:151-163) on a uint8 HWC image:
  * ny x nx windows at stride S -> crops [ny*nx][W][W][C], zero padded outside the image. */
 int vitocm_crop_u8(const uint8_t* img, int img_h, int img_w, int C, int ny, int nx, int W, int S, uint8_t* crops,

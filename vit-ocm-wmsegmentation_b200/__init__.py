@@ -20,7 +20,7 @@ from . import utils, sw_processing, model, optimizer, lr_scheduler, synthetic, p
 from .vision_transformer import VisionTransformer, vit_tiny, vit_small, vit_base, LazyAttention, LazyTensor  # noqa: F401
 from .utils import compute_attention, attention_masks, cropped_attention_masks, head_mean_maps, concat_crops_overlap  # noqa: F401
 from ._lib import VitocmError  # noqa: F401
-from .sw_processing import MosaicSegmenter, sliding_window, grid_size, shard_range, shared_pinned_u8  # noqa: F401
+from .sw_processing import MosaicSegmenter, sliding_window, grid_size, mosaic_grid, shard_range, shared_pinned_u8  # noqa: F401
 from .model import VisionTransformerForSimMIM, MIM, MaskGenerator, build_model  # noqa: F401
 
 __version__ = "0.1.0"

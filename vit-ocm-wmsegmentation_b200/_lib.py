@@ -37,6 +37,8 @@ SIGNATURES = {
                                              c_int, c_void_p]),
     "vitocm_forward_cls_attn_mosaic": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int64, c_int, c_int, c_int, c_int, c_int, c_void_p,
                                                c_void_p, c_void_p, c_size_t, c_int, c_void_p]),
+    "vitocm_forward_cls_attn_mosaic_grid": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int64, c_int, c_int, c_int, c_int, c_int, c_int,
+                                                    c_void_p, c_void_p, c_void_p, c_size_t, c_int, c_void_p]),
     "vitocm_forward_query_attn": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_void_p,
                                           c_size_t, c_int, c_void_p]),
     "vitocm_prepare_tokens": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p]),
@@ -68,6 +70,20 @@ SIGNATURES = {
                                    c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
     "vitocm_concat_crops_f32": (c_int, [c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p]),
     "vitocm_concat_crops_u8": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p]),
+    "vitocm_extract_tiles_grid": (c_int, [c_void_p, c_int, c_int, c_int64, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p,
+                                          c_void_p]),
+    "vitocm_stitch_gray_grid": (c_int, [c_void_p, c_int, c_int, c_int64, c_int, c_int, c_int, c_int, c_void_p, c_int, c_int, c_void_p,
+                                        c_void_p]),
+    "vitocm_stitch_minmax_grid": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p, c_int, c_int, c_void_p,
+                                          c_void_p, c_void_p, c_void_p]),
+    "vitocm_stitch_hist_grid": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_int, c_int,
+                                        c_void_p, c_void_p, c_void_p]),
+    "vitocm_stitch_mask_grid": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p,
+                                        c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "vitocm_stitch_result_grid": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_int, c_int,
+                                          c_void_p, c_void_p, c_void_p, c_void_p]),
+    "vitocm_concat_crops_grid_f32": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p]),
+    "vitocm_concat_crops_grid_u8": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p]),
     "vitocm_concat_crops_overlap_f32": (c_int, [c_void_p, c_int, c_int, c_int, c_void_p, c_void_p]),
     "vitocm_concat_crops_overlap_u8": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p]),
     "vitocm_concat_grid_f32": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p]),

@@ -68,10 +68,10 @@ struct GemmArgs {
   const float* mask;        // [B][n_patches] in {0,1} or nullptr (SimMIM mask-token mixing, SSS/model.py:31-33)
   const float* mask_token;  // [N]
   // A_PATCH, tile ingest straight from a gray uint8 mosaic (sliding_window + ToTensor, SSS/sw_processing.py:151-163, :236): image b of
-  // this launch is window mos_t0 + b of the n x n grid at stride mos_S, pixel value v / 255, zero beyond the mosaic; img is unused
+  // this launch is window mos_t0 + b of the row-major grid mos_nx windows wide at stride mos_S, pixel value v / 255, zero beyond the mosaic; img is unused
   const uint8_t* mos;       // [mos_h][mos_pitch] or nullptr
   long long mos_pitch;
-  int mos_h, mos_w, mos_n, mos_S, mos_t0;
+  int mos_h, mos_w, mos_nx, mos_S, mos_t0;
   float* out_f32;           // X [B][1 + n_patches][N] token stream
   int patch_tma;            // EPI_PATCH_F32: tmap_c = X as 2-D [B (1 + n_patches)][N] and tmap_d = pos [1 + n_patches][N] (fp32, 32 x 32 boxes,
                             // SWIZZLE_128B) are valid: position rows arrive and token rows leave through per-warp staging boxes
@@ -491,8 +491,8 @@ gemm_bf16_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __gri
                 const int k = kb * GEMM_BK + chunk * 8;      // one channel: k = yi * p + xi
                 const int yi = k / p, xi = k - yi * p;
                 const int tl = args.mos_t0 + b;
-                const int gy = (tl / args.mos_n) * args.mos_S + py * p + yi;
-                const int gx = (tl % args.mos_n) * args.mos_S + px * p + xi;
+                const int gy = (tl / args.mos_nx) * args.mos_S + py * p + yi;
+                const int gx = (tl % args.mos_nx) * args.mos_S + px * p + xi;
                 if (gy < args.mos_h && gx < args.mos_w) {
                   const uint8_t* src = args.mos + static_cast<long long>(gy) * args.mos_pitch + gx;
                   if (gx + 8 <= args.mos_w && (reinterpret_cast<uintptr_t>(src) & 7) == 0) {

@@ -356,19 +356,20 @@ tile_threshold_kernel(const float* __restrict__ lowres /*[T][lh][lw]*/, const fl
 }
 
 // ---------------------------------------------------------------------------------------
-// Sliding-window geometry shared by the mosaic kernels.  n x n tiles of size W at stride S
-// (origins range(0, size - 2S, S)); stitched extent E = (n-1) S + W; step = W - S.
+// Sliding-window geometry shared by the mosaic kernels.  ny x nx tiles of size W at stride S
+// (origins range(0, size - 2S, S) over the height and over the width), row-major: tile t = i * nx + j has origin (i S, j S);
+// stitched extent Ey x Ex = ((ny-1) S + W) x ((nx-1) S + W); step = W - S.  A square mosaic is ny = nx = n.
 // wtab[k] = numpy.linspace(1, 0, step)[k] (computed on the host so it is bit-identical).
 // ---------------------------------------------------------------------------------------
 struct StitchGeom {
-  int n, W, S, step, E;
+  int ny, nx, W, S, step, Ey, Ex;
   int lh, lw;        // low-res map size (W / patch)
   double scale;      // lw / W
 };
 
-// sliding_window + ToTensor: mosaic u8 gray [E0][pitch] -> x [T][C][W][W] fp32 = v / 255 (zero padded
-// outside the mosaic like PIL's crop); tiles t0 .. t0+T-1 in row-major order.
-__global__ void extract_tiles_kernel(const uint8_t* __restrict__ mosaic, int mos_h, int mos_w, long long pitch, int n,
+// sliding_window + ToTensor: mosaic u8 gray [mos_h][pitch] -> x [T][C][W][W] fp32 = v / 255 (zero padded
+// outside the mosaic like PIL's crop); tiles t0 .. t0+T-1 in row-major order of a grid nx windows wide.
+__global__ void extract_tiles_kernel(const uint8_t* __restrict__ mosaic, int mos_h, int mos_w, long long pitch, int nx,
                                      int W, int S, int t0, int T, int C, float* __restrict__ x) {
   const long long per_tile = static_cast<long long>(W) * W;
   const long long total = per_tile * T;
@@ -378,7 +379,7 @@ __global__ void extract_tiles_kernel(const uint8_t* __restrict__ mosaic, int mos
     const int r = static_cast<int>(i - tl * per_tile);
     const int y = r / W, xx = r - y * W;
     const int t = t0 + tl;
-    const int gy = (t / n) * S + y, gx = (t % n) * S + xx;
+    const int gy = (t / nx) * S + y, gx = (t % nx) * S + xx;
     const float v = (gy < mos_h && gx < mos_w) ? __fdiv_rn(static_cast<float>(mosaic[gy * pitch + gx]), 255.0f) : 0.f;
     float* xt = x + static_cast<long long>(tl) * C * per_tile + r;
     for (int c = 0; c < C; ++c) xt[c * per_tile] = v;
@@ -395,14 +396,14 @@ __device__ __forceinline__ uint8_t blend_u8(uint8_t a, uint8_t b, double w) {
 template <int V>
 __global__ void __launch_bounds__(256)
 stitch_gray_kernel(const uint8_t* __restrict__ mosaic, int mos_h, int mos_w, long long pitch, StitchGeom g,
-                   const double* __restrict__ wtab, int y_begin, int y_end, uint8_t* __restrict__ out /*[E][E]*/) {
+                   const double* __restrict__ wtab, int y_begin, int y_end, uint8_t* __restrict__ out /*[Ey][Ex]*/) {
   const int X0 = (blockIdx.x * 256 + threadIdx.x) * V;
-  if (X0 >= g.E) return;
+  if (X0 >= g.Ex) return;
   const int dW = g.W / g.S, eW = g.W % g.S;
   const int q0 = X0 / g.S, r0 = X0 - q0 * g.S;
   for (int Y = y_begin + blockIdx.y; Y < y_end; Y += gridDim.y) {
     const int qy = Y / g.S, ry = Y - qy * g.S;
-    int i1 = min(qy, g.n - 1);
+    int i1 = min(qy, g.ny - 1);
     int i0 = qy + 1 - dW - (ry < eW ? 1 : 0);
     if (i0 < 0) i0 = 0;
     uint8_t res[V];
@@ -412,7 +413,7 @@ stitch_gray_kernel(const uint8_t* __restrict__ mosaic, int mos_h, int mos_w, lon
       const int X = X0 + u;
       // every crop holds the same source pixel (zero beyond the mosaic)
       const uint8_t src = (Y < mos_h && X < mos_w) ? __ldg(mosaic + Y * pitch + X) : 0;
-      int j1 = min(q, g.n - 1);
+      int j1 = min(q, g.nx - 1);
       int j0 = q + 1 - dW - (r < eW ? 1 : 0);
       if (j0 < 0) j0 = 0;
       // horizontal sequence is identical for every strip (same source value)
@@ -429,15 +430,15 @@ stitch_gray_kernel(const uint8_t* __restrict__ mosaic, int mos_h, int mos_w, lon
       res[u] = v;
       if (++r == g.S) { r = 0; ++q; }
     }
-    const long long o = static_cast<long long>(Y) * g.E + X0;
+    const long long o = static_cast<long long>(Y) * g.Ex + X0;
     if (V == 4) *reinterpret_cast<uchar4*>(out + o) = make_uchar4(res[0], res[1 % V], res[2 % V], res[3 % V]);
     else out[o] = res[0];
   }
 }
 
-// tiles covering coordinate P = q * S + r (q = P / S): [c0, c1]
-__device__ __forceinline__ void cover_range(const StitchGeom& g, int q, int r, int dW, int eW, int& c0, int& c1) {
-  c1 = min(q, g.n - 1);
+// tiles covering coordinate P = q * S + r (q = P / S) along an axis of `cnt` tiles: [c0, c1]
+__device__ __forceinline__ void cover_range(int cnt, int q, int r, int dW, int eW, int& c0, int& c1) {
+  c1 = min(q, cnt - 1);
   c0 = q + 1 - dW - (r < eW ? 1 : 0);      // = (P - W + S) / S for P >= W - S ... clamped below
   if (c0 < 0) c0 = 0;
 }
@@ -453,7 +454,7 @@ __device__ __forceinline__ uint8_t blend_u8_pre(uint8_t a, uint8_t b, double w, 
 template <int V, int MC>
 __global__ void __launch_bounds__(SG_THREADS)
 stitch_gray_strip_kernel(const uint8_t* __restrict__ mosaic, int mos_h, int mos_w, long long pitch, StitchGeom g,
-                         const double* __restrict__ wtab, int y_begin, int y_end, uint8_t* __restrict__ out /*[E][E]*/) {
+                         const double* __restrict__ wtab, int y_begin, int y_end, uint8_t* __restrict__ out /*[Ey][Ex]*/) {
   constexpr int NS = MC - 1;   // blend steps per direction
   __shared__ int s_n[SG_ROWS];
   __shared__ int s_bl[SG_ROWS][NS];
@@ -465,7 +466,7 @@ stitch_gray_strip_kernel(const uint8_t* __restrict__ mosaic, int mos_h, int mos_
     const int Y = yb + threadIdx.x;
     const int qy = Y / g.S, ry = Y - qy * g.S;
     int i0, i1;
-    cover_range(g, qy, ry, dW, eW, i0, i1);
+    cover_range(g.ny, qy, ry, dW, eW, i0, i1);
     int nb = i1 - i0;
     if (nb > NS) nb = NS;
     s_n[threadIdx.x] = nb;
@@ -483,7 +484,7 @@ stitch_gray_strip_kernel(const uint8_t* __restrict__ mosaic, int mos_h, int mos_
   }
   __syncthreads();
   const int X0 = (blockIdx.x * SG_THREADS + threadIdx.x) * V;
-  if (X0 >= g.E) return;
+  if (X0 >= g.Ex) return;
   int nbx[V], blx[V][NS];
   double wx[V][NS], omwx[V][NS];
   {
@@ -491,7 +492,7 @@ stitch_gray_strip_kernel(const uint8_t* __restrict__ mosaic, int mos_h, int mos_
 #pragma unroll
     for (int u = 0; u < V; ++u) {
       int j0, j1;
-      cover_range(g, q, r, dW, eW, j0, j1);
+      cover_range(g.nx, q, r, dW, eW, j0, j1);
       nbx[u] = min(j1 - j0, NS);
 #pragma unroll
       for (int s2 = 0; s2 < NS; ++s2) {
@@ -531,7 +532,7 @@ stitch_gray_strip_kernel(const uint8_t* __restrict__ mosaic, int mos_h, int mos_
         if (s2 < nb) v = s_bl[t][s2] ? blend_u8_pre(v, hv, s_w[t][s2], s_omw[t][s2]) : hv;
       res[u] = v;
     }
-    const long long o = static_cast<long long>(Y) * g.E + X0;
+    const long long o = static_cast<long long>(Y) * g.Ex + X0;
     if (V == 4) *reinterpret_cast<uchar4*>(out + o) = make_uchar4(res[0], res[1 % V], res[2 % V], res[3 % V]);
     else out[o] = res[0];
   }
@@ -545,9 +546,9 @@ __device__ __forceinline__ float blend_f32(float a, float b, double w) {
 __device__ __forceinline__ float stitched_value(const float* __restrict__ lowres, const StitchGeom& g,
                                                 const double* __restrict__ wtab, int Y, int X) {
   int j0 = (X - g.W + g.S) / g.S; if (X - g.W + 1 <= 0) j0 = 0; if (j0 < 0) j0 = 0;
-  const int j1 = min(X / g.S, g.n - 1);
+  const int j1 = min(X / g.S, g.nx - 1);
   int i0 = (Y - g.W + g.S) / g.S; if (Y - g.W + 1 <= 0) i0 = 0; if (i0 < 0) i0 = 0;
-  const int i1 = min(Y / g.S, g.n - 1);
+  const int i1 = min(Y / g.S, g.ny - 1);
   const int lsz = g.lh * g.lw;
   float v = 0.f;
   for (int i = i0; i <= i1; ++i) {
@@ -555,7 +556,7 @@ __device__ __forceinline__ float stitched_value(const float* __restrict__ lowres
     float hv = 0.f;
     for (int j = j0; j <= j1; ++j) {
       const int kx = X - j * g.S;
-      const float tv = bilinear_up(lowres + static_cast<long long>(i * g.n + j) * lsz, g.lh, g.lw, ky, kx, g.scale);
+      const float tv = bilinear_up(lowres + static_cast<long long>(i * g.nx + j) * lsz, g.lh, g.lw, ky, kx, g.scale);
       hv = (j > j0 && kx < g.step) ? blend_f32(hv, tv, wtab[kx]) : tv;
     }
     v = (i > i0 && ky < g.step) ? blend_f32(v, hv, wtab[ky]) : hv;
@@ -563,25 +564,25 @@ __device__ __forceinline__ float stitched_value(const float* __restrict__ lowres
   return v;
 }
 
-// concat_crops (SSS/sw_processing.py:113-134) on full-resolution float32 crops [n*n][W][W] -> out [E][E]
+// concat_crops (SSS/sw_processing.py:113-134) on full-resolution float32 crops [ny*nx][W][W] -> out [Ey][Ex]
 __global__ void concat_crops_f32_kernel(const float* __restrict__ crops, StitchGeom g, const double* __restrict__ wtab,
                                         float* __restrict__ out) {
-  const long long total = static_cast<long long>(g.E) * g.E;
+  const long long total = static_cast<long long>(g.Ey) * g.Ex;
   const long long tsz = static_cast<long long>(g.W) * g.W;
   for (long long idx = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; idx < total;
        idx += static_cast<long long>(gridDim.x) * blockDim.x) {
-    const int Y = static_cast<int>(idx / g.E), X = static_cast<int>(idx % g.E);
+    const int Y = static_cast<int>(idx / g.Ex), X = static_cast<int>(idx % g.Ex);
     int j0 = (X - g.W + g.S) / g.S; if (X - g.W + 1 <= 0) j0 = 0;
-    const int j1 = min(X / g.S, g.n - 1);
+    const int j1 = min(X / g.S, g.nx - 1);
     int i0 = (Y - g.W + g.S) / g.S; if (Y - g.W + 1 <= 0) i0 = 0;
-    const int i1 = min(Y / g.S, g.n - 1);
+    const int i1 = min(Y / g.S, g.ny - 1);
     float v = 0.f;
     for (int i = i0; i <= i1; ++i) {
       const int ky = Y - i * g.S;
       float hv = 0.f;
       for (int j = j0; j <= j1; ++j) {
         const int kx = X - j * g.S;
-        const float tv = crops[(i * g.n + j) * tsz + static_cast<long long>(ky) * g.W + kx];
+        const float tv = crops[(i * g.nx + j) * tsz + static_cast<long long>(ky) * g.W + kx];
         hv = (j > j0 && kx < g.step) ? blend_f32(hv, tv, wtab[kx]) : tv;
       }
       v = (i > i0 && ky < g.step) ? blend_f32(v, hv, wtab[ky]) : hv;
@@ -589,27 +590,27 @@ __global__ void concat_crops_f32_kernel(const float* __restrict__ crops, StitchG
     out[idx] = v;
   }
 }
-// same on uint8 crops [n*n][W][W][C] (HWC, as PIL / numpy image crops) -> out [E][E][C]
+// same on uint8 crops [ny*nx][W][W][C] (HWC, as PIL / numpy image crops) -> out [Ey][Ex][C]
 __global__ void concat_crops_u8_kernel(const uint8_t* __restrict__ crops, StitchGeom g, int C, const double* __restrict__ wtab,
                                        uint8_t* __restrict__ out) {
-  const long long total = static_cast<long long>(g.E) * g.E * C;
+  const long long total = static_cast<long long>(g.Ey) * g.Ex * C;
   const long long tsz = static_cast<long long>(g.W) * g.W * C;
   for (long long idx = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; idx < total;
        idx += static_cast<long long>(gridDim.x) * blockDim.x) {
     const int c = static_cast<int>(idx % C);
     const long long px = idx / C;
-    const int Y = static_cast<int>(px / g.E), X = static_cast<int>(px % g.E);
+    const int Y = static_cast<int>(px / g.Ex), X = static_cast<int>(px % g.Ex);
     int j0 = (X - g.W + g.S) / g.S; if (X - g.W + 1 <= 0) j0 = 0;
-    const int j1 = min(X / g.S, g.n - 1);
+    const int j1 = min(X / g.S, g.nx - 1);
     int i0 = (Y - g.W + g.S) / g.S; if (Y - g.W + 1 <= 0) i0 = 0;
-    const int i1 = min(Y / g.S, g.n - 1);
+    const int i1 = min(Y / g.S, g.ny - 1);
     uint8_t v = 0;
     for (int i = i0; i <= i1; ++i) {
       const int ky = Y - i * g.S;
       uint8_t hv = 0;
       for (int j = j0; j <= j1; ++j) {
         const int kx = X - j * g.S;
-        const uint8_t tv = crops[(i * g.n + j) * tsz + (static_cast<long long>(ky) * g.W + kx) * C + c];
+        const uint8_t tv = crops[(i * g.nx + j) * tsz + (static_cast<long long>(ky) * g.W + kx) * C + c];
         hv = (j > j0 && kx < g.step) ? blend_u8(hv, tv, wtab[kx]) : tv;
       }
       v = (i > i0 && ky < g.step) ? blend_u8(v, hv, wtab[ky]) : hv;
@@ -729,7 +730,7 @@ struct RowCtx {
 };
 __device__ __forceinline__ void make_row_ctx(const StitchGeom& g, int Y, RowCtx& rc) {
   const int q = Y / g.S, r = Y - q * g.S;
-  cover_range(g, q, r, g.W / g.S, g.W % g.S, rc.i0, rc.i1);
+  cover_range(g.ny, q, r, g.W / g.S, g.W % g.S, rc.i0, rc.i1);
   if (rc.i1 - rc.i0 > 3) rc.i1 = rc.i0 + 3;   // (host guarantees W <= 4 S)
   for (int k = 0; k <= rc.i1 - rc.i0; ++k) {
     rc.ky[k] = Y - (rc.i0 + k) * g.S;
@@ -739,7 +740,7 @@ __device__ __forceinline__ void make_row_ctx(const StitchGeom& g, int Y, RowCtx&
 __device__ __forceinline__ float stitched_value_row(const float* __restrict__ lowres, const StitchGeom& g, const double* __restrict__ wtab,
                                                     const LinTab* __restrict__ tab, const RowCtx& rc, int q, int r, int dW, int eW) {
   int j0, j1;
-  cover_range(g, q, r, dW, eW, j0, j1);
+  cover_range(g.nx, q, r, dW, eW, j0, j1);
   const int lsz = g.lh * g.lw;
   float v = 0.f;
   for (int k = 0; k <= rc.i1 - rc.i0; ++k) {
@@ -748,7 +749,7 @@ __device__ __forceinline__ float stitched_value_row(const float* __restrict__ lo
     for (int j = j0; j <= j1; ++j) {
       const int kx = (q - j) * g.S + r;
       const LinTab t = tab[kx];
-      const float tv = bilinear_tab(lowres + static_cast<long long>(i * g.n + j) * lsz, g.lw, rc.y0[k], rc.y1[k], rc.fy[k], t.s0, t.s1, t.f);
+      const float tv = bilinear_tab(lowres + static_cast<long long>(i * g.nx + j) * lsz, g.lw, rc.y0[k], rc.y1[k], rc.fy[k], t.s0, t.s1, t.f);
       hv = (j > j0 && kx < g.step) ? blend_f32(hv, tv, __ldg(wtab + kx)) : tv;
     }
     v = (k > 0 && rc.ky[k] < g.step) ? blend_f32(v, hv, __ldg(wtab + rc.ky[k])) : hv;
@@ -766,8 +767,8 @@ __device__ __forceinline__ int st_x0() { return (blockIdx.x * ST_THREADS + threa
 template <int V>
 __global__ void __launch_bounds__(ST_THREADS)
 stitch_minmax_kernel(const float* __restrict__ lowres, StitchGeom g, const double* __restrict__ wtab, int y_begin, int y_end,
-                     int* __restrict__ minmax_ord, float* __restrict__ map_out /*[E][E] or null*/,
-                     const float* __restrict__ map_in /*[E][E] or null: use instead of stitching lowres*/) {
+                     int* __restrict__ minmax_ord, float* __restrict__ map_out /*[Ey][Ex] or null*/,
+                     const float* __restrict__ map_in /*[Ey][Ex] or null: use instead of stitching lowres*/) {
   __shared__ LinTab tab[ST_MAX_W];
   __shared__ float red_mn[ST_THREADS / 32], red_mx[ST_THREADS / 32];
   if (map_in == nullptr) {
@@ -777,11 +778,11 @@ stitch_minmax_kernel(const float* __restrict__ lowres, StitchGeom g, const doubl
   const int X0 = st_x0<V>();
   const int dW = g.W / g.S, eW = g.W % g.S;
   float mn = INFINITY, mx = -INFINITY;
-  if (X0 < g.E) {
+  if (X0 < g.Ex) {
     const int q0 = X0 / g.S, r0 = X0 - q0 * g.S;
     for (int Y = y_begin + blockIdx.y; Y < y_end; Y += gridDim.y) {
       float v[V];
-      const long long off = static_cast<long long>(Y) * g.E + X0;
+      const long long off = static_cast<long long>(Y) * g.Ex + X0;
       if (map_in != nullptr) {
         if (V == 4) {
           const float4 t = *reinterpret_cast<const float4*>(map_in + off);
@@ -846,7 +847,7 @@ __device__ __forceinline__ float blend_f32_pre(float a, float b, double w, doubl
 template <int MC>
 __global__ void __launch_bounds__(SC_THREADS)
 stitch_strip_kernel(const float* __restrict__ lowres, StitchGeom g, const double* __restrict__ wtab, int y_begin, int y_end,
-                    int* __restrict__ minmax_ord, float* __restrict__ map_out /*[E][E] or null*/) {
+                    int* __restrict__ minmax_ord, float* __restrict__ map_out /*[Ey][Ex] or null*/) {
   __shared__ StripRow<MC> rows[SC_ROWS];
   __shared__ float red_mn[SC_THREADS / 32], red_mx[SC_THREADS / 32];
   const int yb = y_begin + blockIdx.y * SC_ROWS;
@@ -858,7 +859,7 @@ stitch_strip_kernel(const float* __restrict__ lowres, StitchGeom g, const double
     StripRow<MC>& R = rows[threadIdx.x];
     const int q = Y / g.S, r = Y - q * g.S;
     int i0, i1;
-    cover_range(g, q, r, dW, eW, i0, i1);
+    cover_range(g.ny, q, r, dW, eW, i0, i1);
     if (i1 - i0 > MC - 1) i1 = i0 + MC - 1;
     R.ni = i1 - i0 + 1;
 #pragma unroll
@@ -868,8 +869,8 @@ stitch_strip_kernel(const float* __restrict__ lowres, StitchGeom g, const double
         int y0, y1;
         float fy;
         linear_coeff(ky, g.scale, g.lh, y0, y1, fy);
-        R.base0[k] = i * g.n * lsz + y0 * g.lw;
-        R.base1[k] = i * g.n * lsz + y1 * g.lw;
+        R.base0[k] = i * g.nx * lsz + y0 * g.lw;
+        R.base1[k] = i * g.nx * lsz + y1 * g.lw;
         R.fy[k] = fy;
         R.b0[k] = __fsub_rn(1.0f, fy);
         R.blend[k] = (k > 0 && ky < g.step) ? 1 : 0;
@@ -881,7 +882,7 @@ stitch_strip_kernel(const float* __restrict__ lowres, StitchGeom g, const double
   }
   __syncthreads();
   const int X = blockIdx.x * SC_THREADS + threadIdx.x;
-  const bool live = X < g.E;
+  const bool live = X < g.Ex;
   int nj = 0;
   int o0[MC], o1[MC], bl[MC];
   float fx[MC], a0[MC];
@@ -889,7 +890,7 @@ stitch_strip_kernel(const float* __restrict__ lowres, StitchGeom g, const double
   if (live) {
     const int q = X / g.S, r = X - q * g.S;
     int j0, j1;
-    cover_range(g, q, r, dW, eW, j0, j1);
+    cover_range(g.nx, q, r, dW, eW, j0, j1);
     if (j1 - j0 > MC - 1) j1 = j0 + MC - 1;
     nj = j1 - j0 + 1;
 #pragma unroll
@@ -945,7 +946,7 @@ stitch_strip_kernel(const float* __restrict__ lowres, StitchGeom g, const double
     if (live) {
       mn = fminf(mn, v);
       mx = fmaxf(mx, v);
-      if (map_out != nullptr) map_out[static_cast<long long>(yb + t) * g.E + X] = v;
+      if (map_out != nullptr) map_out[static_cast<long long>(yb + t) * g.Ex + X] = v;
     }
   }
   for (int o = 16; o > 0; o >>= 1) {
@@ -976,7 +977,7 @@ template <int V>
 __device__ __forceinline__ void st_load_px(const float* __restrict__ lowres, const StitchGeom& g, const double* __restrict__ wtab,
                                            const LinTab* __restrict__ tab, const float* __restrict__ map_in, const uint8_t* __restrict__ gray,
                                            int Y, int X0, int q0, int r0, float (&v)[V], int (&img)[V]) {
-  const long long off = static_cast<long long>(Y) * g.E + X0;
+  const long long off = static_cast<long long>(Y) * g.Ex + X0;
   if (map_in != nullptr) {
     if (V == 4) {
       const float4 t = *reinterpret_cast<const float4*>(map_in + off);
@@ -1008,7 +1009,7 @@ __device__ __forceinline__ void st_load_px(const float* __restrict__ lowres, con
 template <int V>
 __global__ void __launch_bounds__(ST_THREADS)
 stitch_hist_kernel(const float* __restrict__ lowres, StitchGeom g, const double* __restrict__ wtab,
-                   const uint8_t* __restrict__ gray /*[E][E]*/, const int* __restrict__ minmax_ord, int y_begin, int y_end,
+                   const uint8_t* __restrict__ gray /*[Ey][Ex]*/, const int* __restrict__ minmax_ord, int y_begin, int y_end,
                    unsigned long long* __restrict__ hists, const float* __restrict__ map_in) {
   __shared__ LinTab tab[ST_MAX_W];
   __shared__ unsigned int h[ST_THREADS / 32][3][256];
@@ -1022,7 +1023,7 @@ stitch_hist_kernel(const float* __restrict__ lowres, StitchGeom g, const double*
   const float att_max = flat ? mx : 1.0f;  // np.max(attention) after min_max_normalize
   const int X0 = st_x0<V>();
   unsigned int (*hw)[256] = h[threadIdx.x >> 5];
-  if (X0 < g.E) {
+  if (X0 < g.Ex) {
     const int q0 = X0 / g.S, r0 = X0 - q0 * g.S;
     for (int Y = y_begin + blockIdx.y; Y < y_end; Y += gridDim.y) {
       float v[V];
@@ -1048,7 +1049,7 @@ stitch_hist_kernel(const float* __restrict__ lowres, StitchGeom g, const double*
 }
 
 // pass 3: masks th (result > t0), th2 (gray > t1), th3 (att_u8 > t2); rows [y_begin, y_end) written at
-// out + (Y - y_begin) * E so that a rank can hold only its own band.
+// out + (Y - y_begin) * Ex so that a rank can hold only its own band.
 template <int V>
 __global__ void __launch_bounds__(ST_THREADS)
 stitch_mask_kernel(const float* __restrict__ lowres, StitchGeom g, const double* __restrict__ wtab,
@@ -1066,7 +1067,7 @@ stitch_mask_kernel(const float* __restrict__ lowres, StitchGeom g, const double*
   const float att_max = flat ? mx : 1.0f;
   const int t0 = thr[0], t1 = thr[1], t2 = thr[2];
   const int X0 = st_x0<V>();
-  if (X0 >= g.E) return;
+  if (X0 >= g.Ex) return;
   const int q0 = X0 / g.S, r0 = X0 - q0 * g.S;
   for (int Y = y_begin + blockIdx.y; Y < y_end; Y += gridDim.y) {
     float v[V];
@@ -1081,7 +1082,7 @@ stitch_mask_kernel(const float* __restrict__ lowres, StitchGeom g, const double*
       m1[u] = img[u] > t1 ? 255 : 0;
       m2[u] = au > t2 ? 255 : 0;
     }
-    const long long o = static_cast<long long>(Y - y_begin) * g.E + X0;
+    const long long o = static_cast<long long>(Y - y_begin) * g.Ex + X0;
     if (V == 4) {
       if (th != nullptr) *reinterpret_cast<uchar4*>(th + o) = make_uchar4(m0[0], m0[1 % V], m0[2 % V], m0[3 % V]);
       if (th2 != nullptr) *reinterpret_cast<uchar4*>(th2 + o) = make_uchar4(m1[0], m1[1 % V], m1[2 % V], m1[3 % V]);
@@ -1111,13 +1112,13 @@ stitch_result_kernel(const float* __restrict__ lowres, StitchGeom g, const doubl
   const float range = __fsub_rn(mx, mn);
   const float att_max = flat ? mx : 1.0f;
   const int X0 = st_x0<V>();
-  if (X0 >= g.E) return;
+  if (X0 >= g.Ex) return;
   const int q0 = X0 / g.S, r0 = X0 - q0 * g.S;
   for (int Y = y_begin + blockIdx.y; Y < y_end; Y += gridDim.y) {
     float v[V];
     int img[V];
     st_load_px<V>(lowres, g, wtab, tab, map_in, gray, Y, X0, q0, r0, v, img);
-    const long long o = static_cast<long long>(Y - y_begin) * g.E + X0;
+    const long long o = static_cast<long long>(Y - y_begin) * g.Ex + X0;
 #pragma unroll
     for (int u = 0; u < V; ++u) {
       int res, au;

@@ -6,6 +6,7 @@
 #include <cuda_runtime.h>
 
 #include <atomic>
+#include <climits>
 #include <cstdarg>
 #include <cstdio>
 #include <cstdlib>
@@ -774,7 +775,7 @@ int run_layernorm(const float* X, const float* g, const float* b, void* out_bf16
 struct MosaicSrc {
   const uint8_t* p;
   long long pitch;
-  int h, w, n, S, t0;
+  int h, w, nx, S, t0;   // nx: windows per grid row (window t has origin ((t / nx) S, (t % nx) S))
 };
 
 int run_patch_embed(const vitocm_engine* e, const float* x, int B, int H, int W, const float* pos, const float* mask,
@@ -787,7 +788,7 @@ int run_patch_embed(const vitocm_engine* e, const float* x, int B, int H, int W,
   if (p % 8 != 0 || K % GEMM_BK != 0) return fail(VITOCM_ERR_INVALID, "patch embedding needs patch %% 8 == 0 and C*p*p %% 64 == 0 (patch %d, chans %d)", p, C);
   if ((mos == nullptr && (reinterpret_cast<uintptr_t>(x) & 15) != 0) || (reinterpret_cast<uintptr_t>(pos) & 15) != 0)
     return fail(VITOCM_ERR_INVALID, "patch embedding inputs must be 16-byte aligned");
-  if (mos != nullptr && (!gray || mos->p == nullptr || mos->n < 1 || mos->S < 1))
+  if (mos != nullptr && (!gray || mos->p == nullptr || mos->nx < 1 || mos->S < 1))
     return fail(VITOCM_ERR_INVALID, "mosaic ingest needs the gray path and a valid window grid");
   const float* mask_token = e->w("mask_token");
   if (mask != nullptr && mask_token == nullptr) return fail(VITOCM_ERR_STATE, "mask given but mask_token was never loaded");
@@ -803,7 +804,7 @@ int run_patch_embed(const vitocm_engine* e, const float* x, int B, int H, int W,
   a.M = M; a.N = D; a.kblocks = K / GEMM_BK; a.nterms = 3; a.lo_k = K; a.a_lo_mask = 4; a.b_lo_mask = 2; a.f16 = e->f16;   // split precision in all modes
   a.bias = e->w("patch_embed.proj.bias");
   a.img = x; a.img_h = H; a.img_w = W; a.patch = p; a.n_patches = n; a.pos = pos; a.mask = mask; a.mask_token = mask_token; a.out_f32 = X;
-  if (mos != nullptr) { a.mos = mos->p; a.mos_pitch = mos->pitch; a.mos_h = mos->h; a.mos_w = mos->w; a.mos_n = mos->n; a.mos_S = mos->S; a.mos_t0 = mos->t0; }
+  if (mos != nullptr) { a.mos = mos->p; a.mos_pitch = mos->pitch; a.mos_h = mos->h; a.mos_w = mos->w; a.mos_nx = mos->nx; a.mos_S = mos->S; a.mos_t0 = mos->t0; }
   // position rows in / token rows out through TMA boxes (VITOCM_PATCH_TMA=0: every lane reads and writes its own 128 bytes)
   static const int patch_tma = [] { const char* v = getenv("VITOCM_PATCH_TMA"); return v == nullptr ? 1 : atoi(v); }();
   CUtensorMap tx = tb, tp = tb;
@@ -1203,12 +1204,25 @@ int vitocm_forward_cls_attn_gray(vitocm_engine* e, const float* x, int B, int H,
   return forward_rows(e, x, B, H, W, pos, nullptr, 1, out_rows, nullptr, ws, ws_bytes, chunk_tiles, stream, true);
 }
 
+// windows [t0, t0 + T) of an ny x nx grid
+static int check_windows(const char* fn, int ny, int nx, int W, int S, int t0, int T) {
+  if (ny < 1 || nx < 1 || S < 1 || W < 1 || t0 < 0 || T < 0 || static_cast<long long>(t0) + T > static_cast<long long>(ny) * nx)
+    return fail(VITOCM_ERR_INVALID, "%s: bad window grid %dx%d W=%d S=%d tiles [%d, %lld)", fn, ny, nx, W, S, t0, static_cast<long long>(t0) + T);
+  return 0;
+}
+
+int vitocm_forward_cls_attn_mosaic_grid(vitocm_engine* e, const uint8_t* mosaic, int mos_h, int mos_w, int64_t pitch, int ny, int nx, int W,
+                                        int S, int t0, int T, const float* pos, float* out_rows, void* ws, size_t ws_bytes, int chunk_tiles,
+                                        void* stream) {
+  if (mosaic == nullptr) return fail(VITOCM_ERR_INVALID, "forward_cls_attn_mosaic: mosaic is NULL");
+  TRY(check_windows("forward_cls_attn_mosaic", ny, nx, W, S, t0, T));
+  const MosaicSrc src{mosaic, static_cast<long long>(pitch), mos_h, mos_w, nx, S, t0};
+  return forward_rows(e, nullptr, T, W, W, pos, nullptr, 1, out_rows, nullptr, ws, ws_bytes, chunk_tiles, stream, true, &src);
+}
+
 int vitocm_forward_cls_attn_mosaic(vitocm_engine* e, const uint8_t* mosaic, int mos_h, int mos_w, int64_t pitch, int n, int W, int S, int t0,
                                    int T, const float* pos, float* out_rows, void* ws, size_t ws_bytes, int chunk_tiles, void* stream) {
-  if (mosaic == nullptr || n < 1 || S < 1 || W < 1 || t0 < 0 || T < 0 || t0 + T > n * n)
-    return fail(VITOCM_ERR_INVALID, "forward_cls_attn_mosaic: bad window grid n=%d W=%d S=%d tiles [%d, %d)", n, W, S, t0, t0 + T);
-  const MosaicSrc src{mosaic, static_cast<long long>(pitch), mos_h, mos_w, n, S, t0};
-  return forward_rows(e, nullptr, T, W, W, pos, nullptr, 1, out_rows, nullptr, ws, ws_bytes, chunk_tiles, stream, true, &src);
+  return vitocm_forward_cls_attn_mosaic_grid(e, mosaic, mos_h, mos_w, pitch, n, n, W, S, t0, T, pos, out_rows, ws, ws_bytes, chunk_tiles, stream);
 }
 
 int vitocm_forward_cls_attn(vitocm_engine* e, const float* x, int B, int H, int W, const float* pos, float* out_rows,
@@ -1469,20 +1483,26 @@ static int grid_for(long long total, int block) {
   return static_cast<int>(g < 1 ? 1 : (g > cap ? cap : g));
 }
 
-int vitocm_extract_tiles(const uint8_t* mosaic, int mos_h, int mos_w, int64_t pitch, int n, int W, int S, int t0, int T, int C,
-                         float* x, void* stream) {
+int vitocm_extract_tiles_grid(const uint8_t* mosaic, int mos_h, int mos_w, int64_t pitch, int ny, int nx, int W, int S, int t0, int T, int C,
+                              float* x, void* stream) {
   if (T <= 0) return 0;
+  TRY(check_windows("extract_tiles", ny, nx, W, S, t0, T));
   const long long total = static_cast<long long>(T) * W * W;
   ProfScope prof(PC_POST, static_cast<cudaStream_t>(stream));
-  extract_tiles_kernel<<<grid_for(total, 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(mosaic, mos_h, mos_w, pitch, n, W, S, t0, T, C, x);
+  extract_tiles_kernel<<<grid_for(total, 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(mosaic, mos_h, mos_w, pitch, nx, W, S, t0, T, C, x);
   LAUNCH_CHECK();
   return 0;
 }
 
+int vitocm_extract_tiles(const uint8_t* mosaic, int mos_h, int mos_w, int64_t pitch, int n, int W, int S, int t0, int T, int C,
+                         float* x, void* stream) {
+  return vitocm_extract_tiles_grid(mosaic, mos_h, mos_w, pitch, n, n, W, S, t0, T, C, x, stream);
+}
+
 // Row-organised mosaic kernels: grid.x covers one row in groups of 256 * V pixels (V = 4 when every row of every buffer is
-// 16-byte aligned, i.e. E % 4 == 0 and aligned bases, else 1); grid.y strides over the rows of the band, ~8 blocks per SM
+// 16-byte aligned, i.e. Ex % 4 == 0 and aligned bases, else 1); grid.y strides over the rows of the band, ~8 blocks per SM
 struct StitchLaunch { dim3 grid; int V; };
-static StitchLaunch stitch_launch(int E, int rows, int num_sms, std::initializer_list<const void*> f32_ptrs, std::initializer_list<const void*> u8_ptrs) {
+static StitchLaunch stitch_launch(int E /*row length Ex*/, int rows, int num_sms, std::initializer_list<const void*> f32_ptrs, std::initializer_list<const void*> u8_ptrs) {
   bool vec = (E % 4) == 0;
   for (const void* p : f32_ptrs) if (p != nullptr && (reinterpret_cast<uintptr_t>(p) & 15) != 0) vec = false;
   for (const void* p : u8_ptrs) if (p != nullptr && (reinterpret_cast<uintptr_t>(p) & 3) != 0) vec = false;
@@ -1511,31 +1531,33 @@ static int check_tab(const void* map_in, int W) {
   return 0;
 }
 
-static StitchGeom make_geom(int n, int W, int S, int lh, int lw) {
+static StitchGeom make_geom(int ny, int nx, int W, int S, int lh, int lw) {
   StitchGeom g;
-  g.n = n; g.W = W; g.S = S; g.step = W - S; g.E = (n - 1) * S + W; g.lh = lh; g.lw = lw;
+  g.ny = ny; g.nx = nx; g.W = W; g.S = S; g.step = W - S; g.Ey = (ny - 1) * S + W; g.Ex = (nx - 1) * S + W; g.lh = lh; g.lw = lw;
   g.scale = static_cast<double>(lw) / static_cast<double>(W);
   return g;
 }
-static int check_geom(int n, int W, int S, int y_begin, int y_end) {
-  if (n < 1 || S < 1 || W <= S) return fail(VITOCM_ERR_INVALID, "bad sliding-window geometry n=%d W=%d S=%d", n, W, S);
+static int check_geom(int ny, int nx, int W, int S, int y_begin, int y_end) {
+  if (ny < 1 || nx < 1 || S < 1 || W <= S) return fail(VITOCM_ERR_INVALID, "bad sliding-window geometry %dx%d W=%d S=%d", ny, nx, W, S);
   if (W > 4 * S) return fail(VITOCM_ERR_INVALID, "sliding-window geometry W=%d S=%d: at most four windows may overlap (W <= 4 S)", W, S);
-  const int E = (n - 1) * S + W;
-  if (y_begin < 0 || y_end > E || y_begin > y_end) return fail(VITOCM_ERR_INVALID, "bad row band [%d,%d) for extent %d", y_begin, y_end, E);
+  const long long Ey = static_cast<long long>(ny - 1) * S + W, Ex = static_cast<long long>(nx - 1) * S + W;
+  if (Ey > INT_MAX || Ex > INT_MAX || Ey * Ex > (1LL << 40))
+    return fail(VITOCM_ERR_INVALID, "sliding-window grid %dx%d at stride %d: extent %lldx%lld too large", ny, nx, S, Ey, Ex);
+  if (y_begin < 0 || y_end > Ey || y_begin > y_end) return fail(VITOCM_ERR_INVALID, "bad row band [%d,%d) for extent %lld", y_begin, y_end, Ey);
   return 0;
 }
 
-int vitocm_stitch_gray(const uint8_t* mosaic, int mos_h, int mos_w, int64_t pitch, int n, int W, int S, const double* wtab,
-                       int y_begin, int y_end, uint8_t* out, void* stream) {
-  TRY(check_geom(n, W, S, y_begin, y_end));
+int vitocm_stitch_gray_grid(const uint8_t* mosaic, int mos_h, int mos_w, int64_t pitch, int ny, int nx, int W, int S, const double* wtab,
+                            int y_begin, int y_end, uint8_t* out, void* stream) {
+  TRY(check_geom(ny, nx, W, S, y_begin, y_end));
   if (y_end == y_begin) return 0;
-  const StitchGeom g = make_geom(n, W, S, 1, 1);
+  const StitchGeom g = make_geom(ny, nx, W, S, 1, 1);
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   ProfScope prof(PC_POST, st);
-  const StitchLaunch L = stitch_launch(g.E, y_end - y_begin, device_sms(), {}, {out});
+  const StitchLaunch L = stitch_launch(g.Ex, y_end - y_begin, device_sms(), {}, {out});
   static const int strip = [] { const char* v = getenv("VITOCM_STITCH_STRIP"); return v == nullptr ? 1 : atoi(v); }();
   if (strip) {   // column-strip kernels (VITOCM_STITCH_STRIP=0: the row-organised ones)
-    const dim3 grid((g.E + SG_THREADS * L.V - 1) / (SG_THREADS * L.V), (y_end - y_begin + SG_ROWS - 1) / SG_ROWS);
+    const dim3 grid((g.Ex + SG_THREADS * L.V - 1) / (SG_THREADS * L.V), (y_end - y_begin + SG_ROWS - 1) / SG_ROWS);
     if (L.V == 4 && W <= 2 * S) stitch_gray_strip_kernel<4, 2><<<grid, SG_THREADS, 0, st>>>(mosaic, mos_h, mos_w, pitch, g, wtab, y_begin, y_end, out);
     else if (L.V == 4) stitch_gray_strip_kernel<4, 4><<<grid, SG_THREADS, 0, st>>>(mosaic, mos_h, mos_w, pitch, g, wtab, y_begin, y_end, out);
     else if (W <= 2 * S) stitch_gray_strip_kernel<1, 2><<<grid, SG_THREADS, 0, st>>>(mosaic, mos_h, mos_w, pitch, g, wtab, y_begin, y_end, out);
@@ -1549,50 +1571,65 @@ int vitocm_stitch_gray(const uint8_t* mosaic, int mos_h, int mos_w, int64_t pitc
   return 0;
 }
 
+int vitocm_stitch_gray(const uint8_t* mosaic, int mos_h, int mos_w, int64_t pitch, int n, int W, int S, const double* wtab,
+                       int y_begin, int y_end, uint8_t* out, void* stream) {
+  return vitocm_stitch_gray_grid(mosaic, mos_h, mos_w, pitch, n, n, W, S, wtab, y_begin, y_end, out, stream);
+}
+
 int vitocm_minmax_init(int* minmax_ord, void* stream) {
   const int init[2] = {0x7fffffff, static_cast<int>(0x80000000u)};
   CUDA_TRY(cudaMemcpyAsync(minmax_ord, init, sizeof(init), cudaMemcpyHostToDevice, static_cast<cudaStream_t>(stream)));
   return 0;
 }
 
-int vitocm_stitch_minmax(const float* lowres, int n, int W, int S, int lh, int lw, const double* wtab, int y_begin, int y_end,
-                         int* minmax_ord, float* map_out, const float* map_in, void* stream) {
-  TRY(check_geom(n, W, S, y_begin, y_end));
+int vitocm_stitch_minmax_grid(const float* lowres, int ny, int nx, int W, int S, int lh, int lw, const double* wtab, int y_begin, int y_end,
+                              int* minmax_ord, float* map_out, const float* map_in, void* stream) {
+  TRY(check_geom(ny, nx, W, S, y_begin, y_end));
   TRY(check_tab(map_in, W));
   if (y_end == y_begin) return 0;
-  const StitchGeom g = make_geom(n, W, S, lh, lw);
+  const StitchGeom g = make_geom(ny, nx, W, S, lh, lw);
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   ProfScope prof(PC_POST, st);
   // stitched from the low-res maps: column-strip kernel (VITOCM_STITCH_STRIP=0: the row-organised one)
   static const int strip = [] { const char* v = getenv("VITOCM_STITCH_STRIP"); return v == nullptr ? 1 : atoi(v); }();
   if (map_in == nullptr && strip) {
-    const dim3 grid((g.E + SC_THREADS - 1) / SC_THREADS, (y_end - y_begin + SC_ROWS - 1) / SC_ROWS);
+    const dim3 grid((g.Ex + SC_THREADS - 1) / SC_THREADS, (y_end - y_begin + SC_ROWS - 1) / SC_ROWS);
     if (W <= 2 * S) stitch_strip_kernel<2><<<grid, SC_THREADS, 0, st>>>(lowres, g, wtab, y_begin, y_end, minmax_ord, map_out);
     else stitch_strip_kernel<4><<<grid, SC_THREADS, 0, st>>>(lowres, g, wtab, y_begin, y_end, minmax_ord, map_out);
     LAUNCH_CHECK();
     return 0;
   }
-  const StitchLaunch L = stitch_launch(g.E, y_end - y_begin, device_sms(), {map_out, map_in}, {});
+  const StitchLaunch L = stitch_launch(g.Ex, y_end - y_begin, device_sms(), {map_out, map_in}, {});
   if (L.V == 4) stitch_minmax_kernel<4><<<L.grid, ST_THREADS, 0, st>>>(lowres, g, wtab, y_begin, y_end, minmax_ord, map_out, map_in);
   else stitch_minmax_kernel<1><<<L.grid, ST_THREADS, 0, st>>>(lowres, g, wtab, y_begin, y_end, minmax_ord, map_out, map_in);
   LAUNCH_CHECK();
   return 0;
 }
 
-int vitocm_stitch_hist(const float* lowres, int n, int W, int S, int lh, int lw, const double* wtab, const uint8_t* gray,
-                       const int* minmax_ord, int y_begin, int y_end, uint64_t* hists, const float* map_in, void* stream) {
-  TRY(check_geom(n, W, S, y_begin, y_end));
+int vitocm_stitch_minmax(const float* lowres, int n, int W, int S, int lh, int lw, const double* wtab, int y_begin, int y_end,
+                         int* minmax_ord, float* map_out, const float* map_in, void* stream) {
+  return vitocm_stitch_minmax_grid(lowres, n, n, W, S, lh, lw, wtab, y_begin, y_end, minmax_ord, map_out, map_in, stream);
+}
+
+int vitocm_stitch_hist_grid(const float* lowres, int ny, int nx, int W, int S, int lh, int lw, const double* wtab, const uint8_t* gray,
+                            const int* minmax_ord, int y_begin, int y_end, uint64_t* hists, const float* map_in, void* stream) {
+  TRY(check_geom(ny, nx, W, S, y_begin, y_end));
   TRY(check_tab(map_in, W));
   if (y_end == y_begin) return 0;
-  const StitchGeom g = make_geom(n, W, S, lh, lw);
+  const StitchGeom g = make_geom(ny, nx, W, S, lh, lw);
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   ProfScope prof(PC_POST, st);
-  const StitchLaunch L = stitch_launch(g.E, y_end - y_begin, device_sms(), {map_in}, {gray});
+  const StitchLaunch L = stitch_launch(g.Ex, y_end - y_begin, device_sms(), {map_in}, {gray});
   unsigned long long* h = reinterpret_cast<unsigned long long*>(hists);
   if (L.V == 4) stitch_hist_kernel<4><<<L.grid, ST_THREADS, 0, st>>>(lowres, g, wtab, gray, minmax_ord, y_begin, y_end, h, map_in);
   else stitch_hist_kernel<1><<<L.grid, ST_THREADS, 0, st>>>(lowres, g, wtab, gray, minmax_ord, y_begin, y_end, h, map_in);
   LAUNCH_CHECK();
   return 0;
+}
+
+int vitocm_stitch_hist(const float* lowres, int n, int W, int S, int lh, int lw, const double* wtab, const uint8_t* gray,
+                       const int* minmax_ord, int y_begin, int y_end, uint64_t* hists, const float* map_in, void* stream) {
+  return vitocm_stitch_hist_grid(lowres, n, n, W, S, lh, lw, wtab, gray, minmax_ord, y_begin, y_end, hists, map_in, stream);
 }
 
 int vitocm_otsu(const uint64_t* hists, int nhist, int* thresholds, void* stream) {
@@ -1603,53 +1640,73 @@ int vitocm_otsu(const uint64_t* hists, int nhist, int* thresholds, void* stream)
   return 0;
 }
 
-int vitocm_stitch_mask(const float* lowres, int n, int W, int S, int lh, int lw, const double* wtab, const uint8_t* gray,
-                       const int* minmax_ord, const int* thr, int y_begin, int y_end, uint8_t* th, uint8_t* th2, uint8_t* th3,
-                       const float* map_in, void* stream) {
-  TRY(check_geom(n, W, S, y_begin, y_end));
+int vitocm_stitch_mask_grid(const float* lowres, int ny, int nx, int W, int S, int lh, int lw, const double* wtab, const uint8_t* gray,
+                            const int* minmax_ord, const int* thr, int y_begin, int y_end, uint8_t* th, uint8_t* th2, uint8_t* th3,
+                            const float* map_in, void* stream) {
+  TRY(check_geom(ny, nx, W, S, y_begin, y_end));
   TRY(check_tab(map_in, W));
   if (y_end == y_begin) return 0;
-  const StitchGeom g = make_geom(n, W, S, lh, lw);
+  const StitchGeom g = make_geom(ny, nx, W, S, lh, lw);
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   ProfScope prof(PC_POST, st);
-  const StitchLaunch L = stitch_launch(g.E, y_end - y_begin, device_sms(), {map_in}, {gray, th, th2, th3});
+  const StitchLaunch L = stitch_launch(g.Ex, y_end - y_begin, device_sms(), {map_in}, {gray, th, th2, th3});
   if (L.V == 4) stitch_mask_kernel<4><<<L.grid, ST_THREADS, 0, st>>>(lowres, g, wtab, gray, minmax_ord, thr, y_begin, y_end, th, th2, th3, map_in);
   else stitch_mask_kernel<1><<<L.grid, ST_THREADS, 0, st>>>(lowres, g, wtab, gray, minmax_ord, thr, y_begin, y_end, th, th2, th3, map_in);
   LAUNCH_CHECK();
   return 0;
 }
 
-int vitocm_stitch_result(const float* lowres, int n, int W, int S, int lh, int lw, const double* wtab, const uint8_t* gray,
-                         const int* minmax_ord, int y_begin, int y_end, uint8_t* result, uint8_t* att_u8, const float* map_in, void* stream) {
-  TRY(check_geom(n, W, S, y_begin, y_end));
+int vitocm_stitch_mask(const float* lowres, int n, int W, int S, int lh, int lw, const double* wtab, const uint8_t* gray,
+                       const int* minmax_ord, const int* thr, int y_begin, int y_end, uint8_t* th, uint8_t* th2, uint8_t* th3,
+                       const float* map_in, void* stream) {
+  return vitocm_stitch_mask_grid(lowres, n, n, W, S, lh, lw, wtab, gray, minmax_ord, thr, y_begin, y_end, th, th2, th3, map_in, stream);
+}
+
+int vitocm_stitch_result_grid(const float* lowres, int ny, int nx, int W, int S, int lh, int lw, const double* wtab, const uint8_t* gray,
+                              const int* minmax_ord, int y_begin, int y_end, uint8_t* result, uint8_t* att_u8, const float* map_in,
+                              void* stream) {
+  TRY(check_geom(ny, nx, W, S, y_begin, y_end));
   TRY(check_tab(map_in, W));
   if (y_end == y_begin) return 0;
-  const StitchGeom g = make_geom(n, W, S, lh, lw);
+  const StitchGeom g = make_geom(ny, nx, W, S, lh, lw);
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   ProfScope prof(PC_POST, st);
-  const StitchLaunch L = stitch_launch(g.E, y_end - y_begin, device_sms(), {map_in}, {gray});
+  const StitchLaunch L = stitch_launch(g.Ex, y_end - y_begin, device_sms(), {map_in}, {gray});
   if (L.V == 4) stitch_result_kernel<4><<<L.grid, ST_THREADS, 0, st>>>(lowres, g, wtab, gray, minmax_ord, y_begin, y_end, result, att_u8, map_in);
   else stitch_result_kernel<1><<<L.grid, ST_THREADS, 0, st>>>(lowres, g, wtab, gray, minmax_ord, y_begin, y_end, result, att_u8, map_in);
   LAUNCH_CHECK();
   return 0;
 }
 
-int vitocm_concat_crops_f32(const float* crops, int n, int W, int S, const double* wtab, float* out, void* stream) {
-  TRY(check_geom(n, W, S, 0, 0));
-  const StitchGeom g = make_geom(n, W, S, 1, 1);
+int vitocm_stitch_result(const float* lowres, int n, int W, int S, int lh, int lw, const double* wtab, const uint8_t* gray,
+                         const int* minmax_ord, int y_begin, int y_end, uint8_t* result, uint8_t* att_u8, const float* map_in, void* stream) {
+  return vitocm_stitch_result_grid(lowres, n, n, W, S, lh, lw, wtab, gray, minmax_ord, y_begin, y_end, result, att_u8, map_in, stream);
+}
+
+int vitocm_concat_crops_grid_f32(const float* crops, int ny, int nx, int W, int S, const double* wtab, float* out, void* stream) {
+  TRY(check_geom(ny, nx, W, S, 0, 0));
+  const StitchGeom g = make_geom(ny, nx, W, S, 1, 1);
   ProfScope prof(PC_POST, static_cast<cudaStream_t>(stream));
-  concat_crops_f32_kernel<<<grid_for(static_cast<long long>(g.E) * g.E, 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(crops, g, wtab, out);
+  concat_crops_f32_kernel<<<grid_for(static_cast<long long>(g.Ey) * g.Ex, 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(crops, g, wtab, out);
+  LAUNCH_CHECK();
+  return 0;
+}
+
+int vitocm_concat_crops_f32(const float* crops, int n, int W, int S, const double* wtab, float* out, void* stream) {
+  return vitocm_concat_crops_grid_f32(crops, n, n, W, S, wtab, out, stream);
+}
+
+int vitocm_concat_crops_grid_u8(const uint8_t* crops, int ny, int nx, int W, int S, int C, const double* wtab, uint8_t* out, void* stream) {
+  TRY(check_geom(ny, nx, W, S, 0, 0));
+  const StitchGeom g = make_geom(ny, nx, W, S, 1, 1);
+  ProfScope prof(PC_POST, static_cast<cudaStream_t>(stream));
+  concat_crops_u8_kernel<<<grid_for(static_cast<long long>(g.Ey) * g.Ex * C, 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(crops, g, C, wtab, out);
   LAUNCH_CHECK();
   return 0;
 }
 
 int vitocm_concat_crops_u8(const uint8_t* crops, int n, int W, int S, int C, const double* wtab, uint8_t* out, void* stream) {
-  TRY(check_geom(n, W, S, 0, 0));
-  const StitchGeom g = make_geom(n, W, S, 1, 1);
-  ProfScope prof(PC_POST, static_cast<cudaStream_t>(stream));
-  concat_crops_u8_kernel<<<grid_for(static_cast<long long>(g.E) * g.E * C, 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(crops, g, C, wtab, out);
-  LAUNCH_CHECK();
-  return 0;
+  return vitocm_concat_crops_grid_u8(crops, n, n, W, S, C, wtab, out, stream);
 }
 
 int vitocm_crop_u8(const uint8_t* img, int img_h, int img_w, int C, int ny, int nx, int W, int S, uint8_t* crops, void* stream) {

@@ -374,10 +374,12 @@ class VisionTransformer(nn.Module):
         return out
 
     @torch.no_grad()
-    def cls_attention_rows_mosaic(self, mosaic: torch.Tensor, grid: int, window: int, stride: int, t0: int, count: int) -> torch.Tensor:
-        """cls_attention_rows of the windows t0 .. t0+count-1 (row-major in the grid x grid sliding-window grid,
-        SSS/sw_processing.py:151-163) of a gray uint8 CUDA mosaic, cut out by the patch-embedding producer itself: no crop
-        is ever materialised.  -> [count, heads, N] fp32."""
+    def cls_attention_rows_mosaic(self, mosaic: torch.Tensor, grid, window: int, stride: int, t0: int, count: int) -> torch.Tensor:
+        """cls_attention_rows of the windows t0 .. t0+count-1 (row-major in the sliding-window grid, SSS/sw_processing.py:151-163)
+        of a gray uint8 CUDA mosaic, cut out by the patch-embedding producer itself: no crop is ever materialised.  grid: n for an
+        n x n grid, or (ny, nx) for a rectangular one (ny rows of windows over the height, nx columns over the width; window t
+        has origin ((t // nx) * stride, (t % nx) * stride)).  -> [count, heads, N] fp32."""
+        ny, nx = (grid, grid) if isinstance(grid, int) else (int(grid[0]), int(grid[1]))
         if isinstance(mosaic, tuple):      # (device address of row 0, height, width, pitch, device): a band buffer addressed by absolute rows
             mos_ptr, mos_h, mos_w, pitch, dev = mosaic
         else:
@@ -395,9 +397,9 @@ class VisionTransformer(nn.Module):
         chunk = max(1, min(self.chunk_tiles, count))
         ws = self._workspace(chunk, N, dev)
         out = torch.empty(count, self.num_heads, N, dtype=torch.float32, device=dev)
-        check(_lib.load_library().vitocm_forward_cls_attn_mosaic(eng, mos_ptr, mos_h, mos_w, pitch, grid,
-                                                                 window, stride, t0, count, ptr(pos), ptr(out), ptr(ws), ws.numel(), chunk,
-                                                                 cur_stream()))
+        check(_lib.load_library().vitocm_forward_cls_attn_mosaic_grid(eng, mos_ptr, mos_h, mos_w, pitch, ny, nx,
+                                                                      window, stride, t0, count, ptr(pos), ptr(out), ptr(ws), ws.numel(), chunk,
+                                                                      cur_stream()))
         return out
 
     @torch.no_grad()
