@@ -332,7 +332,7 @@ int vitocm_layernorm(vitocm_engine* e, const float* X, const float* gamma, const
  * `stream` without synchronising.  The first use still needs one vitocm_finalize_weights. */
 int vitocm_bind_weight(vitocm_engine* e, const char* name, float* dev_data, int64_t numel);
 int vitocm_refresh_weights(vitocm_engine* e, void* stream);
-/* Where vitocm_mim_backward ACCUMULATES dL/d(name) (fp32, same shape as the parameter; the caller zeroes it, like
+/* Where vitocm_mim_backward and vitocm_encoder_backward ACCUMULATE dL/d(name) (fp32, same shape as the parameter; the caller zeroes it, like
  * optimizer.zero_grad(), mim.py:173).  NULL unbinds. */
 int vitocm_bind_grad(vitocm_engine* e, const char* name, float* dev_grad);
 
@@ -359,6 +359,24 @@ int vitocm_mim_backward(vitocm_engine* e, const float* x, int B, int H, int W, c
  * last kernel does.  vitocm_stream_wait_event(stream, event) = cudaStreamWaitEvent, for callers without a CUDA binding. */
 int vitocm_mim_backward_events(vitocm_engine* e, void** events, int n);
 int vitocm_stream_wait_event(void* stream, void* event);
+
+/* ---- Encoder training under any loss: fine-tuning (SSS/finetune.py, heads SSS/model.py:110-174) and DINO's linear evaluation on
+ * get_intermediate_layers (vit.py:248-256).  16-bit engines only, no decoder weights needed; ws sized by
+ * vitocm_mim_train_workspace_bytes(e, B, N). ---- */
+/* forward_feats / get_intermediate_layers(x, n_out) (vit.py:198-223, 248-256) for one batch, keeping the activations the backward
+ * needs in ws: feats [n_out][B][N][D] fp32 = norm(x_l) of the last n_out blocks (slab n_out - 1 = the last block), CLS row
+ * included.  pos [N][D] fp32: the (interpolated) position table, as in vitocm_prepare_tokens. */
+int vitocm_encoder_train_forward(vitocm_engine* e, const float* x, int B, int H, int W, const float* pos, int n_out, float* feats,
+                                 void* ws, size_t ws_bytes, void* stream);
+/* Backward of the vitocm_encoder_train_forward that last ran on the same ws, for the upstream gradient dfeats [n_out][B][N][D]
+ * fp32 (DEVICE): parameter gradients are ACCUMULATED into the buffers bound with vitocm_bind_grad (every encoder parameter except
+ * pos_embed; mask_token and the decoder are not touched), dpos [N][D] is WRITTEN, and so is dx [B][C][H][W] fp32 unless dx is NULL.
+ * fp16 engines: S = 2^e is picked on the device from max |dfeats| so that max |dfeats| S lies in [1, 2) (S = 1 for an all-zero
+ * upstream) and undone exactly as in vitocm_mim_backward.  The events of vitocm_mim_backward_events are recorded here too; with
+ * n_out > 1 the gradients of norm.* complete with block depth - n_out + 1's event instead of events[depth].  The first call with
+ * dx adds a transposed copy of the patch filter to the engine's repack (one extra refresh, then kept up to date by it). */
+int vitocm_encoder_backward(vitocm_engine* e, const float* x, int B, int H, int W, int n_out, const float* dfeats, float* dpos,
+                            float* dx, void* ws, size_t ws_bytes, void* stream);
 
 /* torch.nn.utils.clip_grad_norm_ (mim.py:176), first half: out[0] = sum g^2 over a flat fp32 gradient buffer (fp64). */
 int vitocm_grad_sumsq(const float* g, int64_t n, double* out, void* stream);

@@ -111,6 +111,10 @@ SIGNATURES = {
     "vitocm_mim_backward": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
                                     c_size_t, c_void_p]),
     "vitocm_mim_backward_events": (c_int, [c_void_p, c_void_p, c_int]),
+    "vitocm_encoder_train_forward": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_int, c_void_p, c_void_p, c_size_t,
+                                             c_void_p]),
+    "vitocm_encoder_backward": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p,
+                                        c_size_t, c_void_p]),
     "vitocm_stream_wait_event": (c_int, [c_void_p, c_void_p]),
     "vitocm_grad_sumsq": (c_int, [c_void_p, c_int64, c_void_p, c_void_p]),
     "vitocm_grad_clip": (c_int, [c_void_p, c_int64, c_float, c_void_p, c_void_p]),

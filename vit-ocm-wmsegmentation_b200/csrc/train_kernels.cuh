@@ -37,6 +37,19 @@ __device__ __forceinline__ float h16hi(uint32_t v) {
 // and nothing else: every scaled 16-bit tensor keeps its bits.  The value of K0 and the headroom it leaves: DESIGN.md §6.
 constexpr int LOSS_SCALE_K0 = 0;
 
+// exponent e of the loss scale S = 2^e for a gradient of magnitude a: a S in [2^LOSS_SCALE_K0, 2^(LOSS_SCALE_K0 + 1)); 0 (S = 1)
+// when a is 0 or not finite
+__device__ __forceinline__ int loss_scale_exp(float a) {
+  int e = 0;
+  if (a != 0.f && isfinite(a)) {
+    int ex;
+    frexpf(a, &ex);                          // |a| = f 2^ex, f in [0.5, 1)
+    e = LOSS_SCALE_K0 + 1 - ex;
+    e = e < -126 ? -126 : (e > 126 ? 126 : e);
+  }
+  return e;
+}
+
 // ------------------------------------------------------------------------------------------------ LayerNorm backward
 // One warp per row (grid-stride).  y = (x - mean) * rstd * gamma + beta,  dy = dL/dy (bf16):
 //   g = dy * gamma;  dx = rstd * (g - mean(g) - xhat * mean(g * xhat))
@@ -243,13 +256,7 @@ mim_loss_bwd_kernel(const float* __restrict__ x, const float* __restrict__ x_rec
   const int Wp = W / p, n = (H / p) * Wp, ldy = C * p * p, groups = ldy / 8;
   float coef = (gscale != nullptr ? *gscale : 1.0f) / (static_cast<float>(sums[1] + 1e-5) * static_cast<float>(C));
   if (F16) {
-    int e = 0;
-    if (coef != 0.f && isfinite(coef)) {
-      int ex;
-      frexpf(coef, &ex);                     // |coef| = f 2^ex, f in [0.5, 1)
-      e = LOSS_SCALE_K0 + 1 - ex;
-      e = e < -126 ? -126 : (e > 126 ? 126 : e);
-    }
+    const int e = loss_scale_exp(coef);
     const float S = __int_as_float((127 + e) << 23), inv = __int_as_float((127 - e) << 23);
     coef *= S;                               // exact
     if (blockIdx.x == 0 && threadIdx.x == 0 && lscale != nullptr) {
@@ -283,8 +290,48 @@ mim_loss_bwd_kernel(const float* __restrict__ x, const float* __restrict__ x_rec
   }
 }
 
+// ------------------------------------------------------------------------------------------------ encoder gradient seeding
+// vitocm_encoder_backward: the caller's upstream gradient dfeats (fp32) becomes the 16-bit dy of the final norm's backward.
+// amax_bits[0] = max |g| as float bits (non-negative floats order like their bit patterns; NaN orders above +inf).  Zeroed by
+// the caller.
+__global__ void __launch_bounds__(256)
+grad_amax_kernel(const float4* __restrict__ g, long long n4, unsigned* __restrict__ amax_bits) {
+  unsigned m = 0u;
+  for (long long i = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; i < n4;
+       i += static_cast<long long>(gridDim.x) * blockDim.x) {
+    const float4 v = g[i];
+    m = max(m, max(max(__float_as_uint(v.x) & 0x7fffffffu, __float_as_uint(v.y) & 0x7fffffffu),
+                   max(__float_as_uint(v.z) & 0x7fffffffu, __float_as_uint(v.w) & 0x7fffffffu)));
+  }
+  for (int o = 16; o > 0; o >>= 1) m = max(m, __shfl_xor_sync(0xffffffffu, m, o));
+  if ((threadIdx.x & 31) == 0) atomicMax(amax_bits, m);
+}
+
+// out[i] = 16-bit(g[i] * S).  F16: S = 2^loss_scale_exp(amax) from grad_amax_kernel's result (S = 1 for an all-zero or non-finite
+// gradient), written with 1 / S to lscale[0], lscale[1] as mim_loss_bwd_kernel does; a power-of-two change of g changes S and
+// nothing else.  bf16: S = 1, nothing read or written besides g and out.
+template <bool F16 = false>
+__global__ void __launch_bounds__(256)
+seed_grad_kernel(const float4* __restrict__ g, long long n4, const unsigned* __restrict__ amax_bits, __nv_bfloat16* __restrict__ out,
+                 float* __restrict__ lscale) {
+  float S = 1.0f;
+  if (F16) {
+    const int e = loss_scale_exp(__uint_as_float(*amax_bits));
+    S = __int_as_float((127 + e) << 23);
+    if (blockIdx.x == 0 && threadIdx.x == 0) {
+      lscale[0] = S;
+      lscale[1] = __int_as_float((127 - e) << 23);
+    }
+  }
+  for (long long i = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; i < n4;
+       i += static_cast<long long>(gridDim.x) * blockDim.x) {
+    const float4 v = g[i];
+    *reinterpret_cast<uint2*>(out + 4 * i) = make_uint2(ptx::pack_h2<F16>(v.x * S, v.y * S), ptx::pack_h2<F16>(v.z * S, v.w * S));
+  }
+}
+
 // ------------------------------------------------------------------------------------------------ token-embedding backward
-// G[b*n + i][:] = 16-bit((1 - mask[b, i]) * dX0[b, 1 + i, :])    (model.py:31-33: only unmasked patches see the conv)
+// G[b*n + i][:] = 16-bit((1 - mask[b, i]) * dX0[b, 1 + i, :])    (model.py:31-33: only unmasked patches see the conv; mask NULL: 0)
 template <bool F16 = false>
 __global__ void __launch_bounds__(256)
 patch_grad_rows_kernel(const float4* __restrict__ dX0, const float* __restrict__ mask, __nv_bfloat16* __restrict__ G, int B, int n, int D) {
@@ -295,7 +342,7 @@ patch_grad_rows_kernel(const float4* __restrict__ dX0, const float* __restrict__
     const long long m = idx / nvec;
     const int c = static_cast<int>(idx - m * nvec);
     const int b = static_cast<int>(m / n), i = static_cast<int>(m - static_cast<long long>(b) * n);
-    const float w = 1.0f - mask[m];
+    const float w = mask != nullptr ? 1.0f - mask[m] : 1.0f;
     const float4 v = dX0[(static_cast<long long>(b) * (n + 1) + 1 + i) * nvec + c];
     *reinterpret_cast<uint2*>(G + m * D + 4 * c) = make_uint2(ptx::pack_h2<F16>(v.x * w, v.y * w), ptx::pack_h2<F16>(v.z * w, v.w * w));
   }
@@ -321,7 +368,28 @@ im2col_bf16_kernel(const float* __restrict__ x, __nv_bfloat16* __restrict__ P, i
   }
 }
 
-// dpos[t][:] = sum_b dX0[b, t, :];  dcls += dpos[0];  dmask_token += sum_{b, i} mask[b, i] * dX0[b, 1 + i, :]
+// inverse of im2col_bf16_kernel for the input gradient: dx[b, c, py p + yi, px p + xi] = dP[b*n + py*Wp + px][c p^2 + yi p + xi] *
+// (*inv_scale, NULL: 1).  Patches do not overlap, so every pixel has exactly one source: a permutation, no atomics.
+__global__ void __launch_bounds__(256)
+col2im_dx_kernel(const float* __restrict__ dP, float* __restrict__ dx, int B, int C, int H, int W, int p, const float* __restrict__ inv_scale) {
+  const int Wp = W / p, n = (H / p) * Wp, K = C * p * p, groups = K / 8;
+  const float s = inv_scale != nullptr ? *inv_scale : 1.0f;
+  const long long total = static_cast<long long>(B) * n * groups;
+  for (long long idx = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; idx < total;
+       idx += static_cast<long long>(gridDim.x) * blockDim.x) {
+    const long long m = idx / groups;
+    const int k = static_cast<int>(idx - m * groups) * 8;
+    const int b = static_cast<int>(m / n), i = static_cast<int>(m - static_cast<long long>(b) * n);
+    const int py = i / Wp, px = i - py * Wp;
+    const int c = k / (p * p), rem = k - c * p * p, yi = rem / p, xi = rem - yi * p;
+    const float4 a = *reinterpret_cast<const float4*>(dP + m * K + k), bq = *reinterpret_cast<const float4*>(dP + m * K + k + 4);
+    float* dst = dx + ((static_cast<long long>(b) * C + c) * H + py * p + yi) * W + px * p + xi;
+    *reinterpret_cast<float4*>(dst) = make_float4(a.x * s, a.y * s, a.z * s, a.w * s);
+    *reinterpret_cast<float4*>(dst + 4) = make_float4(bq.x * s, bq.y * s, bq.z * s, bq.w * s);
+  }
+}
+
+// dpos[t][:] = sum_b dX0[b, t, :];  dcls += dpos[0];  dmask_token += sum_{b, i} mask[b, i] * dX0[b, 1 + i, :]  (mask NULL: no mix)
 // one thread per (token t, float4 column group), looping over the batch.  F16: dX0 carries the loss scale; the sums are
 // multiplied by lscale[1] = 1 / S
 template <bool F16 = false>
@@ -337,7 +405,7 @@ token_grad_kernel(const float4* __restrict__ dX0, const float* __restrict__ mask
   for (int b = 0; b < B; ++b) {
     const float4 v = dX0[(static_cast<long long>(b) * (n + 1) + t) * nvec + c];
     s.x += v.x; s.y += v.y; s.z += v.z; s.w += v.w;
-    if (t > 0) {
+    if (t > 0 && mask != nullptr) {
       const float w = mask[static_cast<long long>(b) * n + t - 1];
       sm.x += w * v.x; sm.y += w * v.y; sm.z += w * v.z; sm.w += w * v.w;
     }
@@ -434,7 +502,7 @@ adamw_kernel(float* __restrict__ p, float* __restrict__ g, float* __restrict__ m
 // bf16 [C][R] (input-gradient B operand).  blockIdx.x walks 32 x 32 tiles; the table gives each matrix its first tile.
 struct RepackEntry {
   const float* src;
-  __nv_bfloat16* dst;     // [R][C]
+  __nv_bfloat16* dst;     // [R][C] or nullptr
   __nv_bfloat16* dst_t;   // [C][R] or nullptr
   int R, C;
   int tile0;              // index of this matrix's first tile
@@ -458,8 +526,10 @@ repack_weights_kernel(const RepackEntry* __restrict__ table, int n_entries, int 
     float v = 0.f;
     if (r < e.R && c < e.C) {
       v = e.src[static_cast<long long>(r) * e.C + c];
-      if (f16) reinterpret_cast<__half*>(e.dst)[static_cast<long long>(r) * e.C + c] = __float2half_rn(ptx::f16_round(v));
-      else e.dst[static_cast<long long>(r) * e.C + c] = __float2bfloat16_rn(v);
+      if (e.dst != nullptr) {
+        if (f16) reinterpret_cast<__half*>(e.dst)[static_cast<long long>(r) * e.C + c] = __float2half_rn(ptx::f16_round(v));
+        else e.dst[static_cast<long long>(r) * e.C + c] = __float2bfloat16_rn(v);
+      }
     }
     tile[k][tx] = v;
   }

@@ -175,6 +175,8 @@ struct vitocm_engine {
   DevBuf patch_w_gray_f32, patch_w_gray;   // the filter summed over input channels, fp32 [D][p*p] and bf16 [D][2 p*p]: gray fast path
   DevBuf dec_w;     // MIM decoder 1x1 conv weight, bf16 [C p^2][D * parts] (present iff "decoder.0.weight" was loaded)
   DevBuf dec_w_t;   // bf16 [D][C p^2] (training)
+  DevBuf patch_w_t;          // 16-bit [C p^2][D]: the transposed patch filter, B operand of the input-gradient GEMM
+  bool patch_w_t_on = false; // set by the first vitocm_encoder_backward that asks for dx; the repack keeps patch_w_t from then on
   DevBuf repack_table;   // RepackEntry[] for the one-launch repack of the Linear weights (bf16 engines)
   int repack_entries = 0, repack_tiles = 0;
   std::vector<const void*> repack_key;   // the pointers the table was built for
@@ -1087,6 +1089,12 @@ static int repack_weights(vitocm_engine* e, cudaStream_t st) {
     TRY(need("decoder.0.bias", dec_rows));
     if (S) TRY(pack(e->dec_w, e->w("decoder.0.weight"), static_cast<int>(dec_rows), D, S));
     else TRY(add_entry(e->dec_w, e->dec_w_t, e->w("decoder.0.weight"), static_cast<int>(dec_rows), D));
+  }
+  if (e->patch_w_t_on && !S) {   // transposed copy only: the forward reads the filter as hi | lo (patch_w)
+    TRY(e->patch_w_t.alloc(static_cast<size_t>(D) * K * 2));
+    RepackEntry en{e->w("patch_embed.proj.weight"), nullptr, e->patch_w_t.as<__nv_bfloat16>(), D, K, total_tiles, (K + 31) / 32};
+    total_tiles += ((D + 31) / 32) * en.tiles_c;
+    entries.push_back(en);
   }
   if (!entries.empty()) {
     std::vector<const void*> key;

@@ -63,13 +63,17 @@ class VisionTransformerForSimMIM(VisionTransformer):
             tensor.uniform_(2 * lo - 1, 2 * hi - 1).erfinv_().mul_(std * math.sqrt(2.0)).add_(mean).clamp_(min=-std, max=std)
         return tensor
 
-    def _mim_pos(self, x):
+    def _mim_pos_args(self, x):
+        """(npatch, w, h) of the position table for input x: resized to img_size when that is not 224."""
         size = self.img_size[0] if isinstance(self.img_size, (list, tuple)) else self.img_size
         B, _, H, W = x.shape
         n = (H // self.patch_embed.patch_size) * (W // self.patch_embed.patch_size)
         if size != 224:
-            return self._pos_table(n, size, size)
-        return self._pos_table(self.pos_embed.shape[1] - 1, 224, 224)
+            return n, size, size
+        return self.pos_embed.shape[1] - 1, 224, 224
+
+    def _mim_pos(self, x):
+        return self._pos_table(*self._mim_pos_args(x))
 
     @torch.no_grad()
     def forward(self, x, mask):
@@ -91,21 +95,6 @@ class VisionTransformerForSimMIM(VisionTransformer):
 
     # NB: like the reference's encoder (SSS/model.py:11-53, vit.py:135-258) this class has no ``no_weight_decay``: the
     # skip list of build_pretrain_optimizer is empty and cls_token / pos_embed / mask_token (3-D) do get weight decay.
-
-    def _mim_pos_graph(self, x):
-        """The position table as a differentiable function of ``pos_embed`` (training): [N, D] on x's device."""
-        size = self.img_size[0] if isinstance(self.img_size, (list, tuple)) else self.img_size
-        pos = self.pos_embed
-        if size == 224:
-            return pos[0]
-        p = self.patch_embed.patch_size
-        N = pos.shape[1] - 1
-        dim = pos.shape[-1]
-        w0 = h0 = size // p + 0.1
-        s_ = int(math.sqrt(N))
-        grid = nn.functional.interpolate(pos[:, 1:].reshape(1, s_, s_, dim).permute(0, 3, 1, 2),
-                                         scale_factor=(w0 / math.sqrt(N), h0 / math.sqrt(N)), mode="bicubic")
-        return torch.cat((pos[:, :1], grid.permute(0, 2, 3, 1).reshape(1, -1, dim)), dim=1)[0]
 
 
 class _MIMStep(torch.autograd.Function):
@@ -178,7 +167,6 @@ class MIM(nn.Module):
         self._param_list = None      # [(engine name, parameter)] in flat-buffer order
         self._pflat = self._gflat = None
         self._grad_views = None
-        self._grads_bound_to = None
         self._flat_ptrs = None
         self._overlap_group = None   # overlap_grad_allreduce(): process group (or True = WORLD) for the bucketed all-reduce
         self._overlap = False
@@ -221,7 +209,7 @@ class MIM(nn.Module):
         self._pflat, self._gflat, self._grad_views, self._flat_offsets = pflat, gflat, views, offs
         self._param_list = [(self._engine_name(n), p) for n, p in named]
         self._flat_ptrs = tuple(p.data_ptr() for _, p in named)
-        self._grads_bound_to = None
+        self.encoder._grads_bound_to = None
         self.encoder._bind_weights = True
         return self
 
@@ -253,13 +241,14 @@ class MIM(nn.Module):
                     g.copy_(p.grad)
                 p.grad = g
         eng = self.encoder._engine
-        key = (eng.value, self._gflat.data_ptr())
-        if self._grads_bound_to != key:
+        # the binding cache lives on the encoder: a differentiable encoder call on the same engine rebinds to its own buffers
+        key = ("mim", eng.value, self._gflat.data_ptr())
+        if self.encoder._grads_bound_to != key:
             lib = _lib.load_library()
             for (name, p), g in zip(self._param_list, self._grad_views):
                 if name != "pos_embed":
                     check(lib.vitocm_bind_grad(eng, name.encode(), g.data_ptr()))
-            self._grads_bound_to = key
+            self.encoder._grads_bound_to = key
 
     def overlap_grad_allreduce(self, enabled: bool = True, group=None):
         """Data-parallel training: launch the gradient all-reduce from INSIDE the next backward(s), one bucket per transformer
@@ -339,7 +328,7 @@ class MIM(nn.Module):
         xx = enc._check_input(x)
         B = xx.shape[0]
         N = enc._tokens(xx)
-        pos = enc._mim_pos_graph(xx)
+        pos = enc._pos_graph(*enc._mim_pos_args(xx))
         assert pos.shape[0] == N, "position table does not match the token count (img_size vs input size)"
         m = mask.detach().reshape(B, -1).to(device=xx.device, dtype=torch.float32).contiguous()
         loss, x_rec = _MIMStep.apply(self, xx, m, pos, *[p for _, p in self._param_list])

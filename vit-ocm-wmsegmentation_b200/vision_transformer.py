@@ -210,7 +210,11 @@ class VisionTransformer(nn.Module):
         self._engine_key = None
         self._pos_cache = {}
         self._ws = None
-        self._zero_qkv_bias = torch.zeros(3 * embed_dim)
+        # a buffer so that it follows .cuda() and the engine can bind it in place like the parameters (training)
+        self.register_buffer("_zero_qkv_bias", torch.zeros(3 * embed_dim), persistent=False)
+        self._train_ws = None          # the differentiable forward's saved activations (vitocm_encoder_train_forward)
+        self._train_ws_gen = 0
+        self._grads_bound_to = None    # MIM's gradient buffers when they are the ones bound (vitocm_bind_grad); None otherwise
 
     # ------------------------------------------------------------------ engine plumbing
     def _engine_params(self):
@@ -325,7 +329,14 @@ class VisionTransformer(nn.Module):
         hit = self._pos_cache.get(key)
         if hit is not None:
             return hit
-        pos = self.pos_embed.detach().to(device=dev, dtype=torch.float32)
+        table = self._pos_graph(npatch, w, h, self.pos_embed.detach().to(device=dev, dtype=torch.float32)).contiguous()
+        self._pos_cache[key] = table
+        return table
+
+    def _pos_graph(self, npatch: int, w: int, h: int, pos=None) -> torch.Tensor:
+        """vit.py:176-196 as torch operations on ``pos`` (default: ``pos_embed`` itself, so that the table is differentiable
+        with respect to it) -> [1 + npatch, D].  ``w``, ``h``: the input's dims 2 and 3, named as in the reference."""
+        pos = self.pos_embed if pos is None else pos
         N = pos.shape[1] - 1
         if not (npatch == N and w == h):
             p = self.patch_embed.patch_size
@@ -336,9 +347,7 @@ class VisionTransformer(nn.Module):
                                              scale_factor=(w0 / math.sqrt(N), h0 / math.sqrt(N)), mode="bicubic")
             assert int(w0) == grid.shape[-2] and int(h0) == grid.shape[-1]
             pos = torch.cat((pos[:, :1], grid.permute(0, 2, 3, 1).reshape(1, -1, dim)), dim=1)
-        table = pos[0].contiguous()
-        self._pos_cache[key] = table
-        return table
+        return pos[0]
 
     # ------------------------------------------------------------------ C-ABI calls
     def _check_input(self, x, allow_gray: bool = False):
@@ -472,10 +481,76 @@ class VisionTransformer(nn.Module):
         check(_lib.load_library().vitocm_final_norm(self._engine, ptr(X), ptr(out), B * N, cur_stream()))
         return out
 
+    # ------------------------------------------------------------------ training (fine-tuning, linear probing)
+    def _differentiable(self, x) -> bool:
+        """The gate of forward_feats / forward / get_intermediate_layers: with gradients enabled, a call is differentiable
+        when ``x`` requires grad or, in training mode, when an engine parameter does (MIM.forward's rule).  Every other call
+        (no_grad, eval(), frozen parameters) runs the inference path."""
+        if not torch.is_grad_enabled():
+            return False
+        if isinstance(x, torch.Tensor) and x.requires_grad:
+            return True
+        return self.training and (self.pos_embed.requires_grad or any(p.requires_grad for p in self._encoder_grad_params().values()))
+
+    def _encoder_grad_params(self):
+        """{engine name: parameter} of everything vitocm_encoder_backward writes a gradient for (pos_embed excepted: its gradient
+        is dpos, carried through the position-table graph).  A qkv bias that does not exist gets none."""
+        return {n: p for n, p in self._engine_params() if n != "mask_token" and not n.startswith("decoder.") and p is not self._zero_qkv_bias}
+
+    def _encoder_train(self, x, n_out: int):
+        """Differentiable [norm(x_l) for the last n_out blocks] through vitocm_encoder_train_forward / vitocm_encoder_backward."""
+        if parse_precision(self.precision, self.depth)[0] == "fp32":
+            raise _lib.VitocmError("vitocm: training runs on bf16 or fp16 engines only; build the encoder with precision='bf16' or "
+                                   "'fp16' (or call it under torch.no_grad() / .eval() for fp32-parity inference)")
+        if x.dim() == 4 and x.shape[1] == 1 and self.in_chans > 1:
+            raise _lib.VitocmError(f"vitocm: gray [B, 1, H, W] inputs have no backward; pass the {self.in_chans}-channel image, "
+                                   f"e.g. x.expand(-1, {self.in_chans}, -1, -1), or call under torch.no_grad()")
+        n_out = min(n_out, self.depth)            # as the reference: n > depth gives every block, n < 1 none
+        if n_out < 1:
+            return []
+        xx = self._check_input(x)
+        self._bind_weights = True                 # the optimizer updates the parameters in place: repack on the device
+        self._ensure_engine()
+        _, _, H, W = xx.shape
+        N = self._tokens(xx)
+        pos = self._pos_graph(N - 1, H, W)
+        named = self._encoder_grad_params()
+        feats = _EncoderStep.apply(self, x, xx, n_out, pos, tuple(named), *named.values())
+        return list(feats.unbind(0))
+
+    def _bind_encoder_grads(self, names, dev):
+        """A fresh zeroed flat fp32 buffer for one backward's parameter gradients (returned to autograd as views, so .grad may
+        keep them), bound to the engine for that backward only (see _unbind_encoder_grads).  Slots are 16-byte aligned; a missing
+        qkv bias accumulates into a scratch slot.  -> ({name: view} for ``names``, every bound name)."""
+        eng = self._engine
+        sizes = {n: p.numel() for n, p in self._engine_params() if n != "mask_token" and not n.startswith("decoder.")}
+        offs, total = {}, 0
+        for n, k in sizes.items():
+            offs[n] = total
+            total += (k + 3) // 4 * 4
+        flat = torch.zeros(total, dtype=torch.float32, device=dev)
+        lib = _lib.load_library()
+        self._grads_bound_to = None         # the next MIM backward rebinds its own buffers
+        for n, o in offs.items():
+            check(lib.vitocm_bind_grad(eng, n.encode(), flat.data_ptr() + 4 * o))
+        return {n: flat[offs[n]:offs[n] + sizes[n]] for n in names}, list(offs)
+
+    def _unbind_encoder_grads(self, bound):
+        """After the backward's launches: the engine must not keep addresses into a buffer that autograd may free (a later
+        backward that does not bind a name, e.g. MIM's with no qkv bias, then fails with 'no bound gradient buffer')."""
+        lib = _lib.load_library()
+        for n in bound:
+            check(lib.vitocm_bind_grad(self._engine, n.encode(), None))
+
     # ------------------------------------------------------------------ reference methods
-    @torch.no_grad()
     def forward_feats(self, x):
-        """vit.py:218-223 -> norm(x) [B, N, D]."""
+        """vit.py:218-223 -> norm(x) [B, N, D]; differentiable under the rule of ``_differentiable``."""
+        if self._differentiable(x):
+            return self._encoder_train(x, 1)[0]
+        return self._forward_feats(x)
+
+    @torch.no_grad()
+    def _forward_feats(self, x):
         X = self.prepare_tokens(x)
         self._run_blocks(X, 0, self.depth)
         return self._final_norm(X)
@@ -491,9 +566,14 @@ class VisionTransformer(nn.Module):
         self._run_blocks(X, 0, self.depth - 1)
         return self._attn_probs(X, self.depth - 1)[0]
 
-    @torch.no_grad()
     def get_intermediate_layers(self, x, n=1):
-        """vit.py:248-256 -> [norm(x_i)] for the n last blocks."""
+        """vit.py:248-256 -> [norm(x_i)] for the n last blocks; differentiable under the rule of ``_differentiable``."""
+        if self._differentiable(x):
+            return self._encoder_train(x, n)
+        return self._get_intermediate_layers(x, n)
+
+    @torch.no_grad()
+    def _get_intermediate_layers(self, x, n):
         X = self.prepare_tokens(x)
         outs = []
         for i in range(self.depth):
@@ -538,6 +618,57 @@ class VisionTransformer(nn.Module):
         attn = LazyAttention((B, H, N, N), lambda: full()[1][0], rows, row_fn=lambda q: self.attention_rows(x, [q])[:, :, 0, :])
         qkv = LazyTensor((3, B, H, N, D // H), lambda: full()[2][0])
         return [feat], [attn], [qkv]
+
+
+class _EncoderStep(torch.autograd.Function):
+    """feats [n_out, B, N, D] = norm(x_l) of the last n_out blocks, with vitocm_encoder_backward as the backward.  The parameters
+    are inputs, and their gradients come back through autograd, so .grad accumulation, hooks, optimizers and
+    torch.autograd.grad work as for any module.  ``x`` is an input for dx; ``xx`` is its fp32 contiguous copy the kernels read."""
+
+    @staticmethod
+    def forward(ctx, enc, x, xx, n_out, pos, names, *params):
+        lib = _lib.load_library()
+        eng = enc._engine
+        B, _, H, W = xx.shape
+        N = enc._tokens(xx)
+        need = int(lib.vitocm_mim_train_workspace_bytes(eng, B, N))
+        if enc._train_ws is None or enc._train_ws.numel() < need or enc._train_ws.device != xx.device:
+            enc._train_ws = None
+            enc._train_ws = torch.empty(need, dtype=torch.uint8, device=xx.device)
+        posc = pos.detach().to(torch.float32).contiguous()
+        feats = torch.empty(n_out, B, N, enc.embed_dim, dtype=torch.float32, device=xx.device)
+        check(lib.vitocm_encoder_train_forward(eng, ptr(xx), B, H, W, ptr(posc), n_out, ptr(feats), ptr(enc._train_ws),
+                                               enc._train_ws.numel(), cur_stream()))
+        # the saved activations live in the encoder's one training workspace: stamp it, so that a backward whose forward has since
+        # been overwritten by another differentiable forward fails loudly instead of producing wrong gradients
+        enc._train_ws_gen += 1
+        ctx.enc, ctx.ws_gen, ctx.n_out, ctx.names = enc, enc._train_ws_gen, n_out, names
+        ctx.pos_shape, ctx.x_dtype, ctx.shapes = tuple(pos.shape), x.dtype, [p.shape for p in params]
+        ctx.save_for_backward(xx)
+        return feats
+
+    @staticmethod
+    def backward(ctx, dfeats):
+        enc = ctx.enc
+        if torch.is_grad_enabled():
+            raise _lib.VitocmError("vitocm: the encoder's backward is not differentiable (double backward); "
+                                   "call backward() / torch.autograd.grad without create_graph=True")
+        if ctx.ws_gen != enc._train_ws_gen:
+            raise _lib.VitocmError("vitocm: the activations of this forward were overwritten by a later differentiable forward "
+                                   "(call backward() before the next forward, or run evaluation under torch.no_grad() / .eval())")
+        xx, = ctx.saved_tensors
+        B, C, H, W = xx.shape
+        dpos = torch.empty(ctx.pos_shape, dtype=torch.float32, device=xx.device)
+        dx = torch.empty_like(xx) if ctx.needs_input_grad[1] else None
+        dfe = dfeats.detach().to(torch.float32).contiguous()
+        grads, bound = enc._bind_encoder_grads(ctx.names, xx.device)
+        try:
+            check(_lib.load_library().vitocm_encoder_backward(enc._engine, ptr(xx), B, H, W, ctx.n_out, ptr(dfe), ptr(dpos), ptr(dx),
+                                                              ptr(enc._train_ws), enc._train_ws.numel(), cur_stream()))
+        finally:
+            enc._unbind_encoder_grads(bound)
+        param_grads = [grads[n].view(shape) for n, shape in zip(ctx.names, ctx.shapes)]
+        return (None, None if dx is None else dx.to(ctx.x_dtype), None, None, dpos, None, *param_grads)
 
 
 def vit_tiny(patch_size=16, **kwargs):
