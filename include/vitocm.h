@@ -285,7 +285,9 @@ int vitocm_concat_grid_f32(const float* src, int B, int cr, int C, int c0, int h
 /* ---- kernel-level entry points used by the tests / the bench roofline leg ---- */
 
 /* C = epilogue(A[M][K] . B[N][K]^T): A, B bf16 device (split: [rows][2K] = hi|lo); epilogue enum:
- * 0 bias->bf16, 1 bias+gelu->bf16, 2 bias + in-place fp32 residual add, 3 bias->fp32. */
+ * 0 bias->bf16, 1 bias+gelu->bf16, 2 bias + in-place fp32 residual add, 3 bias->fp32.
+ * split_out (16-bit outputs): 1 = out[:, lo_off:lo_off+N] also receives lo = v - 16-bit(v); 2 with epilogue 1 (the training fc1) =
+ * out[:, :N] = gelu(pre) and out[:, lo_off:lo_off+N] = pre = acc + bias, the GELU input the backward reads. */
 int vitocm_gemm(vitocm_engine* e, const void* A, int64_t lda, const void* B, int64_t ldb, int M, int N, int K,
                 int split_in, int epilogue, const float* bias, void* out, int64_t ldo, int split_out, int lo_off,
                 void* stream);
@@ -406,6 +408,23 @@ int vitocm_attention_fwd_lse(vitocm_engine* e, const void* qkv, int64_t ld, int 
 int vitocm_attention_bwd(vitocm_engine* e, const void* qkv, int64_t ld, const void* ctx, const void* dctx, int64_t ldc,
                          const float* lse2, float* delta, float* dqacc, void* dqkv, int64_t ldq, int B, int n_tokens,
                          void* stream);
+/* kernel-level: out[M][N] = (dY[M][K] . Wt[N][K]^T) * gelu'(pre[M][N]), all 16-bit in the engine's format (bf16 or fp16 engines):
+ * the input gradient of fc2 through the GELU as the training step computes it, the derivative of the GELU form the engine's
+ * forward uses.  pre [M][ld_pre] 16-byte aligned, ld_pre a multiple of 8 (the step passes HP + hidden with ld_pre = 2 hidden). */
+int vitocm_gemm_dgelu(vitocm_engine* e, const void* dY, int64_t ldy, const void* Wt, int64_t ldw, int M, int N, int K, const void* pre,
+                      int64_t ld_pre, void* out, int64_t ldo, void* stream);
+/* kernel-level: nn.LayerNorm backward with the engine's eps for rows X [M][D] fp32 and dy [M][ld_dy] (16-bit, the engine's format):
+ * dX [M][D] fp32 = (accumulate ? dX : 0) + dx;  dXb [M][D] = 16-bit(dX);  dgamma[D] += sum dy xhat;  dbeta[D] += sum dy;
+ * dbias_out[D] (or NULL) += column sums of the new dX.  fp16 engines: lscale = DEVICE [S, 1 / S], dy and dX carry S and the three
+ * column sums are multiplied by 1 / S (NULL: 1); bf16 engines ignore it.  D % 4 == 0, D <= 1024. */
+int vitocm_layernorm_bwd(vitocm_engine* e, const float* X, const void* dy, int64_t ld_dy, const float* gamma, float* dX, void* dXb,
+                         float* dgamma, float* dbeta, float* dbias_out, int accumulate, int M, int D, const float* lscale, void* stream);
+/* kernel-level: the loss gradient of vitocm_mim_backward, dY [B (n + 1)][C p^2] (16-bit, the engine's format; C and p from the engine,
+ * n = (H / p) (W / p)) = *grad_scale * mask * sign(x_rec - x) / ((loss_sums[1] + 1e-5) C) through PixelShuffle, 0 at ties and in CLS
+ * rows.  fp16 engines multiply it by the loss scale S described at vitocm_mim_backward and write [S, 1 / S] to lscale (DEVICE, or
+ * NULL).  16-bit engines only. */
+int vitocm_mim_loss_bwd(vitocm_engine* e, const float* x, const float* x_rec, const float* mask, const double* loss_sums,
+                        const float* grad_scale, int B, int H, int W, void* dY, float* lscale, void* stream);
 
 /* Diagnostics: SM-clock stamps of one CTA of the last vitocm_attention_bwd run under VITOCM_ABW_DEBUG=2: host int64
  * [role: softmax warp 0, MMA thread][query tile < 8][event < 8]. */

@@ -165,9 +165,12 @@ def _step_vs_oracle(cfg_init, cfg, img, batch, seed, scale_linear=1.0):
     return ref_loss.item(), out
 
 
-# (ViT-S/8 at batch 2 and 32, the reference's encoder, ViT-B width at 64^2, N = 5): fp16 against bf16 on the same inputs
+# (ViT-S/8 at batch 2, 32 and 84, the reference's encoder, ViT-B width at 64^2, N = 5): fp16 against bf16 on the same inputs.  At
+# batch 84 M = 65 940 tokens, so fc1 and the input gradient through the GELU run on CTA pairs (BN 192 at D = 384, 256 at D = 128).
 @pytest.mark.parametrize("D,heads,depth,img,batch", [pytest.param(384, 6, 12, 224, 2, id="vit-small-b2"),
                                                      pytest.param(384, 6, 2, 224, 32, id="vit-small-b32"),
+                                                     pytest.param(384, 6, 2, 224, 84, id="vit-small-b84"),
+                                                     pytest.param(128, 2, 2, 224, 84, id="d128-b84"),
                                                      pytest.param(384, 3, 4, 224, 32, id="reference-encoder-b32"),
                                                      pytest.param(768, 12, 2, 64, 3, id="vit-base-width-64px"),
                                                      pytest.param(128, 2, 2, 16, 4, id="n5")])

@@ -124,6 +124,12 @@ SIGNATURES = {
     "vitocm_attention_fwd_lse": (c_int, [c_void_p, c_void_p, c_int64, c_int, c_int, c_void_p, c_int64, c_void_p, c_void_p]),
     "vitocm_attention_bwd": (c_int, [c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p,
                                      c_int64, c_int, c_int, c_void_p]),
+    "vitocm_gemm_dgelu": (c_int, [c_void_p, c_void_p, c_int64, c_void_p, c_int64, c_int, c_int, c_int, c_void_p, c_int64, c_void_p,
+                                  c_int64, c_void_p]),
+    "vitocm_layernorm_bwd": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                     c_int, c_int, c_int, c_void_p, c_void_p]),
+    "vitocm_mim_loss_bwd": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p,
+                                    c_void_p]),
     "vitocm_debug_abw_timeline": (c_int, [c_void_p]),
     "vitocm_launch_count": (c_int64, []),
     "vitocm_profile_enable": (c_int, [c_int]),
