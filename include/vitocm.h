@@ -316,6 +316,15 @@ int vitocm_block_tail(vitocm_engine* e, const void* CTX, int64_t ld_ctx, const v
                       const float* ln2_b, const void* W1, int64_t ldw1, const void* W2, int64_t ldw2, int M, int D, int hidden, const float* bias1,
                       const float* bias2, float* X, const float* next_ln_w, const float* next_ln_b, void* XN, int64_t ld_xn, const void* Wqkv,
                       int64_t ldwqkv, const float* bias_qkv, void* QKV, int64_t ld_qkv, int64_t* stamps, void* stream);
+/* vitocm_block_tail in the form the forward runs after vitocm_finalize_weights: W1 / bias1 are taken to carry norm2's affine
+ * parameters (W1 diag(ln2_w), bias1 + W1 ln2_b; ln2_w / ln2_b are not read) and, when Wqkv is not NULL, Wqkv / bias_qkv the next
+ * norm1's (next_ln_w / next_ln_b are then only tested against NULL).  Without Wqkv, XN = LayerNorm(X; next_ln) keeps its affine
+ * parameters.  Same arguments as vitocm_block_tail. */
+int vitocm_block_tail_folded(vitocm_engine* e, const void* CTX, int64_t ld_ctx, const void* Wp, int64_t ldwp, const float* bias_p,
+                             const float* ln2_w, const float* ln2_b, const void* W1, int64_t ldw1, const void* W2, int64_t ldw2, int M, int D,
+                             int hidden, const float* bias1, const float* bias2, float* X, const float* next_ln_w, const float* next_ln_b,
+                             void* XN, int64_t ld_xn, const void* Wqkv, int64_t ldwqkv, const float* bias_qkv, void* QKV, int64_t ld_qkv,
+                             int64_t* stamps, void* stream);
 /* ctx = MHSA(qkv) for B images of n_tokens tokens: qkv bf16 [B*N][ld] (columns [3][heads][head_dim]), ctx bf16 [B*N][ldo]. */
 int vitocm_attention(vitocm_engine* e, const void* qkv, int64_t ld, int B, int n_tokens, void* ctx, int64_t ldo,
                      void* stream);

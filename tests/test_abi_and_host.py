@@ -25,6 +25,9 @@ def test_library_exports_every_declared_symbol(lib):
     for s in syms:
         assert hasattr(lib, s), f"libvitocm.so does not export {s}"
     assert set(syms) == set(vob._lib.SIGNATURES), "ctypes table and header disagree"
+    # the block tail's two forms (plain affine, folded into the weights) take one argument list
+    assert {"vitocm_block_tail", "vitocm_block_tail_folded"} <= set(syms)
+    assert vob._lib.SIGNATURES["vitocm_block_tail_folded"] == vob._lib.SIGNATURES["vitocm_block_tail"]
     assert lib.vitocm_version() == 100
 
 

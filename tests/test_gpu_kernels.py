@@ -5,6 +5,7 @@ import math
 import pytest
 import torch
 
+import block_half_oracle as BO
 import vitocm_b200 as vob
 from gpu_util import attention, attention_reference, gemm, make_engine, split_bf16
 from vitocm_b200._lib import check, cur_stream, ptr
@@ -273,6 +274,15 @@ def _tail_reference(ctx, Wp, bp, g2, be2, W1, b1, W2, b2, gn, ben, resid, dt, ep
     return x, xn
 
 
+def _tail_oracle_check(precision, ctx, Wp, bp, resid, W1, b1, W2, b2, g2, be2, gn, ben, x, xn=None, Wq=None, bq=None, qkv=None):
+    """every element against the rounding-faithful float64 reference (tests/block_half_oracle.py) of the plain form"""
+    nxt = "qkv" if Wq is not None else ("xn" if xn is not None else None)
+    ops = BO.Operands(precision, ctx, Wp, bp, resid, W1, b1, W2, b2, g2, be2, gn, ben, Wq, bq, 1e-6, nxt=nxt)
+    got = {k: v for k, v in (("x", x), ("xn", xn), ("qkv", qkv)) if v is not None}
+    rep = BO.check_launch(ops, got)
+    assert rep.ok(), str(rep)
+
+
 @pytest.mark.parametrize("M,D,Hd", [(785, 384, 1536), (256, 384, 1536), (130, 128, 512), (1, 128, 128), (5000, 384, 1536), (80000, 384, 1536),
                                     (257, 128, 256), (40000, 128, 384), (60000, 128, 128)])   # odd chunk counts: the epilogue groups swap per item
 @pytest.mark.parametrize("precision", ["bf16", "fp16"])
@@ -314,6 +324,7 @@ def test_block_tail(M, D, Hd, precision, with_next_ln):
         assert (got - ref_xn).abs().max().item() <= tol_n
     else:
         assert torch.isnan(xn.float()).all()
+    _tail_oracle_check(precision, ctx, Wp, bp, resid, W1, b1, W2, b2, g2, be2, gn, ben, x, xn[:, :D] if with_next_ln else None)
 
 
 @pytest.mark.parametrize("M,D,Hd", [(785, 384, 1536), (130, 128, 512), (1, 128, 128), (5000, 384, 1536), (80000, 384, 1536), (257, 128, 256),
@@ -355,6 +366,7 @@ def test_block_tail_with_next_qkv(M, D, Hd, precision):
     # one 16-bit ulp of the output + normalised rows that landed on the neighbouring 16-bit value (each worth |w| 2^-8 / 2^-11)
     assert err <= (6e-3 if precision == "fp16" else 4e-2) * ref_q.abs().max().item(), (err, ref_q.abs().max().item())
     assert (got - ref_q).abs().mean().item() <= (4e-4 if precision == "fp16" else 3e-3) * ref_q.abs().max().item()
+    _tail_oracle_check(precision, ctx, Wp, bp, resid, W1, b1, W2, b2, g2, be2, gn, ben, x, Wq=Wq, bq=bq, qkv=qkv)
 
 
 @pytest.mark.parametrize("precision", ["bf16", "fp16"])
@@ -398,6 +410,7 @@ def test_block_tail_statistics_with_large_means(precision):
     for k in range(5):
         rows = slice(k, M, 5)
         assert (err[rows].max() <= (2e-3 if precision == "fp16" else 1.2e-2) * ref_n[rows].abs().max()).item(), k
+    _tail_oracle_check(precision, ctx, Wp, bp, resid, W1, b1, W2, b2, g2, be2, gn, ben, x, xn[:, :D])
 
 
 def test_block_tail_matches_separate_kernels(engine):

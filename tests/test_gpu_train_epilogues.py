@@ -12,6 +12,7 @@ import pytest
 import torch
 
 import vitocm_b200 as vob
+from block_half_oracle import MANT, gelu64, ulp16
 from gpu_util import gemm, make_engine
 from vitocm_b200._lib import check, cur_stream, ptr
 
@@ -24,8 +25,6 @@ EPS24 = 2.0 ** -24
 GELU_ERR = {"bf16": 2.5e-5, "fp16": 3.0e-6}
 DGELU_ERR = {"bf16": 1.1e-4, "fp16": 1.5e-5}
 DT = {"bf16": torch.bfloat16, "fp16": torch.float16}
-MANT = {"bf16": 7, "fp16": 10}        # stored significand bits
-EMIN = {"bf16": -126, "fp16": -14}    # exponent of the smallest normal value
 PAD = 64
 
 
@@ -48,17 +47,6 @@ def engines():
 def _rand(shape, seed, scale=1.0):
     g = torch.Generator(device="cuda").manual_seed(seed)
     return torch.randn(shape, generator=g, device="cuda") * scale
-
-
-def ulp16(x, prec):
-    """ulp of the 16-bit format at |x| (float64 tensor), subnormal spacing below the smallest normal"""
-    _, ex = torch.frexp(x.abs())
-    e = torch.where(x == 0, EMIN[prec], torch.clamp(ex.to(torch.float64) - 1, min=EMIN[prec]))
-    return torch.pow(2.0, e - MANT[prec])
-
-
-def gelu64(x):
-    return 0.5 * x * (1.0 + torch.special.erf(x / math.sqrt(2.0)))
 
 
 def dgelu64(x):

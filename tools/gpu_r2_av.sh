@@ -3,7 +3,6 @@
 mkdir -p gpurun_out
 L=gpurun_out/r2av.log
 : > $L
-export VITOCM_TAIL_ASSUME_FOLDED=1
 for b in a b; do
   if [ $b = a ]; then export VITOCM_LIB=$PWD/tools/bin/libvitocm_a.so; else unset VITOCM_LIB; fi
   echo "=== build $b" >> $L

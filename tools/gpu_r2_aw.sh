@@ -3,7 +3,6 @@
 mkdir -p gpurun_out
 L=gpurun_out/r2aw.log
 : > $L
-export VITOCM_TAIL_ASSUME_FOLDED=1
 for item in 5 20 35; do
   echo "=== item $item" >> $L
   VITOCM_MLP_TL_ITEM=$item timeout 200 python tools/tail_timeline.py 1225 2 1 >> $L 2>&1

@@ -3,11 +3,9 @@
 mkdir -p gpurun_out
 L=gpurun_out/r2ba.log
 : > $L
-export VITOCM_TAIL_ASSUME_FOLDED=1
 for stg in 0 90000 120000 150000 180000 240000 360000; do
   echo "stagger $stg: $(VITOCM_TAIL_STAGGER=$stg VITOCM_MLP_TL_ITEM=20 timeout 200 python tools/tail_timeline.py 1225 2 1 2>&1 | head -1) | 175 tiles: $(VITOCM_TAIL_STAGGER=$stg VITOCM_MLP_TL_ITEM=4 timeout 200 python tools/tail_timeline.py 175 2 1 2>&1 | head -1 | sed 's/.*: //')" >> $L
 done
-unset VITOCM_TAIL_ASSUME_FOLDED
 for rep in 0 1; do
   for stg in 0 120000 180000; do
     VITOCM_TAIL_STAGGER=$stg timeout 300 python bench.py --no-cpu-baseline --no-extras > gpurun_out/r2ba_bench_${stg}_${rep}.json 2> gpurun_out/r2ba_bench_${stg}_${rep}.err

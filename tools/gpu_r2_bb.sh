@@ -8,5 +8,5 @@ timeout 600 python -m pytest tests/test_gpu_kernels.py tests/test_gpu_fp16.py -m
 for stg in 0 10000 20000 40000 80000 160000 0 40000; do
   echo "attn stagger $stg: $(VITOCM_ATTN_STAGGER=$stg TILES=1225 PRECISION=2 timeout 200 python tools/attn_bench.py 2>&1 | tail -1)" >> $L
 done
-echo "tail auto stagger: $(VITOCM_TAIL_ASSUME_FOLDED=1 VITOCM_MLP_TL_ITEM=20 timeout 200 python tools/tail_timeline.py 1225 2 1 2>&1 | head -1)" >> $L
+echo "tail auto stagger: $(VITOCM_MLP_TL_ITEM=20 timeout 200 python tools/tail_timeline.py 1225 2 1 2>&1 | head -1)" >> $L
 cat $L

@@ -3,7 +3,6 @@
 mkdir -p gpurun_out
 L=gpurun_out/r2be.log
 : > $L
-export VITOCM_TAIL_ASSUME_FOLDED=1
 for stg in auto 0; do
   for item in 10 30; do
     echo "=== stagger $stg item $item" >> $L

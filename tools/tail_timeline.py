@@ -1,4 +1,4 @@
-"""SM-clock timeline of one work item of the block-tail kernel (vitocm_block_tail with stamps; layout: TailArgs::timeline in
+"""SM-clock timeline of one work item of the block-tail kernel in the form the forward runs (vitocm_block_tail_folded with stamps; layout: TailArgs::timeline in
 csrc/block_tail_sm100.cuh) + its launch time.  Usage: python tools/tail_timeline.py [tiles] [precision]"""
 import os
 import sys
@@ -33,7 +33,7 @@ stamps = torch.zeros(64, device="cuda", dtype=torch.int64)
 
 
 def run(st):
-    check(lib.vitocm_block_tail(eng, ptr(ctx), ctx.stride(0), ptr(Wp), Wp.stride(0), ptr(bp), ptr(g2), ptr(be2), ptr(W1), W1.stride(0), ptr(W2),
+    check(lib.vitocm_block_tail_folded(eng, ptr(ctx), ctx.stride(0), ptr(Wp), Wp.stride(0), ptr(bp), ptr(g2), ptr(be2), ptr(W1), W1.stride(0), ptr(W2),
                                 W2.stride(0), M, D, Hd, ptr(b1), ptr(b2), ptr(x), ptr(gn), ptr(ben), ptr(xn), xn.stride(0), wq_p, Wq.stride(0), bq_p, qkv_p, qkv.stride(0), st, cur_stream()))
 
 

@@ -99,6 +99,9 @@ SIGNATURES = {
     "vitocm_block_tail": (c_int, [c_void_p, c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_int64,
                                   c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_int64, c_void_p,
                                   c_void_p, c_int64, c_void_p, c_void_p]),
+    "vitocm_block_tail_folded": (c_int, [c_void_p, c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_int64,
+                                         c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_int64, c_void_p,
+                                         c_void_p, c_int64, c_void_p, c_void_p]),
     "vitocm_attention": (c_int, [c_void_p, c_void_p, c_int64, c_int, c_int, c_void_p, c_int64, c_void_p]),
     "vitocm_attention_timeline": (c_int, [c_void_p, c_void_p, c_int64, c_int, c_int, c_void_p, c_int64, c_void_p, c_void_p]),
     "vitocm_layernorm": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int, c_int, c_int, c_void_p]),

@@ -1790,19 +1790,33 @@ int vitocm_mlp_fused_timeline(vitocm_engine* e, const void* XN, int64_t ld_xn, c
   if (rc == 1) return fail(VITOCM_ERR_INVALID, "fused MLP: no instantiation for D=%d hidden=%d in this engine mode", D, hidden);
   return rc;
 }
-int vitocm_block_tail(vitocm_engine* e, const void* CTX, int64_t ld_ctx, const void* Wp, int64_t ldwp, const float* bias_p, const float* ln2_w,
-                      const float* ln2_b, const void* W1, int64_t ldw1, const void* W2, int64_t ldw2, int M, int D, int hidden, const float* bias1,
-                      const float* bias2, float* X, const float* next_ln_w, const float* next_ln_b, void* XN, int64_t ld_xn, const void* Wqkv,
-                      int64_t ldwqkv, const float* bias_qkv, void* QKV, int64_t ld_qkv, int64_t* stamps, void* stream) {
+static int block_tail_entry(vitocm_engine* e, const void* CTX, int64_t ld_ctx, const void* Wp, int64_t ldwp, const float* bias_p,
+                            const float* ln2_w, const float* ln2_b, const void* W1, int64_t ldw1, const void* W2, int64_t ldw2, int M, int D,
+                            int hidden, const float* bias1, const float* bias2, float* X, const float* next_ln_w, const float* next_ln_b,
+                            void* XN, int64_t ld_xn, const void* Wqkv, int64_t ldwqkv, const float* bias_qkv, void* QKV, int64_t ld_qkv,
+                            int64_t* stamps, void* stream, bool folded) {
   if (e == nullptr) return fail(VITOCM_ERR_INVALID, "null engine");
-  // diagnostics (tools/tail_timeline.py): VITOCM_TAIL_ASSUME_FOLDED=1 runs the kernel as the engine's forward does after
-  // vitocm_finalize_weights -- the caller's W1 / bias1 / Wqkv / bias_qkv are taken to carry the LayerNorm affine parameters already
-  static const bool folded = [] { const char* v = getenv("VITOCM_TAIL_ASSUME_FOLDED"); return v != nullptr && atoi(v) != 0; }();
   const int rc = run_block_tail(e, CTX, ld_ctx, Wp, ldwp, bias_p, ln2_w, ln2_b, W1, ldw1, W2, ldw2, M, D, hidden, bias1, bias2, X, next_ln_w,
                                 next_ln_b, e->cfg.ln_eps, XN, ld_xn, Wqkv, ldwqkv, bias_qkv, QKV, ld_qkv, reinterpret_cast<cudaStream_t>(stream), true,
                                 reinterpret_cast<long long*>(stamps), folded, folded);
   if (rc == 1) return fail(VITOCM_ERR_INVALID, "block tail: no instantiation for D = %d, hidden = %d on this engine (or inconsistent optional arguments)", D, hidden);
   return rc;
+}
+int vitocm_block_tail(vitocm_engine* e, const void* CTX, int64_t ld_ctx, const void* Wp, int64_t ldwp, const float* bias_p, const float* ln2_w,
+                      const float* ln2_b, const void* W1, int64_t ldw1, const void* W2, int64_t ldw2, int M, int D, int hidden, const float* bias1,
+                      const float* bias2, float* X, const float* next_ln_w, const float* next_ln_b, void* XN, int64_t ld_xn, const void* Wqkv,
+                      int64_t ldwqkv, const float* bias_qkv, void* QKV, int64_t ld_qkv, int64_t* stamps, void* stream) {
+  return block_tail_entry(e, CTX, ld_ctx, Wp, ldwp, bias_p, ln2_w, ln2_b, W1, ldw1, W2, ldw2, M, D, hidden, bias1, bias2, X, next_ln_w, next_ln_b,
+                          XN, ld_xn, Wqkv, ldwqkv, bias_qkv, QKV, ld_qkv, stamps, stream, false);
+}
+// the form block_forward runs after vitocm_finalize_weights: W1 / bias1 carry norm2's gamma / beta, Wqkv / bias_qkv the next norm1's
+int vitocm_block_tail_folded(vitocm_engine* e, const void* CTX, int64_t ld_ctx, const void* Wp, int64_t ldwp, const float* bias_p,
+                             const float* ln2_w, const float* ln2_b, const void* W1, int64_t ldw1, const void* W2, int64_t ldw2, int M, int D,
+                             int hidden, const float* bias1, const float* bias2, float* X, const float* next_ln_w, const float* next_ln_b,
+                             void* XN, int64_t ld_xn, const void* Wqkv, int64_t ldwqkv, const float* bias_qkv, void* QKV, int64_t ld_qkv,
+                             int64_t* stamps, void* stream) {
+  return block_tail_entry(e, CTX, ld_ctx, Wp, ldwp, bias_p, ln2_w, ln2_b, W1, ldw1, W2, ldw2, M, D, hidden, bias1, bias2, X, next_ln_w, next_ln_b,
+                          XN, ld_xn, Wqkv, ldwqkv, bias_qkv, QKV, ld_qkv, stamps, stream, true);
 }
 int vitocm_attention(vitocm_engine* e, const void* qkv, int64_t ld, int B, int n_tokens, void* ctx, int64_t ldo, void* stream) {
   if (e == nullptr) return fail(VITOCM_ERR_INVALID, "null engine");
