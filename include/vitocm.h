@@ -347,12 +347,19 @@ int vitocm_refresh_weights(vitocm_engine* e, void* stream);
  * optimizer.zero_grad(), mim.py:173).  NULL unbinds. */
 int vitocm_bind_grad(vitocm_engine* e, const char* name, float* dev_grad);
 
+/* Includes a slab of 8 depth B bytes (plus alignment) for the stochastic-depth scales of the _dp forwards. */
 size_t vitocm_mim_train_workspace_bytes(const vitocm_engine* e, int B, int n_tokens);
 /* MIM.forward (model.py:71-77) for one batch, keeping the activations the backward needs in ws (same arguments as
- * vitocm_mim_forward; the whole batch is one chunk). */
+ * vitocm_mim_forward; the whole batch is one chunk).  = vitocm_mim_train_forward_dp with branch_scale NULL. */
 int vitocm_mim_train_forward(vitocm_engine* e, const float* x, int B, int H, int W, const float* pos, const float* mask,
                              float* x_rec, double* loss_sums, void* ws, size_t ws_bytes, void* stream);
-/* loss.backward() (mim.py:174) for the batch vitocm_mim_train_forward just ran on the same ws: gradients of
+/* The same with stochastic depth (DINO's DropPath, vit.py:101,110-111): branch_scale = DEVICE fp32 [depth][2][B], [l][0][b] the
+ * scale of block l's attention branch for image b and [l][1][b] that of its MLP branch (0 or 1 / keep in training; any value is
+ * applied): x += s (proj(...) + bias) and x += s (fc2(...) + bias).  The scales are copied into ws on the stream, and the backward on
+ * this ws uses that copy: the gradient entering a branch is s dX, the residual path carries dX unscaled.  NULL = no drop path. */
+int vitocm_mim_train_forward_dp(vitocm_engine* e, const float* x, int B, int H, int W, const float* pos, const float* mask,
+                                float* x_rec, double* loss_sums, const float* branch_scale, void* ws, size_t ws_bytes, void* stream);
+/* loss.backward() (mim.py:174) for the batch vitocm_mim_train_forward(_dp) just ran on the same ws (with its branch scales): gradients of
  * (*grad_scale) * loss (grad_scale = DEVICE pointer to the upstream gradient of the scalar loss, NULL = 1) are accumulated into the buffers bound with vitocm_bind_grad (all parameters except pos_embed);
  * dpos [N][D] fp32 is WRITTEN with the gradient of the (interpolated) position table passed to the forward.
  * Loss scale (fp16 engines): fp16's range would flush the loss gradient (~4e-7 at batch 32, 224^2) towards zero, so the backward
@@ -379,7 +386,10 @@ int vitocm_stream_wait_event(void* stream, void* event);
  * included.  pos [N][D] fp32: the (interpolated) position table, as in vitocm_prepare_tokens. */
 int vitocm_encoder_train_forward(vitocm_engine* e, const float* x, int B, int H, int W, const float* pos, int n_out, float* feats,
                                  void* ws, size_t ws_bytes, void* stream);
-/* Backward of the vitocm_encoder_train_forward that last ran on the same ws, for the upstream gradient dfeats [n_out][B][N][D]
+/* vitocm_encoder_train_forward with stochastic depth: branch_scale as in vitocm_mim_train_forward_dp (NULL = none). */
+int vitocm_encoder_train_forward_dp(vitocm_engine* e, const float* x, int B, int H, int W, const float* pos, int n_out, float* feats,
+                                    const float* branch_scale, void* ws, size_t ws_bytes, void* stream);
+/* Backward of the vitocm_encoder_train_forward(_dp) that last ran on the same ws (with its branch scales), for the upstream gradient dfeats [n_out][B][N][D]
  * fp32 (DEVICE): parameter gradients are ACCUMULATED into the buffers bound with vitocm_bind_grad (every encoder parameter except
  * pos_embed; mask_token and the decoder are not touched), dpos [N][D] is WRITTEN, and so is dx [B][C][H][W] fp32 unless dx is NULL.
  * fp16 engines: S = 2^e is picked on the device from max |dfeats| so that max |dfeats| S lies in [1, 2) (S = 1 for an all-zero
@@ -428,6 +438,16 @@ int vitocm_gemm_dgelu(vitocm_engine* e, const void* dY, int64_t ldy, const void*
  * column sums are multiplied by 1 / S (NULL: 1); bf16 engines ignore it.  D % 4 == 0, D <= 1024. */
 int vitocm_layernorm_bwd(vitocm_engine* e, const float* X, const void* dy, int64_t ld_dy, const float* gamma, float* dX, void* dXb,
                          float* dgamma, float* dbeta, float* dbias_out, int accumulate, int M, int D, const float* lscale, void* stream);
+/* kernel-level: vitocm_layernorm_bwd where dXb and the dbias_out column sums use s dX with s = row_scale[row / rows_per_scale] (DEVICE
+ * fp32; the stochastic-depth scale of the branch this gradient enters); dX, dgamma and dbeta are those of vitocm_layernorm_bwd.
+ * row_scale NULL = vitocm_layernorm_bwd. */
+int vitocm_layernorm_bwd_scaled(vitocm_engine* e, const float* X, const void* dy, int64_t ld_dy, const float* gamma, float* dX, void* dXb,
+                                float* dgamma, float* dbeta, float* dbias_out, int accumulate, int M, int D, const float* lscale,
+                                const float* row_scale, int rows_per_scale, void* stream);
+/* kernel-level: vitocm_gemm with epilogue 2, X[M][ldx] (fp32, in place) += (A . B^T + bias) * row_scale[row / rows_per_scale]
+ * (DEVICE fp32; the proj / fc2 residual add under stochastic depth).  row_scale NULL = vitocm_gemm with epilogue 2. */
+int vitocm_gemm_resid_scaled(vitocm_engine* e, const void* A, int64_t lda, const void* B, int64_t ldb, int M, int N, int K, const float* bias,
+                             float* X, int64_t ldx, const float* row_scale, int rows_per_scale, void* stream);
 /* kernel-level: the loss gradient of vitocm_mim_backward, dY [B (n + 1)][C p^2] (16-bit, the engine's format; C and p from the engine,
  * n = (H / p) (W / p)) = *grad_scale * mask * sign(x_rec - x) / ((loss_sums[1] + 1e-5) C) through PixelShuffle, 0 at ties and in CLS
  * rows.  fp16 engines multiply it by the loss scale S described at vitocm_mim_backward and write [S, 1 / S] to lscale (DEVICE, or

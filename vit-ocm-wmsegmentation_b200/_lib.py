@@ -111,11 +111,15 @@ SIGNATURES = {
     "vitocm_mim_train_workspace_bytes": (c_size_t, [c_void_p, c_int, c_int]),
     "vitocm_mim_train_forward": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
                                          c_size_t, c_void_p]),
+    "vitocm_mim_train_forward_dp": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                            c_void_p, c_size_t, c_void_p]),
     "vitocm_mim_backward": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
                                     c_size_t, c_void_p]),
     "vitocm_mim_backward_events": (c_int, [c_void_p, c_void_p, c_int]),
     "vitocm_encoder_train_forward": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_int, c_void_p, c_void_p, c_size_t,
                                              c_void_p]),
+    "vitocm_encoder_train_forward_dp": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_int, c_void_p, c_void_p, c_void_p,
+                                                c_size_t, c_void_p]),
     "vitocm_encoder_backward": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p,
                                         c_size_t, c_void_p]),
     "vitocm_stream_wait_event": (c_int, [c_void_p, c_void_p]),
@@ -131,6 +135,10 @@ SIGNATURES = {
                                   c_int64, c_void_p]),
     "vitocm_layernorm_bwd": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
                                      c_int, c_int, c_int, c_void_p, c_void_p]),
+    "vitocm_layernorm_bwd_scaled": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                            c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_int, c_void_p]),
+    "vitocm_gemm_resid_scaled": (c_int, [c_void_p, c_void_p, c_int64, c_void_p, c_int64, c_int, c_int, c_int, c_void_p, c_void_p, c_int64,
+                                         c_void_p, c_int, c_void_p]),
     "vitocm_mim_loss_bwd": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p,
                                     c_void_p]),
     "vitocm_debug_abw_timeline": (c_int, [c_void_p]),

@@ -34,6 +34,8 @@ enum GemmEpilogue : int {
   EPI_PATCH_F32 = 4,       // X[b, 1+i, :] = mix(acc + bias, mask_token) + pos[1+i]   (patch embedding)
   EPI_RESID_LN = 5,        // resid_f32 += acc + bias;  xn_bf16 = LayerNorm(resid_f32) * gamma + beta   (proj / fc2 + next LN)
   EPI_DGELU_BF16 = 6,      // out_bf16 = acc * gelu'(pre)          (training: input gradient of fc2 through the GELU, vit.py:59)
+  EPI_RESID_SCALED_F32 = 7,  // resid_f32 += (acc + bias) * row_scale[row / rows_per_scale]   (proj, fc2 under stochastic depth;
+                             // callers ask for it as EPI_BIAS_RESID_F32 with a row_scale, run_gemm picks this instantiation)
 };
 
 struct GemmArgs {
@@ -78,6 +80,9 @@ struct GemmArgs {
   // EPI_DGELU_BF16 only: the GELU's input saved by the forward fc1 epilogue, bf16 [M][ld_pre]
   const __nv_bfloat16* pre;
   long long ld_pre;
+  // EPI_RESID_SCALED_F32 only: per-sample residual-branch scale (stochastic depth, vit.py:110-111), [M / rows_per_scale]
+  const float* row_scale;
+  int rows_per_scale;
 };
 
 constexpr int GEMM_BM = 128;
@@ -915,6 +920,12 @@ gemm_bf16_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __gri
           };
           if (args.f16) put_rows(std::true_type{}); else put_rows(std::false_type{});
         } else {
+          if (EPI == EPI_RESID_SCALED_F32) {   // one load per row; rows past M are clipped by the TMA
+            const int m = row_base + lane;
+            const float s = m < args.M ? __ldg(args.row_scale + m / args.rows_per_scale) : 0.f;
+#pragma unroll
+            for (int j = 0; j < 32; ++j) v[j] *= s;
+          }
           // 32 rows x 128 B, SWIZZLE_128B: chunk j of row r sits at r*128 + ((j ^ (r & 7)) << 4)
           const uint32_t rowaddr = stg + lane * 128;
           const int sw = lane & 7;
@@ -926,7 +937,7 @@ gemm_bf16_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __gri
         ptx::fence_proxy_async_smem();
         __syncwarp();
         if (lane == 0) {
-          if (EPI == EPI_BIAS_RESID_F32) {
+          if (EPI == EPI_BIAS_RESID_F32 || EPI == EPI_RESID_SCALED_F32) {
             ptx::tma_reduce_add_2d(&tmap_c, stg, col, row_base);
           } else {
             ptx::tma_store_2d(&tmap_c, stg, col, row_base);

@@ -58,11 +58,14 @@ __device__ __forceinline__ int loss_scale_exp(float a) {
 //   dbias_out += column sums of the new dX      (= the bias gradient of the Linear whose output was added into this
 //                                                residual stream: proj of this block / fc2 of the previous one)
 // F16: dy / dXb are fp16 and carry the loss scale; dgamma, dbeta and dbias_out are multiplied by lscale[1] = 1 / S.
-template <int NV, bool F16 = false>
+// SCALED (stochastic depth): dXb and the dbias_out sums use row_scale[row / rows_per_scale] * dX, the gradient that enters the residual
+// branch whose output was added into this stream; dX itself (the identity path), dgamma and dbeta are unscaled.
+template <int NV, bool F16 = false, bool SCALED = false>
 __global__ void __launch_bounds__(256)
 ln_bwd_kernel(const float* __restrict__ x, const __nv_bfloat16* __restrict__ dy, long long ld_dy, const float* __restrict__ gamma,
               float* __restrict__ dX, __nv_bfloat16* __restrict__ dXb, float* __restrict__ dgamma, float* __restrict__ dbeta,
-              float* __restrict__ dbias_out, int accumulate, int M, int D, float eps, const float* __restrict__ lscale = nullptr) {
+              float* __restrict__ dbias_out, int accumulate, int M, int D, float eps, const float* __restrict__ lscale = nullptr,
+              const float* __restrict__ row_scale = nullptr, int rows_per_scale = 1) {
   constexpr int CNT = NV > 0 ? NV : LN_MAX_VEC;
   extern __shared__ float ln_red[];   // [3][D]
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarps = blockDim.x >> 5;
@@ -84,6 +87,7 @@ ln_bwd_kernel(const float* __restrict__ x, const __nv_bfloat16* __restrict__ dy,
     const uint2* dr = reinterpret_cast<const uint2*>(dy + static_cast<long long>(row) * ld_dy);
     float4 v[CNT], g[CNT], acc_in[CNT];
     float4* dxr = reinterpret_cast<float4*>(dX + static_cast<long long>(row) * D);
+    const float rs = SCALED ? __ldg(row_scale + row / rows_per_scale) : 1.f;
     float s = 0.f;
 #pragma unroll
     for (int i = 0; i < CNT; ++i) {
@@ -134,6 +138,7 @@ ln_bwd_kernel(const float* __restrict__ x, const __nv_bfloat16* __restrict__ dy,
         o.z += rstd * (g[i].z - c1 - v[i].z * c2);
         o.w += rstd * (g[i].w - c1 - v[i].w * c2);
         dxr[idx] = o;
+        if (SCALED) { o.x *= rs; o.y *= rs; o.z *= rs; o.w *= rs; }
         dbr[idx] = make_uint2(ptx::pack_h2<F16>(o.x, o.y), ptx::pack_h2<F16>(o.z, o.w));
         acco[i].x += o.x; acco[i].y += o.y; acco[i].z += o.z; acco[i].w += o.w;
       }

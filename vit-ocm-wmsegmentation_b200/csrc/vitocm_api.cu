@@ -12,6 +12,7 @@
 #include <cstdlib>
 #include <cstring>
 #include <map>
+#include <set>
 #include <string>
 #include <vector>
 
@@ -188,6 +189,9 @@ struct vitocm_engine {
   cudaStream_t aux[MAX_LANES - 1] = {nullptr, nullptr, nullptr};
   cudaEvent_t ev_fork = nullptr, ev_join[MAX_LANES - 1] = {nullptr, nullptr, nullptr};
   std::vector<cudaEvent_t> bwd_events;   // vitocm_mim_backward_events: [depth] blocks + [1] head, recorded as the gradient buckets complete
+  // training workspaces (by the address of their branch-scale slab) whose last forward ran with stochastic-depth scales: the
+  // backward on the same workspace scales its residual branches with that forward's copy (TrainWs::bscale)
+  std::set<const void*> dp_ws;
   ~vitocm_engine() {
     for (cudaEvent_t ev : bwd_events) if (ev) cudaEventDestroy(ev);
     for (auto& kv : master) delete kv.second;
@@ -314,6 +318,7 @@ int launch_gemm_pair_bn(int epi, const CUtensorMap& ta, const CUtensorMap& tb, c
     case EPI_BIAS_BF16: return launch_gemm_pair<BN, EPI_BIAS_BF16>(ta, tb, tc, a, num_sms, st);
     case EPI_BIAS_GELU_BF16: return launch_gemm_pair<BN, EPI_BIAS_GELU_BF16>(ta, tb, tc, a, num_sms, st);
     case EPI_BIAS_RESID_F32: return launch_gemm_pair<BN, EPI_BIAS_RESID_F32>(ta, tb, tc, a, num_sms, st);
+    case EPI_RESID_SCALED_F32: return launch_gemm_pair<BN, EPI_RESID_SCALED_F32>(ta, tb, tc, a, num_sms, st);
     case EPI_BIAS_F32: return launch_gemm_pair<BN, EPI_BIAS_F32>(ta, tb, tc, a, num_sms, st);
     case EPI_DGELU_BF16: return launch_gemm_pair<BN, EPI_DGELU_BF16>(ta, tb, tc, a, num_sms, st, td);
   }
@@ -329,6 +334,7 @@ int launch_gemm_bn(int epi, bool res, const CUtensorMap& ta, const CUtensorMap& 
         case EPI_BIAS_BF16: return launch_gemm_res<BN, EPI_BIAS_BF16>(ta, tb, tc, a, num_sms, st);
         case EPI_BIAS_GELU_BF16: return launch_gemm_res<BN, EPI_BIAS_GELU_BF16>(ta, tb, tc, a, num_sms, st);
         case EPI_BIAS_RESID_F32: return launch_gemm_res<BN, EPI_BIAS_RESID_F32>(ta, tb, tc, a, num_sms, st);
+        case EPI_RESID_SCALED_F32: return launch_gemm_res<BN, EPI_RESID_SCALED_F32>(ta, tb, tc, a, num_sms, st);
         case EPI_BIAS_F32: return launch_gemm_res<BN, EPI_BIAS_F32>(ta, tb, tc, a, num_sms, st);
       }
     }
@@ -337,6 +343,7 @@ int launch_gemm_bn(int epi, bool res, const CUtensorMap& ta, const CUtensorMap& 
     case EPI_BIAS_BF16: return launch_gemm_inst<BN, EPI_BIAS_BF16, false>(ta, tb, tc, a, num_sms, st);
     case EPI_BIAS_GELU_BF16: return launch_gemm_inst<BN, EPI_BIAS_GELU_BF16, false>(ta, tb, tc, a, num_sms, st);
     case EPI_BIAS_RESID_F32: return launch_gemm_inst<BN, EPI_BIAS_RESID_F32, false>(ta, tb, tc, a, num_sms, st);
+    case EPI_RESID_SCALED_F32: return launch_gemm_inst<BN, EPI_RESID_SCALED_F32, false>(ta, tb, tc, a, num_sms, st);
     case EPI_BIAS_F32: return launch_gemm_inst<BN, EPI_BIAS_F32, false>(ta, tb, tc, a, num_sms, st);
     case EPI_DGELU_BF16: return launch_gemm_inst<BN, EPI_DGELU_BF16, false>(ta, tb, tc, a, num_sms, st, td);
   }
@@ -364,9 +371,13 @@ int pick_bn(int M, int N, int num_sms, int max_bn) {
 // A [M][lda] (split: hi at col 0, lo at col K), B [N][ldb] likewise.
 int run_gemm(const vitocm_engine* e, const void* A, long long lda, const void* B, long long ldb, int M, int N, int K,
              int split_in, int epi, const float* bias, void* out, long long ldo, int split_out, int lo_off, cudaStream_t st,
-             int pcls = PC_OTHER, const void* pre = nullptr, long long ld_pre = 0) {
+             int pcls = PC_OTHER, const void* pre = nullptr, long long ld_pre = 0, const float* row_scale = nullptr, int rows_per_scale = 1) {
   if (epi == EPI_DGELU_BF16 && (pre == nullptr || split_in || ld_pre % 8 != 0 || (reinterpret_cast<uintptr_t>(pre) & 15) != 0))
     return fail(VITOCM_ERR_INVALID, "GEMM dGELU epilogue needs a 16-byte aligned bf16 pre-activation and single-bf16 operands");
+  if (row_scale != nullptr && (epi != EPI_BIAS_RESID_F32 || rows_per_scale < 1))
+    return fail(VITOCM_ERR_INVALID, "GEMM row scale needs the residual epilogue (2) and rows_per_scale >= 1");
+  if (epi == EPI_RESID_SCALED_F32) return fail(VITOCM_ERR_INVALID, "unknown GEMM epilogue %d", epi);
+  if (row_scale != nullptr) epi = EPI_RESID_SCALED_F32;   // its own instantiation: the unscaled kernels stay as they are
   if (M <= 0) return 0;
   ProfScope prof(pcls, st);
   if (K % GEMM_BK != 0) return fail(VITOCM_ERR_INVALID, "GEMM K=%d must be a multiple of %d", K, GEMM_BK);
@@ -381,7 +392,7 @@ int run_gemm(const vitocm_engine* e, const void* A, long long lda, const void* B
     static const int gelu_bn = [] { const char* v = getenv("VITOCM_GELU_BN"); return v ? atoi(v) : 192; }();   // measured: 835 vs 794 TFLOP/s
     int pbn = N % 256 == 0 ? 256 : (N % 192 == 0 ? 192 : 128);
     if ((epi == EPI_BIAS_GELU_BF16 || epi == EPI_DGELU_BF16) && gelu_bn == 192 && N % 192 == 0) pbn = 192;   // 12 epilogue warps instead of 8
-    const bool of32 = (epi == EPI_BIAS_RESID_F32 || epi == EPI_BIAS_F32);
+    const bool of32 = (epi == EPI_BIAS_RESID_F32 || epi == EPI_RESID_SCALED_F32 || epi == EPI_BIAS_F32);
     CUtensorMap pa, pb, pc;
     TRY(make_tmap_bf16(&pa, A, M, split_in == 2 ? 2LL * K : K, lda, GEMM_BM));
     TRY(make_tmap_bf16(&pb, B, N, K, ldb, pbn / 2));
@@ -392,6 +403,7 @@ int run_gemm(const vitocm_engine* e, const void* A, long long lda, const void* B
     pg.bias = bias; pg.out_f32 = reinterpret_cast<float*>(out);
     pg.split_out = split_out; pg.lo_off = lo_off;
     pg.pre = reinterpret_cast<const __nv_bfloat16*>(pre); pg.ld_pre = ld_pre;
+    pg.row_scale = row_scale; pg.rows_per_scale = rows_per_scale;
     CUtensorMap pd;
     const CUtensorMap* ppd = nullptr;
     if (epi == EPI_DGELU_BF16) {   // the saved pre-activation, read by the epilogue as 32 x 32 bf16 boxes
@@ -409,7 +421,7 @@ int run_gemm(const vitocm_engine* e, const void* A, long long lda, const void* B
   const int bn = pick_bn(M, N, e->num_sms, res ? 192 : 256);
   if (res && bn < 128) res = false;
   const long long kext = static_cast<long long>(K) * (split_in ? 2 : 1);
-  const bool out_f32 = (epi == EPI_BIAS_RESID_F32 || epi == EPI_BIAS_F32);
+  const bool out_f32 = (epi == EPI_BIAS_RESID_F32 || epi == EPI_RESID_SCALED_F32 || epi == EPI_BIAS_F32);
   CUtensorMap ta, tb, tc;
   TRY(make_tmap_bf16(&ta, A, M, kext, lda, GEMM_BM));
   TRY(make_tmap_bf16(&tb, B, N, split_in == 2 ? K : kext, ldb, bn));
@@ -424,6 +436,7 @@ int run_gemm(const vitocm_engine* e, const void* A, long long lda, const void* B
   static const int dbg = [] { const char* v = getenv("VITOCM_GEMM_DEBUG"); return v ? atoi(v) : 0; }();
   a.debug = dbg; a.out_f32 = reinterpret_cast<float*>(out);
   a.pre = reinterpret_cast<const __nv_bfloat16*>(pre); a.ld_pre = ld_pre;
+  a.row_scale = row_scale; a.rows_per_scale = rows_per_scale;
   CUtensorMap td;
   const CUtensorMap* ptd = nullptr;
   if (epi == EPI_DGELU_BF16) {

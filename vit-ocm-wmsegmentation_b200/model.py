@@ -78,6 +78,7 @@ class VisionTransformerForSimMIM(VisionTransformer):
     @torch.no_grad()
     def forward(self, x, mask):
         """-> [B, D, H/p, W/p] (model.py:25-53)."""
+        self._refuse_drop_path("VisionTransformerForSimMIM.forward")
         assert mask is not None
         xx = self._check_input(x)
         eng = self._ensure_engine()
@@ -100,10 +101,11 @@ class VisionTransformerForSimMIM(VisionTransformer):
 class _MIMStep(torch.autograd.Function):
     """loss = MIM(x, mask) with the backward of SSS/mim.py:174 in libvitocm.  Parameter gradients do not travel through
     autograd: vitocm_mim_backward accumulates them straight into the flat ``.grad`` buffer of ``MIM`` (the parameters are
-    passed as inputs only so that autograd schedules this node); the position table's gradient is returned."""
+    passed as inputs only so that autograd schedules this node); the position table's gradient is returned.  ``scales``: the
+    stochastic-depth scales [depth, 2, B] of this forward, or None; the backward reads the workspace's copy."""
 
     @staticmethod
-    def forward(ctx, mim, xx, maskf, pos, *params):
+    def forward(ctx, mim, xx, maskf, pos, scales, *params):
         enc = mim.encoder
         eng = enc._ensure_engine()
         lib = _lib.load_library()
@@ -116,8 +118,8 @@ class _MIMStep(torch.autograd.Function):
             mim._train_ws = None
             mim._train_ws = torch.empty(need, dtype=torch.uint8, device=xx.device)
         posc = pos.detach().to(torch.float32).contiguous()
-        check(lib.vitocm_mim_train_forward(eng, ptr(xx), B, H, W, ptr(posc), ptr(maskf), ptr(x_rec), ptr(sums), ptr(mim._train_ws),
-                                           mim._train_ws.numel(), cur_stream()))
+        check(lib.vitocm_mim_train_forward_dp(eng, ptr(xx), B, H, W, ptr(posc), ptr(maskf), ptr(x_rec), ptr(sums), ptr(scales),
+                                              ptr(mim._train_ws), mim._train_ws.numel(), cur_stream()))
         ctx.mim = mim
         # the saved activations live in the ONE shared workspace: stamp it, so that a backward whose forward has since been
         # overwritten by another training-mode forward fails loudly instead of producing wrong gradients
@@ -143,7 +145,7 @@ class _MIMStep(torch.autograd.Function):
         check(_lib.load_library().vitocm_mim_backward(mim.encoder._engine, ptr(xx), B, H, W, ptr(maskf), ptr(x_rec), ptr(sums), ptr(gs),
                                                       ptr(dpos), ptr(mim._train_ws), mim._train_ws.numel(), cur_stream()))
         mim._launch_bucket_allreduce()
-        return (None, None, None, dpos) + (None,) * len(mim._param_list)
+        return (None, None, None, dpos, None) + (None,) * len(mim._param_list)
 
 
 class MIM(nn.Module):
@@ -323,24 +325,33 @@ class MIM(nn.Module):
             dist.all_reduce(self._gflat, op=dist.ReduceOp.SUM, group=group)
 
     def _forward_train(self, x, mask):
+        """The training forward; with gradients enabled it keeps the backward.  Under no_grad (training mode with drop path) it
+        only runs the forward, on the engine's own weight copies."""
         enc = self.encoder
-        self.flatten_parameters()
+        grad = torch.is_grad_enabled()
+        if grad:
+            self.flatten_parameters()
         xx = enc._check_input(x)
         B = xx.shape[0]
         N = enc._tokens(xx)
         pos = enc._pos_graph(*enc._mim_pos_args(xx))
         assert pos.shape[0] == N, "position table does not match the token count (img_size vs input size)"
         m = mask.detach().reshape(B, -1).to(device=xx.device, dtype=torch.float32).contiguous()
-        loss, x_rec = _MIMStep.apply(self, xx, m, pos, *[p for _, p in self._param_list])
+        scales = enc._branch_scales(B, xx.device)
+        loss, x_rec = _MIMStep.apply(self, xx, m, pos, scales, *([p for _, p in self._param_list] if grad else []))
         mask_up = mask.repeat_interleave(self.patch_size, 1).repeat_interleave(self.patch_size, 2).unsqueeze(1).contiguous()
         return loss, x_rec, mask_up
 
     def forward(self, x, mask):
         """-> (loss, x_rec, mask upsampled to pixels) (model.py:71-77).  With gradients enabled the loss carries the
         backward of the training step (``model.train()``, as SSS/mim.py:154 sets it); in ``eval()`` mode or under
-        ``torch.no_grad()`` this is a plain evaluation."""
+        ``torch.no_grad()`` this is a plain evaluation -- except that in training mode an encoder with drop_path_rate > 0 drops
+        paths under no_grad too, as the reference does."""
         if self.training and torch.is_grad_enabled() and any(p.requires_grad for p in self.parameters()):
             return self._forward_train(x, mask)
+        if self.training and self.encoder._drop_path_active():
+            with torch.no_grad():
+                return self._forward_train(x, mask)
         return self._forward_eval(x, mask)
 
     @torch.no_grad()
@@ -376,11 +387,12 @@ class MIM(nn.Module):
         return {}
 
 
-def build_model(args, depth=12, num_heads=6, precision="bf16"):
+def build_model(args, depth=12, num_heads=6, precision="bf16", drop_path_rate=0.):
     """SSS/model.py:91-108.  The reference's build_model hard-codes depth=4 / num_heads=3 at embed_dim 384 (head_dim 128):
     ``build_model(args, depth=4, num_heads=3)`` builds exactly that encoder.  The defaults (12 blocks, 6 heads, head_dim 64)
-    are the ViT-S/8 of the shipped training log (SSS/output/log_rank0.txt)."""
+    are the ViT-S/8 of the shipped training log (SSS/output/log_rank0.txt).  ``drop_path_rate``: stochastic depth of the encoder
+    (VisionTransformer); 0 as in the reference's call."""
     return VisionTransformerForSimMIM(patch_size=args.MODEL.PATCH_SIZE, embed_dim=384, depth=depth, num_heads=num_heads,
                                       mlp_ratio=4, img_size=[args.DATA.IMG_SIZE], qkv_bias=True,
                                       norm_layer=partial(nn.LayerNorm, eps=1e-6), interpolate_encoding=True,
-                                      precision=precision)
+                                      precision=precision, drop_path_rate=drop_path_rate)

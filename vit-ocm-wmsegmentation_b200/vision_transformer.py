@@ -75,13 +75,39 @@ class _Attention(nn.Module):
         self.proj = nn.Linear(dim, dim)
 
 
+class _DropPath(nn.Module):
+    """Stochastic depth of one block (vit.py:101): parameter-free; the training kernels apply it (draw_branch_scales)."""
+    def __init__(self, drop_prob=0.):
+        super().__init__()
+        self.drop_prob = float(drop_prob)
+
+    def extra_repr(self):
+        return f"drop_prob={self.drop_prob}"
+
+
 class _Block(nn.Module):
-    def __init__(self, dim, num_heads, mlp_ratio, qkv_bias, norm_layer):
+    def __init__(self, dim, num_heads, mlp_ratio, qkv_bias, norm_layer, drop_path=0.):
         super().__init__()
         self.norm1 = norm_layer(dim)
         self.attn = _Attention(dim, num_heads, qkv_bias)
+        self.drop_path = _DropPath(drop_path)
         self.norm2 = norm_layer(dim)
         self.mlp = _Mlp(dim, int(dim * mlp_ratio))
+
+
+def draw_branch_scales(drop_probs, B: int, device) -> torch.Tensor:
+    """Stochastic-depth scales [depth, 2, B] fp32 on ``device`` for one training forward: [l, 0] scales block l's attention
+    branch, [l, 1] its MLP branch.  The draws are the reference's drop_path calls (vit.py:26-34) in its order -- block by block,
+    attention before MLP, none for a block whose rate is 0 -- each ``floor(keep + torch.rand((B, 1, 1)))`` on ``device``, so one
+    seed gives the reference module's masks.  A scale is r / keep: 0 for a dropped sample, 1 / keep for a kept one."""
+    s = torch.ones(len(drop_probs), 2, B, dtype=torch.float32, device=device)
+    for l, p in enumerate(drop_probs):
+        if p > 0:
+            keep = 1 - p
+            for k in range(2):
+                r = torch.floor(keep + torch.rand((B, 1, 1), dtype=torch.float32, device=device))
+                s[l, k] = r.reshape(B) / keep
+    return s
 
 
 class _PatchEmbed(nn.Module):
@@ -163,15 +189,19 @@ class VisionTransformer(nn.Module):
     """Vision Transformer whose forward passes run in libvitocm (B200 / sm_100a).
 
     Constructor signature follows the reference (vit.py:137-139); ``precision`` ("bf16" |
-    "fp16" | "fp32", see parse_precision), ``chunk_tiles`` (tiles per kernel launch) and ``lanes`` (chunks in flight on concurrent streams) are additions.  Dropout / stochastic depth must be 0 (the
-    reference's inference and MIM configurations all use 0)."""
+    "fp16" | "fp32", see parse_precision), ``chunk_tiles`` (tiles per kernel launch) and ``lanes`` (chunks in flight on concurrent streams) are additions.  Dropout rates must be 0
+    (the reference's configurations all use 0).  ``drop_path_rate`` in [0, 1) is stochastic depth with DINO's linear schedule over the
+    blocks; it acts in training mode only (the training kernels scale each sample's residual branches), and in training mode the
+    attention-map entry points refuse to run."""
 
     def __init__(self, img_size=[224], patch_size=16, in_chans=3, num_classes=0, embed_dim=768, depth=12,
                  num_heads=12, mlp_ratio=4., qkv_bias=False, qk_scale=None, drop_rate=0., attn_drop_rate=0.,
                  drop_path_rate=0., norm_layer=nn.LayerNorm, precision="bf16", chunk_tiles=512, lanes=1, **kwargs):
         super().__init__()
-        if drop_rate or attn_drop_rate or drop_path_rate:
-            raise NotImplementedError("vitocm: dropout / drop-path rates must be 0 on this path")
+        if drop_rate or attn_drop_rate:
+            raise NotImplementedError("vitocm: dropout / attention-dropout rates must be 0 on this path")
+        if not 0 <= drop_path_rate < 1:
+            raise ValueError(f"drop_path_rate must lie in [0, 1) (got {drop_path_rate})")
         if embed_dim % num_heads or embed_dim // num_heads not in (64, 128):
             raise NotImplementedError("vitocm kernels support head_dim 64 and 128 (embed_dim %d / num_heads %d)"
                                       % (embed_dim, num_heads))
@@ -190,7 +220,8 @@ class VisionTransformer(nn.Module):
         n = self.patch_embed.num_patches
         self.cls_token = nn.Parameter(torch.zeros(1, 1, embed_dim))
         self.pos_embed = nn.Parameter(torch.zeros(1, n + 1, embed_dim))
-        self.blocks = nn.ModuleList([_Block(embed_dim, num_heads, mlp_ratio, qkv_bias, norm_layer) for _ in range(depth)])
+        dpr = [v.item() for v in torch.linspace(0, drop_path_rate, depth)]   # stochastic depth decay rule (vit.py:155)
+        self.blocks = nn.ModuleList([_Block(embed_dim, num_heads, mlp_ratio, qkv_bias, norm_layer, dpr[i]) for i in range(depth)])
         self.norm = norm_layer(embed_dim)
         self.head = nn.Linear(embed_dim, num_classes) if num_classes > 0 else nn.Identity()
         self.ln_eps = float(self.norm.eps)
@@ -370,6 +401,7 @@ class VisionTransformer(nn.Module):
 
         A single-channel ``x`` [B, 1, H, W] on a multi-channel model is the gray fast path: it stands for the image with all
         channels equal (what the reference feeds for every OCM tile) and runs the channel-folded patch filter."""
+        self._refuse_drop_path("cls_attention_rows")
         x = self._check_input(x, allow_gray=True)
         eng = self._ensure_engine()
         B, Cx, H, W = x.shape
@@ -388,6 +420,7 @@ class VisionTransformer(nn.Module):
         of a gray uint8 CUDA mosaic, cut out by the patch-embedding producer itself: no crop is ever materialised.  grid: n for an
         n x n grid, or (ny, nx) for a rectangular one (ny rows of windows over the height, nx columns over the width; window t
         has origin ((t // nx) * stride, (t % nx) * stride)).  -> [count, heads, N] fp32."""
+        self._refuse_drop_path("cls_attention_rows_mosaic")
         ny, nx = (grid, grid) if isinstance(grid, int) else (int(grid[0]), int(grid[1]))
         if isinstance(mosaic, tuple):      # (device address of row 0, height, width, pitch, device): a band buffer addressed by absolute rows
             mos_ptr, mos_h, mos_w, pitch, dev = mosaic
@@ -416,6 +449,7 @@ class VisionTransformer(nn.Module):
         """get_last_selfattention(x)[:, :, queries, :] -> [B, heads, nq, N] fp32 for a list of query tokens (0 = CLS,
         1 + i = patch i; SSS/analyse_attention.py:183-247 region queries), without forming N x N.  With ``return_keys``
         also the last block's K features [B, heads, N, head_dim] (= qkv[1] of get_intermediate_feat; SSS/eval.py:186-202)."""
+        self._refuse_drop_path("attention_rows")
         x = self._check_input(x)
         eng = self._ensure_engine()
         B, _, H, W = x.shape
@@ -492,6 +526,23 @@ class VisionTransformer(nn.Module):
             return True
         return self.training and (self.pos_embed.requires_grad or any(p.requires_grad for p in self._encoder_grad_params().values()))
 
+    def _drop_path_probs(self):
+        return [blk.drop_path.drop_prob for blk in self.blocks]
+
+    def _drop_path_active(self) -> bool:
+        """Training mode with a positive stochastic-depth rate: the reference drops paths whenever ``self.training`` holds,
+        with or without autograd, so every feature call then runs the training forward (without a backward under no_grad)."""
+        return self.training and any(p > 0 for p in self._drop_path_probs())
+
+    def _refuse_drop_path(self, name):
+        if self._drop_path_active():
+            raise _lib.VitocmError(f"vitocm: {name} runs the inference kernels, which have no stochastic depth; this model is in "
+                                   f"training mode with drop_path_rate > 0 -- call .eval() first")
+
+    def _branch_scales(self, B, device):
+        """The scales of one training forward (draw_branch_scales) when drop path is active, else None (no drop path)."""
+        return draw_branch_scales(self._drop_path_probs(), B, device) if self._drop_path_active() else None
+
     def _encoder_grad_params(self):
         """{engine name: parameter} of everything vitocm_encoder_backward writes a gradient for (pos_embed excepted: its gradient
         is dpos, carried through the position-table graph).  A qkv bias that does not exist gets none."""
@@ -501,7 +552,7 @@ class VisionTransformer(nn.Module):
         """Differentiable [norm(x_l) for the last n_out blocks] through vitocm_encoder_train_forward / vitocm_encoder_backward."""
         if parse_precision(self.precision, self.depth)[0] == "fp32":
             raise _lib.VitocmError("vitocm: training runs on bf16 or fp16 engines only; build the encoder with precision='bf16' or "
-                                   "'fp16' (or call it under torch.no_grad() / .eval() for fp32-parity inference)")
+                                   "'fp16' (or call it under .eval(), or under torch.no_grad() without drop path, for fp32-parity inference)")
         if x.dim() == 4 and x.shape[1] == 1 and self.in_chans > 1:
             raise _lib.VitocmError(f"vitocm: gray [B, 1, H, W] inputs have no backward; pass the {self.in_chans}-channel image, "
                                    f"e.g. x.expand(-1, {self.in_chans}, -1, -1), or call under torch.no_grad()")
@@ -515,7 +566,8 @@ class VisionTransformer(nn.Module):
         N = self._tokens(xx)
         pos = self._pos_graph(N - 1, H, W)
         named = self._encoder_grad_params()
-        feats = _EncoderStep.apply(self, x, xx, n_out, pos, tuple(named), *named.values())
+        scales = self._branch_scales(xx.shape[0], xx.device)
+        feats = _EncoderStep.apply(self, x, xx, n_out, pos, scales, tuple(named), *named.values())
         return list(feats.unbind(0))
 
     def _bind_encoder_grads(self, names, dev):
@@ -544,8 +596,9 @@ class VisionTransformer(nn.Module):
 
     # ------------------------------------------------------------------ reference methods
     def forward_feats(self, x):
-        """vit.py:218-223 -> norm(x) [B, N, D]; differentiable under the rule of ``_differentiable``."""
-        if self._differentiable(x):
+        """vit.py:218-223 -> norm(x) [B, N, D]; differentiable under the rule of ``_differentiable``.  In training mode with
+        drop_path_rate > 0 it drops paths, under no_grad too."""
+        if self._differentiable(x) or self._drop_path_active():
             return self._encoder_train(x, 1)[0]
         return self._forward_feats(x)
 
@@ -562,13 +615,15 @@ class VisionTransformer(nn.Module):
     @torch.no_grad()
     def get_last_selfattention(self, x):
         """vit.py:239-246 -> attention of the last block, [B, heads, N, N] fp32."""
+        self._refuse_drop_path("get_last_selfattention")
         X = self.prepare_tokens(x)
         self._run_blocks(X, 0, self.depth - 1)
         return self._attn_probs(X, self.depth - 1)[0]
 
     def get_intermediate_layers(self, x, n=1):
-        """vit.py:248-256 -> [norm(x_i)] for the n last blocks; differentiable under the rule of ``_differentiable``."""
-        if self._differentiable(x):
+        """vit.py:248-256 -> [norm(x_i)] for the n last blocks; differentiable under the rule of ``_differentiable``.  In
+        training mode with drop_path_rate > 0 it drops paths, under no_grad too."""
+        if self._differentiable(x) or self._drop_path_active():
             return self._encoder_train(x, n)
         return self._get_intermediate_layers(x, n)
 
@@ -602,6 +657,7 @@ class VisionTransformer(nn.Module):
 
         With ``lazy`` (default) and n == 1 only the CLS attention rows are computed now; the
         returned objects materialise the full tensors on demand (see module docstring)."""
+        self._refuse_drop_path("get_intermediate_feat")
         if not lazy or n != 1:
             return self._intermediate_full(x, n)
         rows = self.cls_attention_rows(x)
@@ -623,10 +679,11 @@ class VisionTransformer(nn.Module):
 class _EncoderStep(torch.autograd.Function):
     """feats [n_out, B, N, D] = norm(x_l) of the last n_out blocks, with vitocm_encoder_backward as the backward.  The parameters
     are inputs, and their gradients come back through autograd, so .grad accumulation, hooks, optimizers and
-    torch.autograd.grad work as for any module.  ``x`` is an input for dx; ``xx`` is its fp32 contiguous copy the kernels read."""
+    torch.autograd.grad work as for any module.  ``x`` is an input for dx; ``xx`` is its fp32 contiguous copy the kernels read.
+    ``scales``: the stochastic-depth scales [depth, 2, B] of this forward, or None; the backward reads the workspace's copy."""
 
     @staticmethod
-    def forward(ctx, enc, x, xx, n_out, pos, names, *params):
+    def forward(ctx, enc, x, xx, n_out, pos, scales, names, *params):
         lib = _lib.load_library()
         eng = enc._engine
         B, _, H, W = xx.shape
@@ -637,8 +694,8 @@ class _EncoderStep(torch.autograd.Function):
             enc._train_ws = torch.empty(need, dtype=torch.uint8, device=xx.device)
         posc = pos.detach().to(torch.float32).contiguous()
         feats = torch.empty(n_out, B, N, enc.embed_dim, dtype=torch.float32, device=xx.device)
-        check(lib.vitocm_encoder_train_forward(eng, ptr(xx), B, H, W, ptr(posc), n_out, ptr(feats), ptr(enc._train_ws),
-                                               enc._train_ws.numel(), cur_stream()))
+        check(lib.vitocm_encoder_train_forward_dp(eng, ptr(xx), B, H, W, ptr(posc), n_out, ptr(feats), ptr(scales), ptr(enc._train_ws),
+                                                  enc._train_ws.numel(), cur_stream()))
         # the saved activations live in the encoder's one training workspace: stamp it, so that a backward whose forward has since
         # been overwritten by another differentiable forward fails loudly instead of producing wrong gradients
         enc._train_ws_gen += 1
@@ -668,7 +725,7 @@ class _EncoderStep(torch.autograd.Function):
         finally:
             enc._unbind_encoder_grads(bound)
         param_grads = [grads[n].view(shape) for n, shape in zip(ctx.names, ctx.shapes)]
-        return (None, None if dx is None else dx.to(ctx.x_dtype), None, None, dpos, None, *param_grads)
+        return (None, None if dx is None else dx.to(ctx.x_dtype), None, None, dpos, None, None, *param_grads)
 
 
 def vit_tiny(patch_size=16, **kwargs):
