@@ -103,6 +103,26 @@ int vitocm_set_concurrency(vitocm_engine* e, int lanes);
 int vitocm_forward_cls_attn(vitocm_engine* e, const float* x, int B, int H, int W, const float* pos, float* out_rows,
                             void* ws, size_t ws_bytes, int chunk_tiles, void* stream);
 
+/* Images of different sizes in one forward (the reference runs each image at its own size: SSS/eval.py:126-136,
+ * SSS/analyse_attention.py:113-177; its datasets only crop to a multiple of 8, SSS/data.py:29-30).  B images packed back to back in
+ * x as fp32 [C][H_i][W_i] (C = in_chans, or 1 for the gray channel-folded path of vitocm_forward_cls_attn_gray); hw host int
+ * [B][2] = (H_i, W_i), positive multiples of the patch size; N_i = (H_i/p)(W_i/p) + 1.  pos: the packed position tables, one per
+ * distinct size (each [N][D] fp32 as in vitocm_forward_cls_attn); pos_off host int [B]: image i's table starts at row pos_off[i].
+ * out_rows fp32: image i owns the [heads][N_i] block at heads * sum_{j<i} N_j.  The token rows of all images form one stream
+ * through every kernel that works on rows; patch embedding, attention and the CLS row take per-image geometry from tables the call
+ * writes into ws on `stream` (nothing allocated on the device).  Images are taken in order into chunks of at most
+ * chunk_tokens rows (<= 0: VITOCM_VARLEN_CHUNK_TOKENS); an image of more tokens than that runs alone.  One lane: the chunks run
+ * on `stream` one after the other (vitocm_set_concurrency does not apply).  Each image's rows are bit-identical to
+ * vitocm_forward_cls_attn(_gray) of that image alone on the same engine.  Refused: B < 1, a size that is not a multiple of the
+ * patch, an N_i whose CLS row does not fit the CLS-row kernel's shared memory, a workspace below
+ * vitocm_varlen_workspace_bytes(e, T) with T = the tokens of the largest chunk (at most max(chunk_tokens, largest N_i) and at most
+ * sum N_i).  The tables go to the device from pinned memory owned by the engine, in two slots used by calls in turn: a call waits on
+ * the host only for the table copies of the call before the previous one. */
+#define VITOCM_VARLEN_CHUNK_TOKENS 401920 /* 512 images of 224^2 at patch 8 */
+size_t vitocm_varlen_workspace_bytes(const vitocm_engine* e, int64_t chunk_tokens);
+int vitocm_forward_cls_attn_varlen(vitocm_engine* e, const float* x, int B, int C, const int* hw, const float* pos, const int* pos_off,
+                                   float* out_rows, void* ws, size_t ws_bytes, int64_t chunk_tokens, void* stream);
+
 /* Gray fast path of vitocm_forward_cls_attn: x [B][1][H][W] fp32 stands for an image whose in_chans channels are all equal
  * (every OCM tile of the reference: PIL "RGB" of a gray PNG, SSS/sw_processing.py:225-236).  The patch filter is folded over
  * the channels at vitocm_finalize_weights, so the patch-embedding GEMM contracts over p*p instead of in_chans*p*p taps and the
@@ -164,6 +184,11 @@ int vitocm_final_norm(vitocm_engine* e, const float* X, float* out, int M, void*
  * (a-min)/(max-min)*255 of SSS/sw_processing.py:253-254. */
 int vitocm_head_mean(const float* rows, float* lowres, int T, int heads, int n_tokens, int mode, void* stream);
 
+/* vitocm_head_mean for T images of different sizes packed as vitocm_forward_cls_attn_varlen writes them: patch_off device int [T + 1]
+ * = patches before image t (patch_off[T] = all); image t's rows are [heads][N_t] at heads (patch_off[t] + t), N_t = patch_off[t + 1]
+ * - patch_off[t] + 1, and its map lowres[patch_off[t] ...] [h_t][w_t]. */
+int vitocm_head_mean_varlen(const float* rows, float* lowres, int T, int heads, const int* patch_off, int mode, void* stream);
+
 /* Cumulative-mass threshold per head (the `--threshold` flag whose help text is at SSS/eval.py:33-34; the arithmetic is upstream
  * DINO's visualize_attention.py, not under /root/reference: parity unpinned by the reference, oracle = a PyTorch restatement):
  * per (tile, head) over the N - 1 patch columns of the CLS row: sort ascending, normalise by the sum, cumulative sum, keep the
@@ -180,6 +205,11 @@ int vitocm_attn_cummass(const float* rows, int T, int heads, int n_tokens, float
  * img_in [T][S][S] u8 (optional): the PIL "L" image, used instead of deriving it from x. */
 int vitocm_tile_threshold(const float* lowres, const float* x, int T, int C, int S, int lh, int lw, uint8_t* masks,
                           int* thresholds, float* att_out, const float* att_in, const uint8_t* img_in, void* stream);
+/* vitocm_tile_threshold for T square images of different sides: geo device int [T][4] = (S_t, l_t, patch offset, pixel offset):
+ * lowres [l_t][l_t] at the patch offset (vitocm_head_mean_varlen's layout), x [C][S_t][S_t] at C x the pixel offset, masks
+ * [3][S_t][S_t] at 3 x it and att_out [S_t][S_t] (or NULL) at it; thresholds [T][3]. */
+int vitocm_tile_threshold_varlen(const float* lowres, const float* x, int T, int C, const int* geo, uint8_t* masks, int* thresholds,
+                                 float* att_out, void* stream);
 /* The same with the two images utils.threshold also writes out (SSS/utils.py:77-81, saved at :107-108): aux [T][2][S][S] u8 =
  * (result = the 0.6 / 0.4 image / attention blend "weighted_iamge_attention.png", att_u8 = the normalised attention * 255). */
 int vitocm_tile_threshold_aux(const float* lowres, const float* x, int T, int C, int S, int lh, int lw, uint8_t* masks,
@@ -328,6 +358,11 @@ int vitocm_block_tail_folded(vitocm_engine* e, const void* CTX, int64_t ld_ctx, 
 /* ctx = MHSA(qkv) for B images of n_tokens tokens: qkv bf16 [B*N][ld] (columns [3][heads][head_dim]), ctx bf16 [B*N][ldo]. */
 int vitocm_attention(vitocm_engine* e, const void* qkv, int64_t ld, int B, int n_tokens, void* ctx, int64_t ldo,
                      void* stream);
+/* vitocm_attention for B images of n_tokens[i] (host int [B]) tokens packed back to back in qkv / ctx ([sum N_i] rows, no pad rows;
+ * the kernels of vitocm_forward_cls_attn_varlen).  ws: device memory for the work-item table (16 bytes per item; a too small ws is
+ * refused and the message names the size). */
+int vitocm_attention_varlen(vitocm_engine* e, const void* qkv, int64_t ld, int B, const int* n_tokens, void* ctx, int64_t ldo, void* ws,
+                            size_t ws_bytes, void* stream);
 /* Diagnostics: vitocm_attention that also records SM-clock stamps of the CTAs of query tiles 0 and 1 of
  * (image 0, head 0): stamps int64 [2 cta][2 role: softmax warp 0, MMA thread][16 kv blocks][8 events]. */
 int vitocm_attention_timeline(vitocm_engine* e, const void* qkv, int64_t ld, int B, int n_tokens, void* ctx, int64_t ldo,

@@ -18,7 +18,7 @@ from . import _lib  # noqa: F401
 from . import vision_transformer as vits  # noqa: F401
 from . import utils, sw_processing, model, optimizer, lr_scheduler, synthetic, pgt  # noqa: F401
 from .vision_transformer import VisionTransformer, vit_tiny, vit_small, vit_base, LazyAttention, LazyTensor  # noqa: F401
-from .utils import compute_attention, attention_masks, cropped_attention_masks, head_mean_maps, concat_crops_overlap  # noqa: F401
+from .utils import compute_attention, attention_masks, attention_masks_varlen, cropped_attention_masks, head_mean_maps, concat_crops_overlap  # noqa: F401
 from ._lib import VitocmError  # noqa: F401
 from .sw_processing import MosaicSegmenter, sliding_window, grid_size, mosaic_grid, shard_range, shared_pinned_u8  # noqa: F401
 from .model import VisionTransformerForSimMIM, MIM, MaskGenerator, build_model  # noqa: F401

@@ -33,6 +33,12 @@ SIGNATURES = {
     "vitocm_set_layer_mode": (c_int, [c_void_p, c_int, c_int]),
     "vitocm_forward_cls_attn": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_size_t,
                                         c_int, c_void_p]),
+    "vitocm_varlen_workspace_bytes": (c_size_t, [c_void_p, c_int64]),
+    "vitocm_forward_cls_attn_varlen": (c_int, [c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                               c_size_t, c_int64, c_void_p]),
+    "vitocm_attention_varlen": (c_int, [c_void_p, c_void_p, c_int64, c_int, c_void_p, c_void_p, c_int64, c_void_p, c_size_t, c_void_p]),
+    "vitocm_head_mean_varlen": (c_int, [c_void_p, c_void_p, c_int, c_int, c_void_p, c_int, c_void_p]),
+    "vitocm_tile_threshold_varlen": (c_int, [c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
     "vitocm_forward_cls_attn_gray": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_size_t,
                                              c_int, c_void_p]),
     "vitocm_forward_cls_attn_mosaic": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int64, c_int, c_int, c_int, c_int, c_int, c_void_p,

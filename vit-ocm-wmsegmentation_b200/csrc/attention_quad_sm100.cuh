@@ -70,7 +70,9 @@ __device__ __forceinline__ void aq_slot_mask(uint32_t (&m)[4]) {
   for (int w = 0; w < 4; ++w) m[w] = ((NS == 4 ? w : (NS == 2 ? (w >> 1) : 0)) == SL) ? 0u : 0xffffffffu;
 }
 
-template <bool F16, bool TL = false>   // TL: clock stamps of tools/attn_quad_timeline.py (a separate instantiation: the stamps cost registers)
+// TL: clock stamps of tools/attn_quad_timeline.py (a separate instantiation: the stamps cost registers)
+// VARLEN: items come from AttnArgs::vitems (images of different sizes packed back to back, see att_vdecode)
+template <bool F16, bool TL = false, bool VARLEN = false>
 __global__ void __launch_bounds__(AQ_THREADS, 1)
 attn_fwd_quad_kernel(const __grid_constant__ CUtensorMap tmap_q /*box 64 x 128*/, const __grid_constant__ CUtensorMap tmap_kv /*box 64 x 64*/,
                      const __grid_constant__ CUtensorMap tmap_q32 /*box 64 x 32: the query slots of packed tail items*/, const AttnArgs args) {
@@ -139,8 +141,9 @@ attn_fwd_quad_kernel(const __grid_constant__ CUtensorMap tmap_q /*box 64 x 128*/
     if (ptx::elect_one()) {
       const uint32_t s_tmem = tmem_base + AQ_S_COL, o_tmem = tmem_base + AQ_O_COL;
       const uint64_t q_desc = ptx::make_smem_desc_sw128(smem_q, 1024, 0);
+      int Ni = N;   // tokens of the current item's image (VARLEN: per item)
       auto kv_len_mma = [&](int j) {   // keys of block j rounded up to the MMA granularity (16)
-        int len = N - j * AQ_BKV;
+        int len = Ni - j * AQ_BKV;
         len = len > AQ_BKV ? AQ_BKV : len;
         return (len + 15) & ~15;
       };
@@ -148,6 +151,19 @@ attn_fwd_quad_kernel(const __grid_constant__ CUtensorMap tmap_q /*box 64 x 128*/
       auto clamp_pair = [&](int pr) { return pr < args.n_pairs ? pr : args.n_pairs - 1; };
       auto load_q = [&](int it) {
         int pair0, qt, ns;
+        if constexpr (VARLEN) {
+          int row0, n, h0;
+          att_vdecode(args, it, row0, n, qt, h0, ns);
+          ptx::mbar_arrive_expect_tx(q_full, AQ_Q_BYTES);
+          if (ns == 1) {
+            ptx::tma_load_2d(smem_q, &tmap_q, q_full, h0 * ATT_DH, row0 + qt * ATT_BQ);
+          } else {
+            const int per = 4 / ns;
+            for (int u = 0; u < 4; ++u)
+              ptx::tma_load_2d(smem_q + u * 4096, &tmap_q32, q_full, min(h0 + u / per, args.heads - 1) * ATT_DH, row0 + qt * ATT_BQ + (u % per) * 32);
+          }
+          return;
+        }
         aq_decode(args, it, pair0, qt, ns);
         ptx::mbar_arrive_expect_tx(q_full, AQ_Q_BYTES);
         if (ns == 1) {
@@ -166,10 +182,17 @@ attn_fwd_quad_kernel(const __grid_constant__ CUtensorMap tmap_q /*box 64 x 128*/
       // K / V stream in consumption order (per block: K of every slot, then V of every slot), running across the items of this pipeline
       int loaded = 0, used = 0;          // tiles requested / handed to an MMA
       int l_it = first, l_j = 0, l_which = 1, l_sl = 0, l_ns = 1;   // next tile to request: item, block, 1 = K / 2 = V, slot; slots of the item
-      int l_col = 0, l_row = 0;
+      int l_col = 0, l_row = 0, l_nkv = n_kv;
       auto set_load_coords = [&]() {
         if (l_it < args.n_items) {
           int pair0, qt;
+          if constexpr (VARLEN) {
+            int n, h0;
+            att_vdecode(args, l_it, l_row, n, qt, h0, l_ns);
+            l_col = min(h0 + l_sl, args.heads - 1) * ATT_DH;
+            l_nkv = (n + AQ_BKV - 1) / AQ_BKV;
+            return;
+          }
           aq_decode(args, l_it, pair0, qt, l_ns);
           const int pr = clamp_pair(pair0 + l_sl);
           const int b = pr / args.heads;
@@ -192,7 +215,7 @@ attn_fwd_quad_kernel(const __grid_constant__ CUtensorMap tmap_q /*box 64 x 128*/
               l_which = 2;
             } else {
               l_which = 1;
-              if (++l_j == n_kv) { l_j = 0; l_it += stride; recode = true; }
+              if (++l_j == l_nkv) { l_j = 0; l_it += stride; recode = true; }
             }
           }
           if (recode) set_load_coords();
@@ -240,12 +263,18 @@ attn_fwd_quad_kernel(const __grid_constant__ CUtensorMap tmap_q /*box 64 x 128*/
       int w = 0;   // items so far: phase of q_full / o_full / o_empty
       for (int it = first; it < args.n_items; it += stride, ++w) {
         const bool tl = TL && args.timeline != nullptr && blockIdx.x == 0 && p < 2 && w == args.timeline_item;
-        int nslots, pair0_unused, qt_unused;
+        int nslots, pair0_unused, qt_unused, nkv = n_kv;
+        if constexpr (VARLEN) {
+          int r0_unused, h0_unused;
+          att_vdecode(args, it, r0_unused, Ni, qt_unused, h0_unused, nslots);
+          nkv = (Ni + AQ_BKV - 1) / AQ_BKV;
+        } else {
         aq_decode(args, it, pair0_unused, qt_unused, nslots);
+        }
         ptx::mbar_wait(q_full, w & 1, 51);
         issue_s(0, nslots);
         if constexpr (TL) att_stamp(args, tl, 1, 0, 0, p);   // S_0 issued
-        for (int j = 0; j < n_kv; ++j, ++g) {
+        for (int j = 0; j < nkv; ++j, ++g) {
           fill();
           constexpr uint32_t idesc_pv = ptx::make_idesc(ATT_BQ, ATT_DH, false, /*B = V is MN-major*/ true, F16 ? 0u : 1u);
           const int ksteps = kv_len_mma(j) / 16;
@@ -254,7 +283,7 @@ attn_fwd_quad_kernel(const __grid_constant__ CUtensorMap tmap_q /*box 64 x 128*/
             // Everything PV_j and S_{j+1} need is prepared BEFORE the wait for P_j: the control warp shares its scheduler with four
             // softmax warps, so every instruction between "P_j seen" and the last MMA costs ~5 clk of the pipeline's serial chain
             // (descriptor arithmetic + operand-landed checks behind the wait: 850 clk from P_j to S_{j+1} issued, of ~3 250 per block)
-            const bool more = j + 1 < n_kv;
+            const bool more = j + 1 < nkv;
             const int slot_v = used % AQ_RING, slot_k = (used + 1) % AQ_RING;
             ptx::mbar_wait(kv_full + 8 * slot_v, (used / AQ_RING) & 1, 55);
             if (more) ptx::mbar_wait(kv_full + 8 * slot_k, ((used + 1) / AQ_RING) & 1, 52);
@@ -312,7 +341,7 @@ attn_fwd_quad_kernel(const __grid_constant__ CUtensorMap tmap_q /*box 64 x 128*/
               ptx::umma_bf16_ts(o_tmem, s_tmem + k * 8, ptx::desc_advance(v_desc, k * 2048), idesc_pv, k ? 1u : acc0);
             ptx::umma_commit(kv_empty + 8 * slot);
             ++used;
-            if (j == n_kv - 1) ptx::umma_commit(o_full);
+            if (j == nkv - 1) ptx::umma_commit(o_full);
           } else {
             auto slot_pv = [&](auto ns_tag, auto sl_tag) {
               if (loaded <= used) fill();
@@ -338,10 +367,10 @@ attn_fwd_quad_kernel(const __grid_constant__ CUtensorMap tmap_q /*box 64 x 128*/
             using I2 = std::integral_constant<int, 2>; using I3 = std::integral_constant<int, 3>; using I4 = std::integral_constant<int, 4>;
             if (nslots == 2) { slot_pv(I2{}, I0{}); slot_pv(I2{}, I1{}); }
             else { slot_pv(I4{}, I0{}); slot_pv(I4{}, I1{}); slot_pv(I4{}, I2{}); slot_pv(I4{}, I3{}); }
-            if (j == n_kv - 1) ptx::umma_commit(o_full);
+            if (j == nkv - 1) ptx::umma_commit(o_full);
           }
           if constexpr (TL) att_stamp(args, tl, 1, j, 2, p);   // PV_j issued
-          if (j + 1 < n_kv) {
+          if (j + 1 < nkv) {
             issue_s(j + 1, nslots);
             if constexpr (TL) att_stamp(args, tl, 1, j + 1, 0, p);   // S_{j+1} issued
           } else if (it + stride < args.n_items) {
@@ -364,8 +393,17 @@ attn_fwd_quad_kernel(const __grid_constant__ CUtensorMap tmap_q /*box 64 x 128*/
       const bool tl = TL && args.timeline != nullptr && blockIdx.x == 0 && p < 2 && q == 0 && lane == 0 && w == args.timeline_item;
       float m_used = -INFINITY;   // the row maximum the exponentials are taken against
       float l_run = 0.f;          // running row sum (same units as O in TMEM)
-      for (int j = 0; j < n_kv; ++j, ++g) {
-        int kv_len = N - j * AQ_BKV;
+      int Ni = N, nkv = n_kv;
+      bool votes = true;   // VARLEN: only rows of the item's own image and heads vote on a redo (see attn_fwd_tcgen05_kernel)
+      if constexpr (VARLEN) {
+        int r0_unused, vqt, vh0, vns;
+        att_vdecode(args, it, r0_unused, Ni, vqt, vh0, vns);
+        nkv = (Ni + AQ_BKV - 1) / AQ_BKV;
+        const int slot_rows = ATT_BQ / vns, sl = r / slot_rows;
+        votes = vh0 + sl < args.heads && vqt * ATT_BQ + (r - sl * slot_rows) < Ni;
+      }
+      for (int j = 0; j < nkv; ++j, ++g) {
+        int kv_len = Ni - j * AQ_BKV;
         kv_len = kv_len > AQ_BKV ? AQ_BKV : kv_len;
         const int nchunks = (((kv_len + 15) & ~15) + 31) >> 5;   // 32-column chunks the MMA produced
         if constexpr (TL) att_stamp(args, tl, 0, j, 0, p);     // waiting for S_j
@@ -420,7 +458,7 @@ attn_fwd_quad_kernel(const __grid_constant__ CUtensorMap tmap_q /*box 64 x 128*/
             };
             run_exps();
             // !(csum <= T) also catches inf / NaN sums
-            if ((j > 0 || c > 0) && __any_sync(0xffffffffu, !(csum <= (F16 ? ATT_SUM_TRIGGER_F16 : ATT_SUM_TRIGGER)))) {
+            if ((j > 0 || c > 0) && __any_sync(0xffffffffu, votes && !(csum <= (F16 ? ATT_SUM_TRIGGER_F16 : ATT_SUM_TRIGGER)))) {
               const float m_new = fmaxf(m_used, chunk_max());
               const float a = ptx::ex2_approx((m_used - m_new) * sl2);
               m_used = m_new;
@@ -480,6 +518,17 @@ attn_fwd_quad_kernel(const __grid_constant__ CUtensorMap tmap_q /*box 64 x 128*/
       __syncwarp();
       if (lane == 0) ptx::mbar_arrive(o_empty);   // the next item's first PV may overwrite O
       int pair, qrow;
+      __nv_bfloat16* o;
+      bool row_ok;
+      if constexpr (VARLEN) {
+        int row0, qt, h0, ns;
+        att_vdecode(args, it, row0, Ni, qt, h0, ns);
+        const int slot_rows = ATT_BQ / ns, sl = r / slot_rows;
+        const int h = h0 + sl;
+        qrow = qt * ATT_BQ + (r - sl * slot_rows);
+        row_ok = h < args.heads && qrow < Ni;   // a ragged tile's rows beyond its image belong to the next image: never written
+        o = args.out + static_cast<long long>(row0 + qrow) * args.ldo + h * ATT_DH;
+      } else {
       {
         int pair0, qt, ns;
         aq_decode(args, it, pair0, qt, ns);
@@ -487,10 +536,11 @@ attn_fwd_quad_kernel(const __grid_constant__ CUtensorMap tmap_q /*box 64 x 128*/
         pair = pair0 + sl;
         qrow = qt * ATT_BQ + (r - sl * slot_rows);
       }
-      const bool row_ok = pair < args.n_pairs && qrow < N;
+      row_ok = pair < args.n_pairs && qrow < N;
       if (!row_ok) pair = 0;
       const int b = pair / args.heads, h = pair - b * args.heads;
-      __nv_bfloat16* o = args.out + static_cast<long long>(b * N + qrow) * args.ldo + h * ATT_DH;
+      o = args.out + static_cast<long long>(b * N + qrow) * args.ldo + h * ATT_DH;
+      }
       if (row_ok)
 #pragma unroll
       for (int c = 0; c < ATT_DH / 32; ++c) {

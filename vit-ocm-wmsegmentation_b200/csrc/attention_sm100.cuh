@@ -66,7 +66,16 @@ struct AttnArgs {
   long long* timeline;  // diagnostics (vitocm_attention_timeline) or nullptr: clock64 stamps of CTAs (0,0,0) and (1,0,0)
   int stagger_clk;      // attn_fwd_quad_kernel: CTA k starts k / gridDim.x x stagger_clk SM clocks late (VITOCM_ATTN_STAGGER) -- every CTA
                         // does the same work in the same time, so without it all of them load K / V and drain O in the same instants
+  const int4* vitems;   // VARLEN kernels (images of different sizes packed back to back): item it = {token base of its image, N of its image,
+                        // query tile, first head | slots << 16}; a packed tail item's slot s is head first + s of that image (heads beyond
+                        // the last are computed against the last head and dropped).  n_tokens is unused.
 };
+
+// VARLEN work item it -> (token base, N, query tile, first head, slots)
+__device__ __forceinline__ void att_vdecode(const AttnArgs& a, int it, int& row0, int& n, int& qt, int& h0, int& nslots) {
+  const int4 v = __ldg(a.vitems + it);
+  row0 = v.x; n = v.y; qt = v.z; h0 = v.w & 0xffff; nslots = v.w >> 16;
+}
 
 // timeline layout: [cta 0..1][role 0 = softmax warp 0, 1 = MMA thread][kv block j < 16][event < 8]
 constexpr int ATT_TL_EVENTS = 8;
@@ -160,7 +169,9 @@ __device__ __forceinline__ void att_slot_mask(int s, int nslots, uint32_t (&m)[4
 //      exp2 of (logit - running maximum) <= 2^ATT_RESCALE_THRESHOLD, or <= 2^redo threshold inside one block: the redo threshold
 //      drops to 14 so that P stays below fp16's 65504; below 6e-8 P flushes to zero, like everything under 2^-24 of the row sum.
 // DH: head_dim (64 or 128, see AttnCfg)
-template <bool SPLIT, uint32_t POLY_MASK, bool PACKED, bool F16 = false, int DH = 64>
+// VARLEN: items come from AttnArgs::vitems (images of different sizes, PACKED only); rows of a ragged tile beyond its image are read
+//         from the next image's rows and never written
+template <bool SPLIT, uint32_t POLY_MASK, bool PACKED, bool F16 = false, int DH = 64, bool VARLEN = false>
 __global__ void __launch_bounds__(ATT_THREADS, AttnCfg<SPLIT, DH>::ONE_CTA ? 1 : 2)
 attn_fwd_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __grid_constant__ CUtensorMap tmap_q32, const AttnArgs args) {
   using Cfg = AttnCfg<SPLIT, DH>;
@@ -231,13 +242,37 @@ attn_fwd_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __gr
       for (int it = blockIdx.x; it < args.n_items; it += gridDim.x) {
       int qt, pair0;
       bool packed;
+      int nslots, nkv = n_kv, vrow0 = 0, vh0 = 0;
+      if constexpr (VARLEN) {
+        int vn;
+        att_vdecode(args, it, vrow0, vn, qt, vh0, nslots);
+        nkv = (vn + ATT_BKV - 1) / ATT_BKV;
+        packed = nslots > 1;
+        pair0 = 0;
+      } else {
       if (!att_decode<PACKED>(args, it, qt, pair0, packed)) continue;
-      const int nslots = (PACKED && packed) ? args.pack : 1;
+      nslots = (PACKED && packed) ? args.pack : 1;
+      }
       // pair of slot s (slots beyond the batch repeat the last pair: their rows are computed and dropped)
       auto pair_of = [&](int s) { const int pr = pair0 + s; return pr < args.n_pairs ? pr : args.n_pairs - 1; };
       ptx::mbar_wait(q_empty, (w & 1) ^ 1, 16);   // the previous item's S MMAs have retired
       ptx::mbar_arrive_expect_tx(q_full, Cfg::Q_BYTES);
-      if (!PACKED || !packed) {
+      if constexpr (VARLEN) {
+        const int per = 4 / nslots;
+        for (int part = 0; part < NPART; ++part)
+          for (int at = 0; at < ATOMS; ++at) {
+            if (nslots == 1) {
+              ptx::tma_load_2d(smem_q + part * Cfg::PART_BYTES + at * ATT_TILE_BYTES, &tmap_qkv, q_full,
+                               part * args.lo_col_off + vh0 * DH + at * 64, vrow0 + qt * ATT_BQ);
+            } else {
+              for (int u = 0; u < 4; ++u) {
+                const int h = min(vh0 + u / per, args.heads - 1);
+                ptx::tma_load_2d(smem_q + part * Cfg::PART_BYTES + at * ATT_TILE_BYTES + u * 4096, &tmap_q32, q_full,
+                                 part * args.lo_col_off + h * DH + at * 64, vrow0 + qt * ATT_BQ + (u % per) * 32);
+              }
+            }
+          }
+      } else if (!PACKED || !packed) {
         const int b = pair0 / args.heads, h = pair0 - b * args.heads;
         for (int part = 0; part < NPART; ++part)
           for (int at = 0; at < ATOMS; ++at)
@@ -258,10 +293,15 @@ attn_fwd_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __gr
       // ring order = consumption order of the MMA warp: K0, K1, V0, K2, V1, ..., V_{n-1} (each entry = one tile per slot)
       int kv_col[4], kv_row[4];   // per slot: first column (head) and first row (image) of its pair's K / V, decoded once per item
       for (int sl = 0; sl < nslots; ++sl) {
+        if constexpr (VARLEN) {
+          kv_col[sl] = min(vh0 + sl, args.heads - 1) * DH;
+          kv_row[sl] = vrow0;
+        } else {
         const int pr = pair_of(sl);
         const int b = pr / args.heads;
         kv_col[sl] = (pr - b * args.heads) * DH;
         kv_row[sl] = b * N;
+        }
       }
       auto load = [&](int which /*1 = K, 2 = V*/, int j) {
         for (int sl = 0; sl < nslots; ++sl) {
@@ -277,8 +317,8 @@ attn_fwd_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __gr
         }
       };
       load(1, 0);
-      for (int j = 0; j < n_kv; ++j) {
-        if (j + 1 < n_kv) load(1, j + 1);
+      for (int j = 0; j < nkv; ++j) {
+        if (j + 1 < nkv) load(1, j + 1);
         load(2, j);
       }
       ++w;
@@ -298,11 +338,18 @@ attn_fwd_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __gr
       for (int it = blockIdx.x; it < args.n_items; it += gridDim.x) {
       int qt_unused, pair0_unused;
       bool packed;
+      int nslots, Ni = N, nkv = n_kv;
+      if constexpr (VARLEN) {
+        int r0_unused, h0_unused;
+        att_vdecode(args, it, r0_unused, Ni, qt_unused, h0_unused, nslots);
+        nkv = (Ni + ATT_BKV - 1) / ATT_BKV;
+      } else {
       if (!att_decode<PACKED>(args, it, qt_unused, pair0_unused, packed)) continue;
-      const int nslots = (PACKED && packed) ? args.pack : 1;
+      nslots = (PACKED && packed) ? args.pack : 1;
+      }
       const bool tl = tl0 && w == args.timeline_item;
       auto kv_len_mma = [&](int j) {  // keys of block j rounded up to the MMA granularity (16)
-        int len = N - j * ATT_BKV;
+        int len = Ni - j * ATT_BKV;
         len = len > ATT_BKV ? ATT_BKV : len;
         return (len + 15) & ~15;
       };
@@ -414,13 +461,13 @@ attn_fwd_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __gr
       if (g > 0) ptx::mbar_wait(s_empty, (g - 1) & 1, 14);   // the previous item's last S has been read out of TMEM
       ptx::tc_fence_after();
       issue_s(0);
-      if (n_kv == 1) ptx::umma_commit(q_empty);
-      for (int j = 0; j < n_kv; ++j, ++g) {
-        if (j + 1 < n_kv) {
+      if (nkv == 1) ptx::umma_commit(q_empty);
+      for (int j = 0; j < nkv; ++j, ++g) {
+        if (j + 1 < nkv) {
           ptx::mbar_wait(s_empty, g & 1, 14);  // softmax has read S_j out of TMEM
           ptx::tc_fence_after();
           issue_s(j + 1);
-          if (j + 2 == n_kv) ptx::umma_commit(q_empty);   // last S MMA of the item: Q tile reusable once it retires
+          if (j + 2 == nkv) ptx::umma_commit(q_empty);   // last S MMA of the item: Q tile reusable once it retires
         }
         ptx::mbar_wait(p_full, g & 1, 15);     // P_j in TMEM, O rescaled if needed
         ptx::tc_fence_after();
@@ -441,7 +488,18 @@ attn_fwd_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __gr
     int g = 0;                    // KV blocks processed so far (all work items): barrier phase counter
     int w = 0;
     for (int it = blockIdx.x; it < args.n_items; it += gridDim.x) {
-    {
+    int Ni = N, nkv = n_kv;
+    // VARLEN: only rows of the item's own image and heads take part in the warp-wide redo decisions below.  The other rows of a
+    // ragged tile are the next image's queries (no pad rows); in the call for the image alone they are zero rows (TMA fill), whose
+    // exponentials sum to at most one per key and never trip a decision -- so the decisions, and every row's bits, are the same.
+    bool votes = true;
+    if constexpr (VARLEN) {
+      int r0_unused, vqt, vh0, vns;
+      att_vdecode(args, it, r0_unused, Ni, vqt, vh0, vns);
+      nkv = (Ni + ATT_BKV - 1) / ATT_BKV;
+      const int slot_rows = ATT_BQ / vns, sl = r / slot_rows;
+      votes = vh0 + sl < args.heads && vqt * ATT_BQ + (r - sl * slot_rows) < Ni;
+    } else {
       int qt0, pair00;
       bool packed0;
       if (!att_decode<PACKED>(args, it, qt0, pair00, packed0)) continue;   // (decoded again for the epilogue: nothing of it stays live over the KV loop)
@@ -451,8 +509,8 @@ attn_fwd_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __gr
     float m_next = -INFINITY;     // a larger maximum seen in the previous block (lazy rescale pending)
     float l_run = 0.f;            // running row sum (same units as O in TMEM)
 
-    for (int j = 0; j < n_kv; ++j, ++g) {
-      int kv_len = N - j * ATT_BKV;
+    for (int j = 0; j < nkv; ++j, ++g) {
+      int kv_len = Ni - j * ATT_BKV;
       kv_len = kv_len > ATT_BKV ? ATT_BKV : kv_len;
       const int nchunks = (((kv_len + 15) & ~15) + 31) >> 5;   // 32-column chunks the MMA produced
       att_stamp(args, tl && warp == 0, 0, j, 0);   // waiting for S_j
@@ -566,7 +624,7 @@ attn_fwd_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __gr
         ptx::unpack_f32x2(sum2[1], b0, b1);
         const float bsum = (a0 + a1) + (b0 + b1);
         // !(bsum <= T) also catches inf / NaN sums
-        if (__any_sync(0xffffffffu, !(bsum <= (F16 ? ATT_SUM_TRIGGER_F16 : ATT_SUM_TRIGGER)))) {
+        if (__any_sync(0xffffffffu, votes && !(bsum <= (F16 ? ATT_SUM_TRIGGER_F16 : ATT_SUM_TRIGGER)))) {
           const float m_blk = row_max();
           const float m_new = fmaxf(m_used, m_blk);
           const float a = ptx::ex2_approx((m_used - m_new) * sl2);
@@ -578,7 +636,7 @@ attn_fwd_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __gr
       } else if (j > 0) {
         const float excess = (row_max() - m_used) * sl2;       // independent of the exponentials above: overlaps them
         constexpr float REDO = F16 ? ATT_REDO_THRESHOLD_F16 : ATT_REDO_THRESHOLD;
-        if (__any_sync(0xffffffffu, excess > REDO)) {
+        if (__any_sync(0xffffffffu, votes && excess > REDO)) {
           // rare: a row jumped so far above the running maximum that exp2 may have overflowed -> raise the maximum
           // now (O is complete up to block j-1 and may be rescaled here) and redo this block's exponentials
           const float m_new = excess > REDO ? m_used + excess / sl2 : m_used;
@@ -611,19 +669,33 @@ attn_fwd_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __gr
     // this thread's row: tile row r of an ordinary item; in a packed item row (r % slot_rows) of the tail of pair0 + r / slot_rows
     int qt, pair0;
     bool packed;
+    int my_pair, row_in_tile = r, slot_rows = ATT_BQ, h, row_base;
+    bool pair_ok;
+    if constexpr (VARLEN) {
+      int vh0, ns;
+      att_vdecode(args, it, row_base, Ni, qt, vh0, ns);
+      slot_rows = ATT_BQ / ns;
+      const int sl = r / slot_rows;
+      row_in_tile = r - sl * slot_rows;
+      h = vh0 + sl;
+      pair_ok = h < args.heads;
+      my_pair = 0;
+    } else {
     att_decode<PACKED>(args, it, qt, pair0, packed);
-    int my_pair = pair0, row_in_tile = r, slot_rows = ATT_BQ;
+    my_pair = pair0;
     if (PACKED && packed) {
       slot_rows = ATT_BQ / args.pack;
       const int sl = r / slot_rows;
       row_in_tile = r - sl * slot_rows;
       my_pair = pair0 + sl;
     }
-    const bool pair_ok = my_pair < args.n_pairs;
-    const int b = my_pair / args.heads, h = my_pair - b * args.heads;
-    const int row_base = b * N;
+    pair_ok = my_pair < args.n_pairs;
+    const int b = my_pair / args.heads;
+    h = my_pair - b * args.heads;
+    row_base = b * N;
+    }
     const int qrow = qt * ATT_BQ + row_in_tile;
-    if (args.lse2 != nullptr && pair_ok) {   // pad rows get +inf: the backward turns that into P = 0 without a bounds test
+    if (!VARLEN && args.lse2 != nullptr && pair_ok) {   // pad rows get +inf: the backward turns that into P = 0 without a bounds test
       float* lrow = args.lse2 + static_cast<long long>(my_pair) * (args.n_qtiles * ATT_BQ);
       lrow[qrow] = qrow < N ? m_used * sl2 + log2f(l_run) : INFINITY;
       for (int k = slot_rows; k < ATT_BQ; k += slot_rows) lrow[qrow + k] = INFINITY;   // packed item: the rest of the pad rows
@@ -643,7 +715,7 @@ attn_fwd_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __gr
         __syncwarp();
         if (lane == 0) ptx::mbar_arrive(o_empty);
       }
-      if (qrow < N && pair_ok) {
+      if (qrow < Ni && pair_ok) {
 #pragma unroll
         for (int c = 0; c < 2; ++c) {
 #pragma unroll

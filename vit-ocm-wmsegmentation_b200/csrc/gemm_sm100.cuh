@@ -83,7 +83,22 @@ struct GemmArgs {
   // EPI_RESID_SCALED_F32 only: per-sample residual-branch scale (stochastic depth, vit.py:110-111), [M / rows_per_scale]
   const float* row_scale;
   int rows_per_scale;
+  // PATCH_VAR only (images of different sizes packed back to back, no mask, no mosaic): vimg[b] = {patches before image b, patches per
+  // row of image b, row of image b's CLS entry in the packed position tables pos, 0}, b < n_img, and vimg[n_img].x = M.  Image b's pixels
+  // start at img + C p^2 vimg[b].x, its token rows at vimg[b].x + b of X; img_h, img_w and n_patches are unused.
+  const int4* vimg;
+  int n_img;
 };
+
+// PATCH_VAR: the image of patch row m (the last b with vimg[b].x <= m)
+__device__ __forceinline__ int patch_image(const GemmArgs& a, int m) {
+  int lo = 0, hi = a.n_img - 1;
+  while (lo < hi) {
+    const int mid = (lo + hi + 1) >> 1;
+    if (__ldg(&a.vimg[mid].x) <= m) lo = mid; else hi = mid - 1;
+  }
+  return lo;
+}
 
 constexpr int GEMM_BM = 128;
 constexpr int GEMM_BK = 64;
@@ -289,7 +304,8 @@ __device__ __forceinline__ void gelu5_grad_mul_x2(float& v0, float& v1, float x0
   ptx::unpack_f32x2(r, v0, v1);
 }
 
-template <int BN, int EPI, bool A_PATCH, bool B_RES = false, int CS = 1, bool PAIR = false>
+// PATCH_VAR: patch embedding of images of different sizes (GemmArgs::vimg); A_PATCH and EPI_PATCH_F32 only
+template <int BN, int EPI, bool A_PATCH, bool B_RES = false, int CS = 1, bool PAIR = false, bool PATCH_VAR = false>
 __global__ void __launch_bounds__(gemm_threads(BN, EPI), 1)
 gemm_bf16_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ CUtensorMap tmap_b,
                          const __grid_constant__ CUtensorMap tmap_c, const __grid_constant__ CUtensorMap tmap_d, const GemmArgs args) {
@@ -300,6 +316,7 @@ gemm_bf16_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __gri
   static_assert(LN || CS == 1, "clusters are only used by the fused-LayerNorm epilogue");
   static_assert(!(LN && (A_PATCH || B_RES)), "fused LayerNorm uses the plain pipeline");
   static_assert(!(A_PATCH && B_RES), "patch embedding uses the plain pipeline");
+  static_assert(!PATCH_VAR || (A_PATCH && EPI == EPI_PATCH_F32), "PATCH_VAR is a patch-embedding mode");
   const int STAGES = B_RES ? args.stages : Cfg::STAGES;
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   // SWIZZLE_128B tiles need 1024-byte alignment; all later accesses use 32-bit shared-window addresses
@@ -481,7 +498,7 @@ gemm_bf16_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __gri
           ptx::mbar_wait(empty_bar + 8 * stage, phase ^ 1, 5);
           const uint32_t a_tile = smem_a + stage * Cfg::A_BYTES;
           // 4 items per thread: all 8 loads are issued before the first conversion so that their latencies overlap
-          if (args.mos != nullptr) {   // gray uint8 mosaic: 8 pixels = 8 bytes of one mosaic row
+          if (!PATCH_VAR && args.mos != nullptr) {   // gray uint8 mosaic: 8 pixels = 8 bytes of one mosaic row
             uint2 raw[4];
 #pragma unroll
             for (int u = 0; u < 4; ++u) {
@@ -535,13 +552,26 @@ gemm_bf16_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __gri
               f[u][0] = make_float4(0.f, 0.f, 0.f, 0.f);
               f[u][1] = f[u][0];
               if (m < args.M) {
+                const float* src;
+                if constexpr (PATCH_VAR) {
+                  const int b = patch_image(args, m);
+                  const int4 g = __ldg(args.vimg + b);
+                  const int i = m - g.x, wpb = g.y, nb = __ldg(&args.vimg[b + 1].x) - g.x;
+                  const int py = i / wpb, px = i - py * wpb;
+                  const int k = kb * GEMM_BK + chunk * 8;
+                  const int c = k / pp, rem = k - c * pp;
+                  const int yi = rem / p, xi = rem - yi * p;
+                  src = args.img + (static_cast<long long>(g.x) * chans + static_cast<long long>(c) * nb) * pp +
+                        static_cast<long long>(py * p + yi) * (wpb * p) + px * p + xi;
+                } else {
                 const int b = m / args.n_patches, i = m - b * args.n_patches;
                 const int py = i / Wp, px = i - py * Wp;
                 const int k = kb * GEMM_BK + chunk * 8;
                 const int c = k / pp, rem = k - c * pp;
                 const int yi = rem / p, xi = rem - yi * p;
-                const float* src = args.img + (static_cast<long long>(b) * chans + c) * plane +
+                src = args.img + (static_cast<long long>(b) * chans + c) * plane +
                                    static_cast<long long>(py * p + yi) * args.img_w + px * p + xi;
+                }
                 f[u][0] = __ldg(reinterpret_cast<const float4*>(src));
                 f[u][1] = __ldg(reinterpret_cast<const float4*>(src) + 1);
               }
@@ -742,7 +772,19 @@ gemm_bf16_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __gri
         // boundary -- one in ~49 -- keep the per-lane path.
         bool patch_fast = false;
         int patch_i0 = 0, patch_b0 = 0;
-        if (EPI == EPI_PATCH_F32) {
+        int patch_pos0 = 0, patch_tok0 = 0;   // PATCH_VAR: first position / token row of the warp's image
+        if constexpr (PATCH_VAR) {   // (a warp's 32 rows inside one image: one position box in, one token box out, as below)
+          patch_b0 = patch_image(args, row_base < args.M ? row_base : args.M - 1);
+          const int4 g = __ldg(args.vimg + patch_b0);
+          patch_i0 = row_base - g.x;
+          patch_pos0 = g.z;
+          patch_tok0 = g.x + patch_b0;
+          patch_fast = args.patch_tma != 0 && row_base + 32 <= args.M && g.x + patch_i0 + 32 <= __ldg(&args.vimg[patch_b0 + 1].x);
+          if (patch_fast && lane == 0) {
+            ptx::mbar_arrive_expect_tx(xin_bar + 8 * ew, 4096);
+            ptx::tma_load_2d(stg_warp, &tmap_d, xin_bar + 8 * ew, col, patch_pos0 + 1 + patch_i0);
+          }
+        } else if (EPI == EPI_PATCH_F32) {
           patch_b0 = row_base / args.n_patches;
           patch_i0 = row_base - patch_b0 * args.n_patches;
           patch_fast = args.patch_tma != 0 && row_base + 32 <= args.M && patch_i0 + 32 <= args.n_patches;
@@ -866,12 +908,23 @@ gemm_bf16_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __gri
             ptx::fence_proxy_async_smem();
             __syncwarp();
             if (lane == 0) {
-              ptx::tma_store_2d(&tmap_c, stg_warp + 4096, col, patch_b0 * (args.n_patches + 1) + 1 + patch_i0);
+              ptx::tma_store_2d(&tmap_c, stg_warp + 4096, col, PATCH_VAR ? patch_tok0 + 1 + patch_i0 : patch_b0 * (args.n_patches + 1) + 1 + patch_i0);
               ptx::bulk_commit();
             }
             continue;
           }
-          if (m < args.M) {
+          if (PATCH_VAR && m < args.M) {
+            const int b = patch_image(args, m);
+            const int4 g = __ldg(args.vimg + b);
+            const int i = m - g.x;
+            const float4* pr = reinterpret_cast<const float4*>(args.pos + static_cast<long long>(g.z + 1 + i) * args.N + col);
+            float4* orow = reinterpret_cast<float4*>(args.out_f32 + static_cast<long long>(g.x + b + 1 + i) * args.N + col);
+#pragma unroll
+            for (int j = 0; j < 8; ++j) {
+              const float4 p4 = __ldg(pr + j);
+              orow[j] = make_float4(v[4 * j] + p4.x, v[4 * j + 1] + p4.y, v[4 * j + 2] + p4.z, v[4 * j + 3] + p4.w);
+            }
+          } else if (m < args.M) {
             const int b = m / args.n_patches, i = m - b * args.n_patches;
             if (args.mask != nullptr) {
               const float mk = __ldg(args.mask + m);

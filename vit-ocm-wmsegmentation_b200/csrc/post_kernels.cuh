@@ -356,6 +356,110 @@ tile_threshold_kernel(const float* __restrict__ lowres /*[T][lh][lw]*/, const fl
 }
 
 // ---------------------------------------------------------------------------------------
+// Ragged forms for images of different sizes packed back to back (vitocm_forward_cls_attn_varlen's layout), one block per image:
+//   head_mean_var_kernel       head_mean_kernel with image t's rows [H][N_t] at heads (patch_off[t] + t) and its map at patch_off[t]
+//   tile_threshold_var_kernel  tile_threshold_kernel (without att_in / img_in / aux) for a square image of side S_t = geo[t].x
+//                              and map side geo[t].y, map at geo[t].z, pixels at geo[t].w (x: C x, masks: 3 x)
+// The per-image arithmetic is the uniform kernels' own.
+// ---------------------------------------------------------------------------------------
+__global__ void __launch_bounds__(256)
+head_mean_var_kernel(const float* __restrict__ rows, float* __restrict__ lowres, int heads, const int* __restrict__ patch_off, int mode) {
+  __shared__ float red_mn[8], red_mx[8];
+  const int t = blockIdx.x, p0 = patch_off[t], n = patch_off[t + 1] - p0, N = n + 1;
+  const float* rt = rows + static_cast<long long>(p0 + t) * heads;
+  float* lt = lowres + p0;
+  float mn = INFINITY, mx = -INFINITY;
+  for (int i = threadIdx.x; i < n; i += blockDim.x) {
+    float s = rt[1 + i];
+    for (int h = 1; h < heads; ++h) s = __fadd_rn(s, rt[static_cast<long long>(h) * N + 1 + i]);
+    s = __fdiv_rn(s, static_cast<float>(heads));
+    lt[i] = s;
+    mn = fminf(mn, s);
+    mx = fmaxf(mx, s);
+  }
+  if (mode == 0) return;
+  for (int o = 16; o > 0; o >>= 1) {
+    mn = fminf(mn, __shfl_xor_sync(0xffffffffu, mn, o));
+    mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, o));
+  }
+  if ((threadIdx.x & 31) == 0) { red_mn[threadIdx.x >> 5] = mn; red_mx[threadIdx.x >> 5] = mx; }
+  __syncthreads();
+  mn = red_mn[0]; mx = red_mx[0];
+  for (int w = 1; w < (blockDim.x >> 5); ++w) { mn = fminf(mn, red_mn[w]); mx = fmaxf(mx, red_mx[w]); }
+  const float range = __fsub_rn(mx, mn);
+  for (int i = threadIdx.x; i < n; i += blockDim.x)
+    lt[i] = __fmul_rn(__fdiv_rn(__fsub_rn(lt[i], mn), range), 255.0f);
+}
+
+__global__ void __launch_bounds__(512)
+tile_threshold_var_kernel(const float* __restrict__ lowres, const float* __restrict__ x, int C, const int4* __restrict__ geo,
+                          uint8_t* __restrict__ masks, int* __restrict__ thresholds, float* __restrict__ att_out) {
+  __shared__ float red_mn[16], red_mx[16];
+  __shared__ unsigned int hist[3][256];
+  __shared__ unsigned long long hist64[256];
+  __shared__ int thr[3];
+  const int t = blockIdx.x;
+  const int4 g = geo[t];
+  const int S = g.x, lh = g.y, lw = g.y;
+  const float* lo = lowres + g.z;
+  const long long plane = static_cast<long long>(S) * S;
+  const float* xt = x + static_cast<long long>(g.w) * C;
+  const double scale = static_cast<double>(lw) / static_cast<double>(S);
+  const int npx = S * S;
+  float mn = INFINITY, mx = -INFINITY;
+  for (int i = threadIdx.x; i < npx; i += blockDim.x) {
+    const float a = bilinear_up(lo, lh, lw, i / S, i % S, scale);
+    if (att_out != nullptr) att_out[g.w + i] = a;
+    mn = fminf(mn, a);
+    mx = fmaxf(mx, a);
+  }
+  for (int o = 16; o > 0; o >>= 1) {
+    mn = fminf(mn, __shfl_xor_sync(0xffffffffu, mn, o));
+    mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, o));
+  }
+  if ((threadIdx.x & 31) == 0) { red_mn[threadIdx.x >> 5] = mn; red_mx[threadIdx.x >> 5] = mx; }
+  for (int i = threadIdx.x; i < 3 * 256; i += blockDim.x) (&hist[0][0])[i] = 0u;
+  __syncthreads();
+  mn = red_mn[0]; mx = red_mx[0];
+  for (int w = 1; w < (blockDim.x >> 5); ++w) { mn = fminf(mn, red_mn[w]); mx = fmaxf(mx, red_mx[w]); }
+  const bool flat = (mx == mn);
+  const float range = __fsub_rn(mx, mn);
+  auto classify = [&](int i, int& img, int& att_u8, int& res) {
+    const float a = bilinear_up(lo, lh, lw, i / S, i % S, scale);
+    const float an = flat ? a : __fdiv_rn(__fsub_rn(a, mn), range);
+    att_u8 = static_cast<int>(static_cast<uint8_t>(static_cast<int>(__fmul_rn(an, 255.0f))));
+    img = gray_u8_from_x(xt, C, plane, i);
+    const double r = __dadd_rn(__dmul_rn(static_cast<double>(img) / 2.0, 1.0 - 0.4), __dmul_rn(static_cast<double>(att_u8) / 2.0, 0.4));
+    res = static_cast<int>(r);
+  };
+  for (int i = threadIdx.x; i < npx; i += blockDim.x) {
+    int img, au, res;
+    classify(i, img, au, res);
+    atomicAdd(&hist[0][res], 1u);
+    atomicAdd(&hist[1][img], 1u);
+    atomicAdd(&hist[2][au], 1u);
+  }
+  __syncthreads();
+  for (int k = 0; k < 3; ++k) {
+    for (int i = threadIdx.x; i < 256; i += blockDim.x) hist64[i] = hist[k][i];
+    __syncthreads();
+    if (threadIdx.x == 0) {
+      thr[k] = otsu_from_hist(hist64);
+      thresholds[t * 3 + k] = thr[k];
+    }
+    __syncthreads();
+  }
+  uint8_t* m0 = masks + static_cast<long long>(g.w) * 3;
+  for (int i = threadIdx.x; i < npx; i += blockDim.x) {
+    int img, au, res;
+    classify(i, img, au, res);
+    m0[i] = res > thr[0] ? 255 : 0;
+    m0[plane + i] = img > thr[1] ? 255 : 0;
+    m0[2 * plane + i] = au > thr[2] ? 255 : 0;
+  }
+}
+
+// ---------------------------------------------------------------------------------------
 // Sliding-window geometry shared by the mosaic kernels.  ny x nx tiles of size W at stride S
 // (origins range(0, size - 2S, S) over the height and over the width), row-major: tile t = i * nx + j has origin (i S, j S);
 // stitched extent Ey x Ex = ((ny-1) S + W) x ((nx-1) S + W); step = W - S.  A square mosaic is ny = nx = n.

@@ -31,6 +31,16 @@ __global__ void cls_rows_kernel(const float* __restrict__ cls_token, const float
   const int b = i / D, d = i - b * D;
   X[static_cast<long long>(b) * image_stride + d] = cls_token[d] + pos[d];
 }
+// the same for images of different sizes packed back to back (vimg as GemmArgs::vimg): image b's CLS row is token row vimg[b].x + b,
+// its position row pos[vimg[b].z]
+__global__ void cls_rows_var_kernel(const float* __restrict__ cls_token, const float* __restrict__ pos, const int4* __restrict__ vimg,
+                                    float* __restrict__ X, int B, int D) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= B * D) return;
+  const int b = i / D, d = i - b * D;
+  const int4 g = vimg[b];
+  X[static_cast<long long>(g.x + b) * D + d] = cls_token[d] + pos[static_cast<long long>(g.z) * D + d];
+}
 
 // ---------------------------------------------------------------------------------------
 // LayerNorm over the last dim of the fp32 token stream, one warp per row, float4 loads.
@@ -117,8 +127,11 @@ layernorm_kernel(const float* __restrict__ x, const float* __restrict__ gamma, c
 //   q_h = Wq[h*DH:(h+1)*DH, :] . xn + bq              (fp32 weights, fp32 math)
 //   out[b, h, j] = softmax_j( scale * q_h . K[b, j, h*DH:(h+1)*DH] )   for j in [0, N)
 // K comes from the (split-precision) K-projection GEMM as fp32 [B*N, D].  DH = head_dim (64 or 128).
+// VAR: the CLS query of images of different sizes packed back to back; `queries` then carries vimg (int4 [B + 1], as GemmArgs::vimg):
+// image b has N_b = vimg[b + 1].x - vimg[b].x + 1 tokens from token row vimg[b].x + b on, its rows are out[heads (vimg[b].x + b) ...]
+// as [H][N_b], and N is the largest N_b (it sizes the shared memory).
 // ---------------------------------------------------------------------------------------
-template <int DH>
+template <int DH, bool VAR = false>
 __global__ void __launch_bounds__(256)
 cls_attn_row_kernel(const float* __restrict__ X, const float* __restrict__ ln_w, const float* __restrict__ ln_b, float eps,
                     const float* __restrict__ Wq /*[D][D] rows = q outputs*/, const float* __restrict__ bq,
@@ -132,8 +145,11 @@ cls_attn_row_kernel(const float* __restrict__ X, const float* __restrict__ ln_w,
   const int h = blockIdx.x, b = blockIdx.y;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, nwarps = blockDim.x >> 5;
   const int qi = blockIdx.z;
-  const int token = queries != nullptr ? queries[qi] : 0;    // 0 = the CLS token (SSS/utils.py:232, query = 0)
-  const float* xr = X + (static_cast<long long>(b) * N + token) * D;
+  const int4* vimg = reinterpret_cast<const int4*>(queries);
+  const long long vrow0 = VAR ? static_cast<long long>(vimg[b].x) + b : 0;   // VAR: the image's first token row and its tokens
+  const int vn = VAR ? vimg[b + 1].x - vimg[b].x + 1 : 0;
+  const int token = VAR ? 0 : (queries != nullptr ? queries[qi] : 0);    // 0 = the CLS token (SSS/utils.py:232, query = 0)
+  const float* xr = X + ((VAR ? vrow0 : static_cast<long long>(b) * N) + token) * D;
 
   // LayerNorm of the CLS row (block-wide two-pass)
   float s = 0.f;
@@ -173,16 +189,16 @@ cls_attn_row_kernel(const float* __restrict__ X, const float* __restrict__ ln_w,
   float lmax = -INFINITY;
   if constexpr (DH == 64) {
     const float q0 = qv[2 * lane], q1 = qv[2 * lane + 1];
-    for (int j = warp; j < N; j += nwarps) {
-      const float2 kk = *reinterpret_cast<const float2*>(Kmat + (static_cast<long long>(b) * N + j) * D + h * 64 + 2 * lane);
+    for (int j = warp; j < (VAR ? vn : N); j += nwarps) {
+      const float2 kk = *reinterpret_cast<const float2*>(Kmat + ((VAR ? vrow0 : static_cast<long long>(b) * N) + j) * D + h * 64 + 2 * lane);
       float acc = warp_sum(fmaf(q0, kk.x, q1 * kk.y)) * scale;
       if (lane == 0) logits[j] = acc;
       lmax = fmaxf(lmax, acc);
     }
   } else {
     const float4 qq = reinterpret_cast<const float4*>(qv)[lane];
-    for (int j = warp; j < N; j += nwarps) {
-      const float4 kk = *reinterpret_cast<const float4*>(Kmat + (static_cast<long long>(b) * N + j) * D + h * DH + 4 * lane);
+    for (int j = warp; j < (VAR ? vn : N); j += nwarps) {
+      const float4 kk = *reinterpret_cast<const float4*>(Kmat + ((VAR ? vrow0 : static_cast<long long>(b) * N) + j) * D + h * DH + 4 * lane);
       float acc = warp_sum(fmaf(qq.x, kk.x, fmaf(qq.y, kk.y, fmaf(qq.z, kk.z, qq.w * kk.w)))) * scale;
       if (lane == 0) logits[j] = acc;
       lmax = fmaxf(lmax, acc);
@@ -194,7 +210,7 @@ cls_attn_row_kernel(const float* __restrict__ X, const float* __restrict__ ln_w,
   for (int w = 0; w < nwarps; ++w) gmax = fmaxf(gmax, red[w]);
   __syncthreads();
   float lsum = 0.f;
-  for (int j = tid; j < N; j += blockDim.x) {
+  for (int j = tid; j < (VAR ? vn : N); j += blockDim.x) {
     const float e = expf(logits[j] - gmax);
     logits[j] = e;
     lsum += e;
@@ -205,8 +221,8 @@ cls_attn_row_kernel(const float* __restrict__ X, const float* __restrict__ ln_w,
   float gsum = 0.f;
   for (int w = 0; w < nwarps; ++w) gsum += red[w];
   const float inv = 1.0f / gsum;
-  float* o = out + ((static_cast<long long>(b) * heads + h) * nq + qi) * N;
-  for (int j = tid; j < N; j += blockDim.x) o[j] = logits[j] * inv;
+  float* o = VAR ? out + vrow0 * heads + static_cast<long long>(h) * vn : out + ((static_cast<long long>(b) * heads + h) * nq + qi) * N;
+  for (int j = tid; j < (VAR ? vn : N); j += blockDim.x) o[j] = logits[j] * inv;
 }
 
 // ---------------------------------------------------------------------------------------

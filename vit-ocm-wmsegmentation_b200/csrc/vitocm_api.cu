@@ -192,6 +192,11 @@ struct vitocm_engine {
   // training workspaces (by the address of their branch-scale slab) whose last forward ran with stochastic-depth scales: the
   // backward on the same workspace scales its residual branches with that forward's copy (TrainWs::bscale)
   std::set<const void*> dp_ws;
+  // pinned staging of the varlen work-item tables (a cudaMemcpyAsync out of pageable memory would first wait for the stream): two
+  // slots used by calls in turn; a slot is rewritten once the last copy that read it has run (its event)
+  struct PinnedTab { int4* p = nullptr; size_t cap = 0; cudaEvent_t sent = nullptr; bool pending = false; };
+  PinnedTab pin[2];
+  int pin_next = 0;
   ~vitocm_engine() {
     for (cudaEvent_t ev : bwd_events) if (ev) cudaEventDestroy(ev);
     for (auto& kv : master) delete kv.second;
@@ -200,6 +205,10 @@ struct vitocm_engine {
       if (ev_join[i]) cudaEventDestroy(ev_join[i]);
     }
     if (ev_fork) cudaEventDestroy(ev_fork);
+    for (PinnedTab& t : pin) {
+      if (t.sent) cudaEventDestroy(t.sent);
+      if (t.p) cudaFreeHost(t.p);
+    }
   }
   const float* w(const std::string& name) const {
     auto it = master.find(name);
@@ -769,6 +778,85 @@ int run_attention(const vitocm_engine* e, const void* qkv, long long ld, int B, 
   return 0;
 }
 
+// Images of different sizes packed back to back ([sum N_i] token rows, no pad rows): work items from a table (AttnArgs::vitems) in
+// device memory.  Every image's rows take the route run_attention takes for that image alone (B = 1, default knobs): full tiles of
+// 16-bit head_dim-64 engines and their packed tails (<= 64 rows, <= 16 full tiles) through the four-pipeline kernel, everything else
+// through the two-CTA kernel.  A packed tail item only holds heads of one image (the tail length is the image's).
+struct VarAttn {
+  const int4* quad;   // items of attn_fwd_quad_kernel
+  int n_quad;
+  const int4* cta;    // items of attn_fwd_tcgen05_kernel
+  int n_cta;
+};
+
+// host: the work items of images with token counts n[0..B) starting at token rows row0[0..B)
+void varlen_attn_items(const vitocm_engine* e, const std::vector<int>& n, const std::vector<int>& row0, std::vector<int4>& quad,
+                       std::vector<int4>& cta) {
+  const int H = e->cfg.num_heads;
+  const bool quad_ok = e->cfg.embed_dim == 64 * H && !e->split;
+  for (size_t i = 0; i < n.size(); ++i) {
+    const int N = n[i], nfull = N / ATT_BQ, tail = N % ATT_BQ;
+    const int pack = (tail == 0 || tail > 64 || nfull > 16) ? 1 : (tail > 32 ? 2 : 4);   // as run_attention
+    const bool q = quad_ok && nfull >= 1;
+    std::vector<int4>& full = q ? quad : cta;
+    for (int h = 0; h < H; ++h)
+      for (int t = 0; t < nfull; ++t) full.push_back(make_int4(row0[i], N, t, h | (1 << 16)));
+    if (tail == 0) continue;
+    const int ns = pack == 1 ? 1 : (q ? 2 : pack);   // the four-pipeline kernel packs two tails per tile
+    std::vector<int4>& tl = (q && pack > 1) ? quad : cta;
+    for (int h = 0; h < H; h += ns) tl.push_back(make_int4(row0[i], N, nfull, h | (ns << 16)));
+  }
+}
+
+int run_attention_var(const vitocm_engine* e, const void* qkv, long long ld, int M, const VarAttn& v, void* ctx, long long ldo, cudaStream_t st) {
+  const int D = e->cfg.embed_dim, H = e->cfg.num_heads;
+  const bool hd128 = D == 128 * H;
+  ProfScope prof(PC_ATTN, st);
+  CUtensorMap tq, tq32;
+  TRY(make_tmap_bf16(&tq, qkv, M, 3LL * D * e->parts, ld, 128));
+  TRY(make_tmap_bf16(&tq32, qkv, M, 3LL * D * e->parts, ld, 32));
+  AttnArgs a{};
+  a.n_tokens = 0; a.embed_dim = D; a.lo_col_off = 3 * D; a.heads = H;
+  a.scale_log2 = e->cfg.qk_scale * 1.44269504088896340736f;
+  a.out = reinterpret_cast<__nv_bfloat16*>(ctx); a.ldo = ldo; a.out_lo_off = D;
+  { static const int tm = [] { const char* v = getenv("VITOCM_ATTN_TRACK_MAX"); return v ? atoi(v) : 0; }(); a.track_max = tm; }
+  a.ctrl_hoist = 1;
+  if (v.n_quad > 0) {
+    AttnArgs aq = a;
+    aq.vitems = v.quad; aq.n_items = v.n_quad;
+    CUtensorMap tkv;
+    TRY(make_tmap_bf16(&tkv, qkv, M, 3LL * D * e->parts, ld, AQ_BKV));
+    const int ctas = (aq.n_items + AQ_PIPES - 1) / AQ_PIPES;
+    const dim3 qgrid(ctas < e->num_sms ? ctas : e->num_sms);
+    static bool qattr[2] = {false, false};
+    auto kern = e->f16 ? attn_fwd_quad_kernel<true, false, true> : attn_fwd_quad_kernel<false, false, true>;
+    if (!qattr[e->f16]) { CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, AQ_SMEM_BYTES)); qattr[e->f16] = true; }
+    kern<<<qgrid, AQ_THREADS, AQ_SMEM_BYTES, st>>>(tq, tkv, tq32, aq);
+    LAUNCH_CHECK();
+  }
+  if (v.n_cta == 0) return 0;
+  a.vitems = v.cta; a.n_items = v.n_cta;
+  const int resident = e->num_sms * ((e->split || hd128) ? 1 : 2);
+  const dim3 grid(a.n_items > resident ? resident : a.n_items);
+  static bool attr[8] = {false, false, false, false, false, false, false, false};
+  auto launch = [&](auto kern, int smem_bytes, bool& set) -> int {
+    if (!set) { CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes)); set = true; }
+    kern<<<grid, ATT_THREADS, smem_bytes, st>>>(tq, tq32, a);
+    LAUNCH_CHECK();
+    return 0;
+  };
+  if (hd128) {
+    if (e->split) return e->f16 ? launch(attn_fwd_tcgen05_kernel<true, 0u, true, true, 128, true>, AttnCfg<true, 128>::SMEM_BYTES, attr[0])
+                                : launch(attn_fwd_tcgen05_kernel<true, 0u, true, false, 128, true>, AttnCfg<true, 128>::SMEM_BYTES, attr[1]);
+    return e->f16 ? launch(attn_fwd_tcgen05_kernel<false, 0u, true, true, 128, true>, AttnCfg<false, 128>::SMEM_BYTES, attr[2])
+                  : launch(attn_fwd_tcgen05_kernel<false, 0u, true, false, 128, true>, AttnCfg<false, 128>::SMEM_BYTES, attr[3]);
+  }
+  if (e->split) return e->f16 ? launch(attn_fwd_tcgen05_kernel<true, 0u, true, true, 64, true>, AttnCfg<true>::SMEM_BYTES, attr[4])
+                              : launch(attn_fwd_tcgen05_kernel<true, 0u, true, false, 64, true>, AttnCfg<true>::SMEM_BYTES, attr[5]);
+  return e->f16 ? launch(attn_fwd_tcgen05_kernel<false, 0u, true, true, 64, true>, AttnCfg<false>::SMEM_BYTES, attr[6])
+                : launch(attn_fwd_tcgen05_kernel<false, 0u, true, false, 64, true>, AttnCfg<false>::SMEM_BYTES, attr[7]);
+}
+
 int run_layernorm(const float* X, const float* g, const float* b, void* out_bf16, long long ldo, int split, int lo_off,
                   float* out_f32, long long ldf, int M, int D, float eps, cudaStream_t st, float* x_copy = nullptr, int f16 = 0) {
   if (M <= 0) return 0;
@@ -835,6 +923,50 @@ int run_patch_embed(const vitocm_engine* e, const float* x, int B, int H, int W,
   }
 }
 
+// run_patch_embed for images of different sizes packed back to back: x holds image b's [C][H_b][W_b] pixels from C p^2 vimg[b].x on,
+// vimg (device, n_img + 1 entries: GemmArgs::vimg) its geometry, pos the packed position tables (pos_rows rows).  M = patches in all.
+int run_patch_embed_var(const vitocm_engine* e, const float* x, bool gray, int n_img, const int4* vimg, int M, const float* pos, int pos_rows,
+                        float* X, cudaStream_t st) {
+  const int p = e->cfg.patch_size, C = gray ? 1 : e->cfg.in_chans, D = e->cfg.embed_dim;
+  if (gray && e->patch_w_gray.p == nullptr) return fail(VITOCM_ERR_STATE, "gray fast path needs in_chans > 1");
+  const int K = C * p * p;
+  if (p % 8 != 0 || K % GEMM_BK != 0) return fail(VITOCM_ERR_INVALID, "patch embedding needs patch %% 8 == 0 and C*p*p %% 64 == 0 (patch %d, chans %d)", p, C);
+  if ((reinterpret_cast<uintptr_t>(x) & 15) != 0 || (reinterpret_cast<uintptr_t>(pos) & 15) != 0)
+    return fail(VITOCM_ERR_INVALID, "patch embedding inputs must be 16-byte aligned");
+  ProfScope prof(PC_PATCH, st);
+  cls_rows_var_kernel<<<(n_img * D + 255) / 256, 256, 0, st>>>(e->w("cls_token"), pos, vimg, X, n_img, D);
+  LAUNCH_CHECK();
+  const int bn = (D % 192 == 0) ? 192 : (D % 128 == 0 ? 128 : 64);
+  CUtensorMap tb;
+  TRY(make_tmap_bf16(&tb, gray ? e->patch_w_gray.p : e->patch_w.p, D, 2LL * K, 2LL * K, bn));
+  GemmArgs a{};
+  a.M = M; a.N = D; a.kblocks = K / GEMM_BK; a.nterms = 3; a.lo_k = K; a.a_lo_mask = 4; a.b_lo_mask = 2; a.f16 = e->f16;
+  a.bias = e->w("patch_embed.proj.bias");
+  a.img = x; a.patch = p; a.pos = pos; a.out_f32 = X; a.vimg = vimg; a.n_img = n_img;
+  static const int patch_tma = [] { const char* v = getenv("VITOCM_PATCH_TMA"); return v == nullptr ? 1 : atoi(v); }();
+  CUtensorMap tx = tb, tp = tb;
+  if (patch_tma && D % 32 == 0 && (reinterpret_cast<uintptr_t>(X) & 15) == 0) {
+    TRY(make_tmap(&tx, X, true, D, static_cast<long long>(M) + n_img, D, 32, 32, CU_TENSOR_MAP_SWIZZLE_128B));
+    TRY(make_tmap(&tp, pos, true, D, pos_rows, D, 32, 32, CU_TENSOR_MAP_SWIZZLE_128B));
+    a.patch_tma = 1;
+  }
+  static bool attr[3] = {false, false, false};
+  auto launch = [&](auto kern, int smem, int threads) -> int {
+    bool& set = attr[bn == 192 ? 0 : (bn == 128 ? 1 : 2)];
+    if (!set) { CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)); set = true; }
+    const int tiles = ((a.M + GEMM_BM - 1) / GEMM_BM) * (a.N / bn);
+    const int grid = tiles < e->num_sms ? tiles : e->num_sms;
+    kern<<<grid, threads, smem, st>>>(tb, tb, tx, tp, a);
+    LAUNCH_CHECK();
+    return 0;
+  };
+  switch (bn) {
+    case 192: return launch(gemm_bf16_tcgen05_kernel<192, EPI_PATCH_F32, true, false, 1, false, true>, GemmCfg<192, EPI_PATCH_F32>::SMEM_BYTES, gemm_threads(192, EPI_PATCH_F32));
+    case 128: return launch(gemm_bf16_tcgen05_kernel<128, EPI_PATCH_F32, true, false, 1, false, true>, GemmCfg<128, EPI_PATCH_F32>::SMEM_BYTES, gemm_threads(128, EPI_PATCH_F32));
+    default: return launch(gemm_bf16_tcgen05_kernel<64, EPI_PATCH_F32, true, false, 1, false, true>, GemmCfg<64, EPI_PATCH_F32>::SMEM_BYTES, gemm_threads(64, EPI_PATCH_F32));
+  }
+}
+
 // workspace carve-up for a chunk of `tiles` images
 struct Workspace {
   float* X;            // [M][D] fp32 token stream
@@ -870,7 +1002,8 @@ Workspace carve(const vitocm_engine* e, void* base, int tiles, int N) {
 // NEXT block, whose QKV projection this block's tail kernel computes when it can (*qkv_done).
 int block_forward(const vitocm_engine* e, int l, const Workspace& ws, int B, int N, cudaStream_t st, bool xn_ready = false,
                   const float* next_ln_w = nullptr, const float* next_ln_b = nullptr, bool* xn_done = nullptr, bool qkv_ready = false,
-                  const LayerW* next_qkv = nullptr, bool* qkv_done = nullptr) {
+                  const LayerW* next_qkv = nullptr, bool* qkv_done = nullptr, const VarAttn* var = nullptr) {
+  // var: images of different sizes packed back to back (B = 1, N = their tokens in all; run_attention_var)
   const LayerW& L = e->layers[l];
   const int D = e->cfg.embed_dim, Hd = e->cfg.mlp_hidden, P = e->parts, S = e->split;
   const int M = B * N;
@@ -881,7 +1014,8 @@ int block_forward(const vitocm_engine* e, int l, const Workspace& ws, int B, int
     TRY(run_gemm(e, ws.XN, 2LL * D, L.wqkv.p, static_cast<long long>(D) * P, M, 3 * D, D, S, EPI_BIAS_BF16, L.bqkv, ws.QKV,
                  3LL * D * P, S, 3 * D, st, PC_GEMM_QKV));
   }
-  TRY(run_attention(e, ws.QKV, 3LL * D * P, B, N, ws.CTX, static_cast<long long>(D) * P, st));
+  if (var != nullptr) TRY(run_attention_var(e, ws.QKV, 3LL * D * P, M, *var, ws.CTX, static_cast<long long>(D) * P, st));
+  else TRY(run_attention(e, ws.QKV, 3LL * D * P, B, N, ws.CTX, static_cast<long long>(D) * P, st));
   // MLP of an act-split block (vitocm_set_layer_mode 1): norm2's output and the hidden activations are kept as (hi, lo) pairs and
   // fc1 / fc2 contract both halves against the single-precision weights (two MMAs per product) -- the rounding of these two
   // activations is where most of the CLS-row error of a 16-bit forward comes from (profiles/r02_precision_sim.txt)
@@ -939,6 +1073,46 @@ int block_forward(const vitocm_engine* e, int l, const Workspace& ws, int B, int
   } else if (xn_done != nullptr) {
     *xn_done = true;
   }
+  return 0;
+}
+
+// Work-item capacity of a varlen chunk of at most `tokens` rows: images hold >= 2 tokens each, and an image of N tokens has at most
+// heads x ceil(N / 128) attention items.  The table region of the workspace holds vimg (images + 1 entries) and both item lists.
+long long varlen_table_entries(const vitocm_engine* e, long long tokens) {
+  const long long imgs = tokens / 2 + 1;
+  return imgs + 1 + static_cast<long long>(e->cfg.num_heads) * (tokens / ATT_BQ + imgs);
+}
+size_t varlen_ws_bytes(const vitocm_engine* e, long long tokens) {
+  return carve(e, nullptr, 1, static_cast<int>(tokens)).total + align_up(static_cast<size_t>(varlen_table_entries(e, tokens)) * sizeof(int4), 1024);
+}
+
+// The tables of one varlen call into a pinned slot of the engine (see vitocm_engine::pin); copy_table sends a part of them to the device
+// on `st` and marks the slot busy until that copy has run.
+int stage_tables(vitocm_engine* e, const std::vector<int4>& tab, int& slot) {
+  slot = e->pin_next;
+  e->pin_next ^= 1;
+  vitocm_engine::PinnedTab& t = e->pin[slot];
+  if (t.sent == nullptr) CUDA_TRY(cudaEventCreateWithFlags(&t.sent, cudaEventDisableTiming));
+  if (t.pending) {   // copies of the call before the previous one may still be queued
+    CUDA_TRY(cudaEventSynchronize(t.sent));
+    t.pending = false;
+  }
+  if (t.cap < tab.size()) {
+    if (t.p != nullptr) CUDA_TRY(cudaFreeHost(t.p));
+    t.p = nullptr;
+    t.cap = 0;
+    const size_t cap = tab.size() < 4096 ? 4096 : tab.size() + tab.size() / 2;
+    CUDA_TRY(cudaHostAlloc(reinterpret_cast<void**>(&t.p), cap * sizeof(int4), cudaHostAllocDefault));
+    t.cap = cap;
+  }
+  memcpy(t.p, tab.data(), tab.size() * sizeof(int4));
+  return 0;
+}
+int copy_table(vitocm_engine* e, int slot, int4* dst, size_t first, size_t count, cudaStream_t st) {
+  vitocm_engine::PinnedTab& t = e->pin[slot];
+  CUDA_TRY(cudaMemcpyAsync(dst, t.p + first, count * sizeof(int4), cudaMemcpyHostToDevice, st));
+  CUDA_TRY(cudaEventRecord(t.sent, st));
+  t.pending = true;
   return 0;
 }
 
@@ -1251,6 +1425,157 @@ int vitocm_forward_cls_attn(vitocm_engine* e, const float* x, int B, int H, int 
   return forward_rows(e, x, B, H, W, pos, nullptr, 1, out_rows, nullptr, ws, ws_bytes, chunk_tiles, stream);
 }
 
+size_t vitocm_varlen_workspace_bytes(const vitocm_engine* e, int64_t chunk_tokens) {
+  if (e == nullptr) return 0;
+  if (chunk_tokens <= 0) chunk_tokens = VITOCM_VARLEN_CHUNK_TOKENS;
+  if (chunk_tokens > INT_MAX / 2) return 0;
+  return varlen_ws_bytes(e, chunk_tokens) + 1024;
+}
+
+int vitocm_forward_cls_attn_varlen(vitocm_engine* e, const float* x, int B, int C, const int* hw, const float* pos, const int* pos_off,
+                                   float* out_rows, void* ws, size_t ws_bytes, int64_t chunk_tokens, void* stream) {
+  TRY(check_engine(e));
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const int p = e->cfg.patch_size, D = e->cfg.embed_dim, heads = e->cfg.num_heads, dh = D / heads;
+  if (B < 1) return fail(VITOCM_ERR_INVALID, "forward_cls_attn_varlen: B must be >= 1 (got %d)", B);
+  if (x == nullptr || hw == nullptr || pos == nullptr || pos_off == nullptr || out_rows == nullptr)
+    return fail(VITOCM_ERR_INVALID, "forward_cls_attn_varlen: null argument");
+  if (C != e->cfg.in_chans && C != 1) return fail(VITOCM_ERR_INVALID, "forward_cls_attn_varlen: C must be in_chans (%d) or 1 (gray), got %d", e->cfg.in_chans, C);
+  const bool gray = C == 1 && e->cfg.in_chans > 1;
+  if (chunk_tokens <= 0) chunk_tokens = VITOCM_VARLEN_CHUNK_TOKENS;
+  // token counts, the largest image, the packed position tables' extent
+  std::vector<int> n(B);
+  int n_max = 0;
+  long long pos_rows = 0;
+  for (int i = 0; i < B; ++i) {
+    const int H = hw[2 * i], W = hw[2 * i + 1];
+    if (H < p || W < p || H % p || W % p)
+      return fail(VITOCM_ERR_INVALID, "forward_cls_attn_varlen: image %d is %dx%d, not a positive multiple of patch %d", i, H, W, p);
+    const long long Ni = static_cast<long long>(H / p) * (W / p) + 1;
+    if (Ni > INT_MAX / 4) return fail(VITOCM_ERR_INVALID, "forward_cls_attn_varlen: image %d too large", i);
+    if (pos_off[i] < 0) return fail(VITOCM_ERR_INVALID, "forward_cls_attn_varlen: pos_off[%d] = %d is negative", i, pos_off[i]);
+    n[i] = static_cast<int>(Ni);
+    if (n[i] > n_max) n_max = n[i];
+    if (pos_off[i] + Ni > pos_rows) pos_rows = pos_off[i] + Ni;
+  }
+  const size_t cls_smem = static_cast<size_t>(D + dh + n_max + 32) * sizeof(float);
+  if (cls_smem > 227 * 1024)
+    return fail(VITOCM_ERR_INVALID, "forward_cls_attn_varlen: an image of %d tokens exceeds the CLS-row kernel's shared memory", n_max);
+  // chunks: images in order, a chunk closed before the next image would push it past chunk_tokens (an image above the budget runs alone)
+  std::vector<int> starts{0};
+  long long acc = 0, cap = 0;
+  for (int i = 0; i < B; ++i) {
+    if (acc > 0 && acc + n[i] > chunk_tokens) { if (acc > cap) cap = acc; starts.push_back(i); acc = 0; }
+    acc += n[i];
+  }
+  if (acc > cap) cap = acc;
+  starts.push_back(B);
+  if (cap > INT_MAX / 2) return fail(VITOCM_ERR_INVALID, "forward_cls_attn_varlen: chunk of %lld tokens too large", cap);
+  uint8_t* base = reinterpret_cast<uint8_t*>(align_up(reinterpret_cast<uintptr_t>(ws), 1024));
+  const size_t need = varlen_ws_bytes(e, cap);
+  if (ws == nullptr || need > ws_avail(ws, base, ws_bytes))
+    return fail(VITOCM_ERR_WORKSPACE, "workspace too small: need %zu, have %zu", need + 1024, ws_bytes);
+  const Workspace wsp = carve(e, base, 1, static_cast<int>(cap));
+  int4* table = reinterpret_cast<int4*>(base + wsp.total);
+  const LayerW& last = e->layers[e->cfg.depth - 1];
+  static size_t cls_smem_set[2] = {0, 0};
+  if (cls_smem > 48 * 1024 && cls_smem > cls_smem_set[dh == 128]) {
+    if (dh == 128) CUDA_TRY(cudaFuncSetAttribute(cls_attn_row_kernel<128, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(cls_smem)));
+    else CUDA_TRY(cudaFuncSetAttribute(cls_attn_row_kernel<64, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(cls_smem)));
+    cls_smem_set[dh == 128] = cls_smem;
+  }
+  const long long pp = static_cast<long long>(p) * p;
+  // every chunk's tables (vimg, then the attention items), back to back, staged once; chunk c's part is copied in front of its kernels
+  struct ChunkTab { size_t first, count, n_q, n_c; int patches, M, n_max; };
+  std::vector<ChunkTab> ct;
+  std::vector<int4> tab, quad, cta;
+  std::vector<int> cn, row0;
+  for (size_t c = 0; c + 1 < starts.size(); ++c) {
+    const int i0 = starts[c], i1 = starts[c + 1];
+    quad.clear(); cta.clear(); cn.clear(); row0.clear();
+    ChunkTab t{tab.size(), 0, 0, 0, 0, 0, 0};
+    for (int i = i0; i < i1; ++i) {
+      tab.push_back(make_int4(t.patches, hw[2 * i + 1] / p, pos_off[i], 0));
+      cn.push_back(n[i]);
+      row0.push_back(t.M);
+      t.patches += n[i] - 1;
+      t.M += n[i];
+      if (n[i] > t.n_max) t.n_max = n[i];
+    }
+    tab.push_back(make_int4(t.patches, 0, 0, 0));
+    varlen_attn_items(e, cn, row0, quad, cta);
+    t.n_q = quad.size();
+    t.n_c = cta.size();
+    tab.insert(tab.end(), quad.begin(), quad.end());
+    tab.insert(tab.end(), cta.begin(), cta.end());
+    t.count = tab.size() - t.first;
+    if (static_cast<long long>(t.count) > varlen_table_entries(e, cap))
+      return fail(VITOCM_ERR_WORKSPACE, "forward_cls_attn_varlen: %zu table entries exceed the workspace's %lld", t.count, varlen_table_entries(e, cap));
+    ct.push_back(t);
+  }
+  int slot = 0;
+  TRY(stage_tables(e, tab, slot));
+  long long patch0 = 0;   // patches before the chunk
+  for (size_t c = 0; c + 1 < starts.size(); ++c) {
+    const int i0 = starts[c], ni = starts[c + 1] - i0;
+    const ChunkTab& t = ct[c];
+    const int patches = t.patches, M = t.M;
+    const size_t n_q = t.n_q, n_c = t.n_c;
+    TRY(copy_table(e, slot, table, t.first, t.count, st));
+    const int4* vimg = table;
+    const VarAttn var{table + ni + 1, static_cast<int>(n_q), table + ni + 1 + n_q, static_cast<int>(n_c)};
+    TRY(run_patch_embed_var(e, x + patch0 * pp * C, gray, ni, vimg, patches, pos, static_cast<int>(pos_rows), wsp.X, st));
+    bool xn_ready = false, qkv_ready = false;
+    for (int l = 0; l + 1 < e->cfg.depth; ++l) {
+      const bool chain = l + 2 < e->cfg.depth;
+      bool done = false, qdone = false;
+      TRY(block_forward(e, l, wsp, 1, M, st, xn_ready, chain ? e->layers[l + 1].ln1w : nullptr, chain ? e->layers[l + 1].ln1b : nullptr,
+                        &done, qkv_ready, chain ? &e->layers[l + 1] : nullptr, &qdone, &var));
+      xn_ready = done;
+      qkv_ready = qdone;
+    }
+    float* KF = reinterpret_cast<float*>(wsp.HID);
+    TRY(run_layernorm(wsp.X, last.ln1w, last.ln1b, wsp.XN, 2LL * D, 1, D, nullptr, 0, M, D, e->cfg.ln_eps, st, nullptr, e->f16));
+    TRY(run_gemm(e, wsp.XN, 2LL * D, last.wk_split.p, 2LL * D, M, D, D, 1, EPI_BIAS_F32, last.bqkv + D, KF, D, 0, 0, st, PC_GEMM_KLAST));
+    ProfScope prof(PC_CLSROW, st);
+    const int n_chunk_max = t.n_max;
+    (dh == 128 ? cls_attn_row_kernel<128, true> : cls_attn_row_kernel<64, true>)<<<dim3(heads, ni), 256, cls_smem, st>>>(
+        wsp.X, last.ln1w, last.ln1b, e->cfg.ln_eps, last.wqkv_f32, last.bqkv, KF, out_rows + (patch0 + i0) * heads, n_chunk_max, D, heads,
+        e->cfg.qk_scale, reinterpret_cast<const int*>(vimg), 1);
+    LAUNCH_CHECK();
+    patch0 += patches;
+  }
+  return 0;
+}
+
+int vitocm_attention_varlen(vitocm_engine* e, const void* qkv, int64_t ld, int B, const int* n_tokens, void* ctx, int64_t ldo, void* ws,
+                            size_t ws_bytes, void* stream) {
+  if (e == nullptr || n_tokens == nullptr) return fail(VITOCM_ERR_INVALID, "null argument");
+  if (B < 1) return fail(VITOCM_ERR_INVALID, "attention_varlen: B must be >= 1 (got %d)", B);
+  std::vector<int> n(B), row0(B);
+  long long M = 0;
+  for (int i = 0; i < B; ++i) {
+    if (n_tokens[i] < 1) return fail(VITOCM_ERR_INVALID, "attention_varlen: image %d has %d tokens", i, n_tokens[i]);
+    n[i] = n_tokens[i];
+    row0[i] = static_cast<int>(M);
+    M += n[i];
+    if (M > INT_MAX) return fail(VITOCM_ERR_INVALID, "attention_varlen: too many tokens");
+  }
+  std::vector<int4> quad, cta;
+  varlen_attn_items(e, n, row0, quad, cta);
+  quad.insert(quad.end(), cta.begin(), cta.end());
+  int4* table = reinterpret_cast<int4*>(align_up(reinterpret_cast<uintptr_t>(ws), 16));
+  const size_t need = quad.size() * sizeof(int4);
+  if (ws == nullptr || need > ws_avail(ws, table, ws_bytes)) return fail(VITOCM_ERR_WORKSPACE, "workspace too small: need %zu, have %zu", need + 16, ws_bytes);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  int slot = 0;
+  TRY(stage_tables(e, quad, slot));
+  TRY(copy_table(e, slot, table, 0, quad.size(), st));
+  const int n_q = static_cast<int>(quad.size() - cta.size());
+  const VarAttn var{table, n_q, table + n_q, static_cast<int>(cta.size())};
+  return run_attention_var(e, qkv, ld, static_cast<int>(M), var, ctx, ldo, st);
+}
+
 int vitocm_forward_query_attn(vitocm_engine* e, const float* x, int B, int H, int W, const float* pos, const int* queries, int nq,
                               float* out_rows, float* k_out, void* ws, size_t ws_bytes, int chunk_tiles, void* stream) {
   if (queries == nullptr || nq < 1) return fail(VITOCM_ERR_INVALID, "forward_query_attn needs a device array of nq >= 1 token indices");
@@ -1454,6 +1779,25 @@ int vitocm_head_mean(const float* rows, float* lowres, int T, int heads, int n_t
   if (T <= 0) return 0;
   ProfScope prof(PC_POST, static_cast<cudaStream_t>(stream));
   head_mean_kernel<<<T, 256, 0, static_cast<cudaStream_t>(stream)>>>(rows, lowres, heads, n_tokens, mode);
+  LAUNCH_CHECK();
+  return 0;
+}
+
+int vitocm_head_mean_varlen(const float* rows, float* lowres, int T, int heads, const int* patch_off, int mode, void* stream) {
+  if (rows == nullptr || lowres == nullptr || patch_off == nullptr || T < 1 || heads < 1 || (mode != 0 && mode != 1))
+    return fail(VITOCM_ERR_INVALID, "head_mean_varlen: bad argument");
+  head_mean_var_kernel<<<T, 256, 0, static_cast<cudaStream_t>(stream)>>>(rows, lowres, heads, patch_off, mode);
+  LAUNCH_CHECK();
+  return 0;
+}
+
+int vitocm_tile_threshold_varlen(const float* lowres, const float* x, int T, int C, const int* geo, uint8_t* masks, int* thresholds,
+                                 float* att_out, void* stream) {
+  if (lowres == nullptr || x == nullptr || geo == nullptr || masks == nullptr || thresholds == nullptr || T < 1 || C < 1)
+    return fail(VITOCM_ERR_INVALID, "tile_threshold_varlen: bad argument");
+  if ((reinterpret_cast<uintptr_t>(geo) & 15) != 0) return fail(VITOCM_ERR_INVALID, "tile_threshold_varlen: geo must be 16-byte aligned");
+  tile_threshold_var_kernel<<<T, 512, 0, static_cast<cudaStream_t>(stream)>>>(lowres, x, C, reinterpret_cast<const int4*>(geo), masks,
+                                                                              thresholds, att_out);
   LAUNCH_CHECK();
   return 0;
 }

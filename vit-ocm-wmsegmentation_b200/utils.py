@@ -144,6 +144,42 @@ def attention_masks(model, x: torch.Tensor, return_attention: bool = False):
     return out
 
 
+@torch.no_grad()
+def attention_masks_varlen(model, images, return_attention: bool = False):
+    """attention_masks for a list of square images of different sizes (the `--crop 1` eval body per image, SSS/eval.py:136-173, whose
+    resize is square, :171), in one forward (VisionTransformer.cls_attention_rows_varlen) and one launch per post-processing step.
+    images: CUDA tensors [C, S_i, S_i].  Returns dict(masks = list of [3, S_i, S_i] u8, thresholds [B, 3] int32, lowres = list of
+    [h_i, w_i], cls_rows = list of [heads, N_i] [, attention = list of [S_i, S_i]]), each entry equal to attention_masks(x_i[None])'s."""
+    for i, im in enumerate(images):
+        if im.dim() != 3 or im.shape[1] != im.shape[2]:
+            raise ValueError(f"attention_masks_varlen expects square [C, S, S] images (image {i} is {tuple(im.shape)})")
+    packed, plan = model._cls_rows_varlen_packed(images)
+    heads = model.num_heads
+    rows = [packed[heads * t0:heads * (t0 + n)].view(heads, n) for t0, n in zip(plan["row0"], plan["n"])]
+    p = model.patch_embed.patch_size
+    B, dev = len(images), images[0].device
+    sides = [int(im.shape[1]) for im in images]
+    npatch = [(s // p) ** 2 for s in sides]
+    poff = torch.tensor([0] + npatch, dtype=torch.int64).cumsum(0)
+    pix = torch.tensor([0] + [s * s for s in sides], dtype=torch.int64).cumsum(0)
+    low = torch.empty(int(poff[-1]), dtype=torch.float32, device=dev)
+    lib = _lib.load_library()
+    poff_d = poff.to(torch.int32).to(dev)
+    check(lib.vitocm_head_mean_varlen(ptr(packed), ptr(low), B, heads, ptr(poff_d), 0, cur_stream()))
+    geo = torch.tensor([[s, s // p, int(poff[i]), int(pix[i])] for i, s in enumerate(sides)], dtype=torch.int32).to(dev)
+    masks = torch.empty(3 * int(pix[-1]), dtype=torch.uint8, device=dev)
+    thr = torch.empty(B, 3, dtype=torch.int32, device=dev)
+    att = torch.empty(int(pix[-1]), dtype=torch.float32, device=dev) if return_attention else None
+    C = images[0].shape[0]
+    xx = torch.cat([im.detach().to(torch.float32).reshape(-1) for im in images])
+    check(lib.vitocm_tile_threshold_varlen(ptr(low), ptr(xx), B, C, ptr(geo), ptr(masks), ptr(thr), ptr(att), cur_stream()))
+    out = dict(masks=[masks[3 * int(pix[i]):3 * int(pix[i + 1])].view(3, s, s) for i, s in enumerate(sides)], thresholds=thr,
+               lowres=[low[int(poff[i]):int(poff[i + 1])].view(s // p, s // p) for i, s in enumerate(sides)], cls_rows=rows)
+    if return_attention:
+        out["attention"] = [att[int(pix[i]):int(pix[i + 1])].view(s, s) for i, s in enumerate(sides)]
+    return out
+
+
 def concat_crops_overlap(crops, stride):
     """SSS/utils.py:319-347: n x n crops overlapping by 2*stride; overlaps are `a // 2 + b // 2` (floor halves), along x
     inside each strip and then along y, the last strip being appended unblended.  float crops accumulate in float32,

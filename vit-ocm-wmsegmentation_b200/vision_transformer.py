@@ -50,6 +50,32 @@ def parse_precision(spec: str, depth: int):
     return base, modes
 
 
+VARLEN_CHUNK_TOKENS = 401920   # include/vitocm.h VITOCM_VARLEN_CHUNK_TOKENS: 512 images of 224^2 at patch 8
+
+
+def varlen_plan(hw, patch: int, chunk_tokens: int = VARLEN_CHUNK_TOKENS) -> dict:
+    """The packing of vitocm_forward_cls_attn_varlen for images of sizes hw = [(H_i, W_i)]: n = token counts N_i, row0 = first
+    token row of each image in the packed stream (its CLS rows start at heads * row0), tokens = all rows, starts = first image of
+    every chunk (images in order, a chunk closed before the next image would push it past chunk_tokens; an image above the budget
+    runs alone), cap = the workspace's row budget: the tokens of the largest chunk."""
+    if chunk_tokens <= 0:
+        chunk_tokens = VARLEN_CHUNK_TOKENS
+    n, row0, starts = [], [], [0]
+    tok = acc = cap = 0
+    for i, (H, W) in enumerate(hw):
+        if H < patch or W < patch or H % patch or W % patch:
+            raise ValueError(f"image {i} is {H}x{W}, not a positive multiple of the patch size {patch}")
+        Ni = (H // patch) * (W // patch) + 1
+        if acc > 0 and acc + Ni > chunk_tokens:
+            cap, acc = max(cap, acc), 0
+            starts.append(i)
+        acc += Ni
+        n.append(Ni)
+        row0.append(tok)
+        tok += Ni
+    return dict(n=n, row0=row0, tokens=tok, starts=starts, cap=max(cap, acc))
+
+
 def _trunc_normal_(t: torch.Tensor, std: float = 0.02, a: float = -2.0, b: float = 2.0) -> torch.Tensor:
     """Truncated-normal init with the reference's recipe (SSS/dino/utils.py:482-520)."""
     cdf = lambda v: (1.0 + math.erf(v / math.sqrt(2.0))) / 2.0   # noqa: E731
@@ -413,6 +439,48 @@ class VisionTransformer(nn.Module):
         fn = _lib.load_library().vitocm_forward_cls_attn_gray if (Cx == 1 and self.in_chans > 1) else _lib.load_library().vitocm_forward_cls_attn
         check(fn(eng, ptr(x), B, H, W, ptr(pos), ptr(out), ptr(ws), ws.numel(), chunk, cur_stream()))
         return out
+
+    @torch.no_grad()
+    def cls_attention_rows_varlen(self, images, chunk_tokens: int = VARLEN_CHUNK_TOKENS):
+        """cls_attention_rows for a list of images of different sizes in one forward: ``images`` = CUDA tensors [C, H_i, W_i]
+        (C = in_chans, or 1 for the gray fast path; one C for the whole list) -> list of [heads, N_i] fp32 views into one packed
+        buffer, each bit-identical to ``cls_attention_rows(images[i][None])[0]``.  The token rows of all images run through the
+        kernels as one stream, in chunks of at most ``chunk_tokens`` rows (an image of more tokens runs alone)."""
+        out, plan = self._cls_rows_varlen_packed(images, chunk_tokens)
+        return [out[self.num_heads * t0:self.num_heads * (t0 + n)].view(self.num_heads, n) for t0, n in zip(plan["row0"], plan["n"])]
+
+    def _cls_rows_varlen_packed(self, images, chunk_tokens: int = VARLEN_CHUNK_TOKENS):
+        """-> (the packed rows [heads * sum N_i] fp32, varlen_plan of the images)"""
+        self._refuse_drop_path("cls_attention_rows_varlen")
+        if len(images) == 0:
+            raise ValueError("cls_attention_rows_varlen needs at least one image")
+        xs = [self._check_input(im[None] if im.dim() == 3 else im, allow_gray=True) for im in images]
+        ch = xs[0].shape[1]
+        if any(x.shape[0] != 1 or x.shape[1] != ch for x in xs):
+            raise ValueError("cls_attention_rows_varlen: every image must be one [C, H, W] tensor with the same C")
+        eng = self._ensure_engine()
+        p = self.patch_embed.patch_size
+        hw = [(int(x.shape[2]), int(x.shape[3])) for x in xs]
+        plan = varlen_plan(hw, p, chunk_tokens)
+        tables, offs, pos_off = {}, [], []
+        rows = 0
+        for H, W in hw:   # one position table per distinct size, packed
+            if (H, W) not in tables:
+                tables[(H, W)] = (rows, self._pos_table((H // p) * (W // p), H, W))
+                rows += tables[(H, W)][1].shape[0]
+            pos_off.append(tables[(H, W)][0])
+        pos = torch.cat([t for _, t in tables.values()]) if len(tables) > 1 else next(iter(tables.values()))[1]
+        x = torch.cat([x.reshape(-1) for x in xs])
+        dev = x.device
+        need = int(_lib.load_library().vitocm_varlen_workspace_bytes(eng, plan["cap"]))
+        if self._ws is None or self._ws.numel() < need or self._ws.device != dev:
+            self._ws = torch.empty(need, dtype=torch.uint8, device=dev)
+        out = torch.empty(self.num_heads * plan["tokens"], dtype=torch.float32, device=dev)
+        hw_c = (C.c_int * (2 * len(hw)))(*[v for s in hw for v in s])
+        po_c = (C.c_int * len(pos_off))(*pos_off)
+        check(_lib.load_library().vitocm_forward_cls_attn_varlen(eng, ptr(x), len(xs), ch, hw_c, ptr(pos), po_c, ptr(out),
+                                                                 ptr(self._ws), self._ws.numel(), int(chunk_tokens), cur_stream()))
+        return out, plan
 
     @torch.no_grad()
     def cls_attention_rows_mosaic(self, mosaic: torch.Tensor, grid, window: int, stride: int, t0: int, count: int) -> torch.Tensor:
